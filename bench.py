@@ -18,6 +18,8 @@ K_true=20, generate_gaussian_data restated), one NCCL all-reduce of the packed s
            kernel works for its living)
 Unit at every N: "iters/s" = Gibbs sweeps over ONE C2-sized (1e6-point) problem per second; a weak-scaling step
 over N GPUs completes N of them (config.n_points_total says how many points one step covers).
+  --dump-outputs DIR: after the timed steps, writes what the last timed step computed (see dump_outputs) as
+           DIR/<name>.npy, so that two builds run with the same arguments can be compared output for output
 """
 import argparse
 import json
@@ -291,10 +293,36 @@ def check_allreduce(pkg, g, case, args, rank, world, dist, torch):
     return res
 
 
+DUMP_MAX_POINTS = 1 << 21   # per-point arrays: 2 x 8 MB as float32; the statistics add at most ~10 MB (C5: K=100, D=64)
+
+
+def dump_outputs(g, out_dir, write):
+    """The arrays a caller of the timed sweep receives, from its last step: labels and sub-labels of this rank's
+    points (float32, exact for these small integers) and the statistics of every cluster and sub-cluster (float64:
+    counts, sum x, and sum x x' for NIW).  Beyond DUMP_MAX_POINTS points the labels are those of a fixed sample of
+    points (the same sorted indices for every build: the sample depends only on n).  Every rank fetches (the fetch
+    of the statistics is a collective); `write` says whether this one writes."""
+    lab, sub = g.get_labels(), g.get_sublabels()
+    counts, sum_x, sum_xx = g.suff_stats()
+    if not write:
+        return
+    if g.n > DUMP_MAX_POINTS:
+        sel = np.sort(np.random.default_rng(0).choice(g.n, DUMP_MAX_POINTS, replace=False))
+        lab, sub = lab[sel], sub[sel]
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"labels": lab.astype(np.float32), "sublabels": sub.astype(np.float32),
+              "counts": counts.astype(np.float64), "sum_x": sum_x}
+    if sum_xx is not None:
+        arrays["sum_xx"] = sum_xx
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"[bench] wrote {', '.join(arrays)} to {out_dir} ({sum(a.nbytes for a in arrays.values()) / 1e6:.1f} MB)")
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200, help="timed sweeps (>= 1)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="c2", choices=sorted(WORKLOADS))
@@ -306,7 +334,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-fit", action="store_true")
     ap.add_argument("--no-check", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the labels, sub-labels and statistics of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -326,7 +358,6 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
         dist.barrier()
     pkg = dpmm_pkg.load()
-    args.steps = max(args.steps, 1)
     args.warmup = max(args.warmup, 3)
     strong = args.scaling == "strong" and world > 1
 
@@ -424,6 +455,8 @@ def main():
     dev_ms = max(dev_ms_all)
     clocks = sampler.result()
     ms_step = dev_ms / args.steps
+    if args.dump_outputs:
+        dump_outputs(g, args.dump_outputs, rank == 0)
 
     # ---- e2e (round 1's definition): host parameters in, host statistics out, every step ----
     for _ in range(3):

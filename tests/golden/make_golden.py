@@ -1,7 +1,7 @@
 """Generate the golden fixtures under tests/golden/ from the reference's own checkpoints.
 
-Run HERE (build container), where /root/reference exists; the outputs are committed because
-/root/reference does not exist on the GPU box.
+usage: python tests/golden/make_golden.py <checkout of BGU-CS-VIL/DPMMSubClusters.jl>
+The outputs are committed, so that the tests need no copy of the reference.
 
 Sources (data files only, no reference source code is copied):
   examples/save_load_model/2d1ksample.npy + checkpoint__50.jld2   (NIW, D=2, K=5)
@@ -17,7 +17,7 @@ import os
 import sys
 import numpy as np
 
-REF = "/root/reference"
+REF = sys.argv[1] if len(sys.argv) > 1 else None
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -141,7 +141,7 @@ def make_mnm():
 
 
 if __name__ == "__main__":
-    if not os.path.isdir(REF):
-        sys.exit("needs /root/reference (build container only)")
+    if REF is None or not os.path.isdir(REF):
+        sys.exit("usage: make_golden.py <checkout of BGU-CS-VIL/DPMMSubClusters.jl>")
     make_niw()
     make_mnm()

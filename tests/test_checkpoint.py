@@ -13,8 +13,6 @@ from dpmmsubclusters_jl_b200 import host as H  # noqa: E402
 from dpmmsubclusters_jl_b200 import checkpoint as CK  # noqa: E402
 from dpmmsubclusters_jl_b200 import priors as P  # noqa: E402
 
-REF = "/root/reference"
-
 
 def oracle_factory(x, kind, seed, goff):
     return O.OracleSweep(x, kind, seed=seed, global_offset=goff)
@@ -67,12 +65,20 @@ def test_load_data_matches_the_reference_loader(tmp_path):
     np.testing.assert_array_equal(CK.load_data(str(tmp_path) + "/", prefix="bob", swapDimension=False)[0], a[0])
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference tree not present (GPU box)")
-def test_load_data_reads_the_reference_fixtures():
-    x = CK.load_data(REF + "/examples/save_load_model/", prefix="2d1ksample")
+def test_load_data_reads_the_reference_fixtures(tmp_path, golden_dir):
+    """The reference's data files examples/save_load_model/2d1ksample.npy (1000 x 2 Float64) and
+    test/save_load_test/mnm_data.npy (1000 x 100 Float32), N x D on disk, restored from the golden fixtures that
+    tests/golden/make_golden.py stored them in (D x N, same values)."""
+    gn = np.load(os.path.join(golden_dir, "niw_2d1k_checkpoint50.npz"))
+    gm = np.load(os.path.join(golden_dir, "mnm_1k_checkpoint20.npz"))
+    np.save(tmp_path / "2d1ksample.npy", gn["x"].T)
+    np.save(tmp_path / "mnm_data.npy", gm["x"].T)
+    x = CK.load_data(str(tmp_path) + "/", prefix="2d1ksample")
     assert x.shape == (2, 1000)
-    m = CK.load_data(REF + "/test/save_load_test/", prefix="mnm_data")
+    np.testing.assert_array_equal(x, gn["x"])
+    m = CK.load_data(str(tmp_path) + "/", prefix="mnm_data")
     assert m.shape[0] == 100 and (m.sum(0) == 50).all()          # generate_mnmm_data: 50 trials per point
+    np.testing.assert_array_equal(m, gm["x"])
 
 
 def test_parameter_file_in_the_reference_style(tmp_path):
@@ -84,13 +90,6 @@ def test_parameter_file_in_the_reference_style(tmp_path):
     hp = gp["hyper_params"]
     assert isinstance(hp, P.niw_hyperparams) and hp.ν == 5 and hp.m.shape == (2,)
     np.testing.assert_array_equal(hp.ψ, np.eye(2))
-
-
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference tree not present (GPU box)")
-def test_the_reference_own_global_params_file_parses():
-    gp = CK.read_params(REF + "/src/global_params.jl")
-    assert gp["iterations"] == 100 and gp["burnout_period"] == 20 and gp["smart_splits"] is False
-    assert isinstance(gp["hyper_params"], P.niw_hyperparams)
 
 
 def _advanced_run(tmp_path, device_params, factory, iters=30, interval=10):
