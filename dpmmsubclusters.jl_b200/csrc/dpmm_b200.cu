@@ -738,8 +738,6 @@ static int niw_pack_launch(dpmm_ctx* ctx, int K, const double* lfac) {
   if (ctx->t2_ok) {
     t2_nch = gauss_tc2_nch(D, K);
     t2_ks = (D == 32 && t2_nch <= 4) ? D : 8;
-    const int ks_env = env_int("DPMM_TC2_KS", 0);
-    if (ks_env == 8 || ks_env == D) t2_ks = ks_env;
     t2p = K <= T2_MAX_K && GaussTc2Smem(D, K, t2_ks, t2_nch, std::max(K, ctx->label_bound) + 8).total <= (size_t)ctx->smem_optin;
     if (t2p) CK(cudaMemsetAsync(ctx->t2_scr, 0, (size_t)t2_nch * (t2_ks / 8) * 4096, ctx->stream));
   }
@@ -926,7 +924,7 @@ static int launch_label_tc2(dpmm_ctx* ctx, int final_iter, int nkeys) {
   ctx->ctr_clean = true;
   // the last block of the overflow kernel scans the new label histogram (label_scan_kernel's job) when the scan's
   // width is the K of this call: one launch fewer between the label kernel and the sort
-  l.ticket = env_int("DPMM_SCAN_FUSED", 1) != 0 ? ctx->tc_stats + 3 : nullptr; l.scan_k = K; l.seg_off = ctx->seg_off; l.scat_cursor = ctx->scat_cursor; l.lr_cursor = ctx->lr_cursor;
+  l.ticket = ctx->tc_stats + 3; l.scan_k = K; l.seg_off = ctx->seg_off; l.scat_cursor = ctx->scat_cursor; l.lr_cursor = ctx->lr_cursor;
   const size_t lsm = (size_t)8 * K * 4;
   if (lsm > 48 * 1024) CK(cudaFuncSetAttribute(gauss_label_list_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lsm));
   {
@@ -979,11 +977,9 @@ static int run_sample_labels(dpmm_ctx* ctx, int final_iter, float* dump) {
     if (rc) return rc;
   }
   CK(cudaMemsetAsync(ctx->hist, 0, (size_t)K * 4, ctx->stream));
-  bool scanned = false;
   if (use_t2) {
     int rc = ctx->D == 32 ? launch_label_tc2<32>(ctx, final_iter, nkeys) : launch_label_tc2<64>(ctx, final_iter, nkeys);
     if (rc) return rc;
-    scanned = env_int("DPMM_SCAN_FUSED", 1) != 0;
   } else if (ctx->prior == DPMM_PRIOR_NIW && ctx->tc_params && dump == nullptr && ctx->sampler == DPMM_SAMPLER_INVERSE_CDF &&
       env_int("DPMM_LABEL_TC", 2) != 0) {
     // K2: tcgen05 TF32 screen + FP32 refine
@@ -1045,7 +1041,7 @@ static int run_sample_labels(dpmm_ctx* ctx, int final_iter, float* dump) {
     CK(cudaGetLastError());
   }
   ctx->hist_valid = true;
-  ctx->scan_valid = scanned;   // the overflow kernel's last block already scanned the new histogram (width K)
+  ctx->scan_valid = use_t2;   // the overflow kernel's last block already scanned the new histogram (width K)
   ctx->sorted = false;
   ctx->partitioned = ctx->stats_cached = false;
   ctx->label_bound = K;
@@ -1122,7 +1118,7 @@ static int run_sublabels(dpmm_ctx* ctx, bool sample, float* dump) {
     f.x = ctx->x; f.n = ctx->n; f.K = K; f.perm = ctx->perm; f.seg_off = ctx->seg_off; f.w = ctx->ss_w; f.bias = ctx->ss_b;
     f.cen = ctx->ss_c; f.cst = ctx->cst; f.loglr = ctx->loglr; f.sub = ctx->sub; f.acc = ctx->acc; f.rec = recs;
     f.lcount = ctx->lcount; f.centers = ctx->centers; f.u_inj = ctx->u_sub; f.seed = ctx->seed; f.call = ctx->call;
-    f.goff = ctx->goff; f.dump = dump; f.dbg = env_int("DPMM_SS_DEBUG", 0);
+    f.goff = ctx->goff; f.dump = dump;
     const size_t smem = SubStatsSmem(K).total;
     CK(cudaFuncSetAttribute(niw_substats_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     {

@@ -47,24 +47,8 @@ __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t by
 // Wait for the phase with the given parity.  try_wait suspends the thread in hardware until the phase completes or a
 // time limit passes; without a hint that limit is short and the loop around it spins -- in the warp-specialised
 // kernels here a quarter of all issued instructions were such polls, competing with the working warps of the same
-// scheduler.  TC_WAIT_HINT_NS (> 0) passes an explicit suspend-time hint.
-#ifndef TC_WAIT_HINT_NS
-#define TC_WAIT_HINT_NS 0
-#endif
+// scheduler.  Yet an explicit suspend-time hint measured slower (see the header of kernels_substats_tc.cuh).
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-#if TC_WAIT_HINT_NS > 0
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "LAB_WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n\t"
-      "@p bra LAB_DONE_%=;\n\t"
-      "bra LAB_WAIT_%=;\n\t"
-      "LAB_DONE_%=:\n\t"
-      "}" ::"r"(smem_u32(bar)),
-      "r"(parity), "r"((uint32_t)TC_WAIT_HINT_NS)
-      : "memory");
-#else
   asm volatile(
       "{\n\t"
       ".reg .pred p;\n\t"
@@ -76,7 +60,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
       "}" ::"r"(smem_u32(bar)),
       "r"(parity)
       : "memory");
-#endif
 }
 __device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }

@@ -48,25 +48,10 @@
 #define T2_R 8             // screen rows per cluster
 #define T2_DELTA 30.0f
 #define T2_MAX_K 256        // bias tables are K x K
-#ifndef T2_COOP_MAX
 #define T2_COOP_MAX 12      // candidate pairs in a warp up to which they are evaluated one at a time by all lanes
-#endif
 // (measured and rejected: sending the candidate points of a warp with more pairs than that to the overflow list --
 //  the all-K list kernel then costs 6 ms on the overlapping-clusters state of C2, against 1 ms evaluated in place)
-#ifndef T2_NS32
 #define T2_NS32 4          // stage ring at D = 32 (D = 64: 3)
-#endif
-#ifndef T2_ABL
-#define T2_ABL 0           // development: ablation bits (timing experiments only, results are wrong)
-#endif
-#ifndef T2_PROF
-#define T2_PROF 0          // 1: CTA 0 prints the cycles its role leaders spent in each wait (development only)
-#endif
-#if T2_PROF
-#define T2_WAIT(slot, stmt) do { const long long t__ = clock64(); stmt; prof[slot] += clock64() - t__; } while (0)
-#else
-#define T2_WAIT(slot, stmt) do { stmt; } while (0)
-#endif
 
 struct GaussTc2Args {
   const float* x;          // [n][D]
@@ -144,12 +129,8 @@ __host__ __device__ inline int gauss_tc2_nch(int D, int K) {
 // Every new run re-stages the pivot image behind a drained MMA pipeline (~1.5 us), so the number of rounds adapts:
 // segments of at least T2_SEG_MIN tiles, at most T2_ROUNDS rounds (C2, 53 tiles per CTA: one contiguous range as
 // before; 8 rounds of 6.6 tiles cost it 76.6 -> 88 us).
-#ifndef T2_ROUNDS
 #define T2_ROUNDS 8
-#endif
-#ifndef T2_SEG_MIN
 #define T2_SEG_MIN 32
-#endif
 struct T2Seq {
   const int32_t* B;   // [nkeys + 1] key boundaries (positions)
   const int32_t* P;   // [nkeys + 1] exclusive prefix of tiles per key
@@ -344,8 +325,6 @@ __global__ void __launch_bounds__(T2_THREADS(D), 1) gauss_label_tc2_kernel(const
   const int K = a.K, KS = a.KS, nch = a.nch, n0 = a.n0, nkeys = a.nkeys;
   const GaussTc2Smem L(D, K, KS, nch, nkeys);
   constexpr int NS = D == 32 ? T2_NS32 : 3;
-  [[maybe_unused]] long long prof[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-  [[maybe_unused]] const long long t_start = T2_PROF ? clock64() : 0;
   constexpr int PF = NS - 2;
   constexpr int PIVF = D * D;                     // floats of a pivot image
   uint8_t* stage0 = smem + L.stages;
@@ -457,19 +436,19 @@ __global__ void __launch_bounds__(T2_THREADS(D), 1) gauss_label_tc2_kernel(const
         if ((li & 1) != g) continue;
         const int s = li % NS;
         const int key = min(w.key, K - 1);
-        T2_WAIT(0, tc::mbar_wait(&full[s], (li / NS) & 1));
+        tc::mbar_wait(&full[s], (li / NS) & 1);
         tc::tc_fence_after();
         const uint32_t st_a = tc::smem_u32(stage0 + (size_t)s * L.stage_bytes);
         for (int c = 0; c < nch; ++c, ++cc) {
           const int b = cc & 1;
-          T2_WAIT(1, tc::mbar_wait(&tempty[g * 2 + b], ((cc >> 1) & 1) ^ 1));   // epilogue drained this buffer
+          tc::mbar_wait(&tempty[g * 2 + b], ((cc >> 1) & 1) ^ 1);   // epilogue drained this buffer
           tc::tc_fence_after();
           const uint32_t tmem_d = tmem_u + g * 256 + b * 128;
           int col = 0;
           if (c == 0) {
             if (key != prevkey) {
               // (at most the previous tile's MMAs are outstanding here: the buffer wait above ordered the rest)
-              if (ntile_g > 0) T2_WAIT(2, tc::mbar_wait(&wdone[g], (ntile_g - 1) & 1));
+              if (ntile_g > 0) tc::mbar_wait(&wdone[g], (ntile_g - 1) & 1);
               const float4* src = reinterpret_cast<const float4*>(a.wpiv + (size_t)key * PIVF);
               float4* dst = reinterpret_cast<float4*>(pivs);
               for (int e = lane; e < PIVF / 4; e += 32) dst[e] = __ldg(src + e);
@@ -533,8 +512,7 @@ __global__ void __launch_bounds__(T2_THREADS(D), 1) gauss_label_tc2_kernel(const
         const bool valid = row < npts;
         const int32_t idx = valid ? __ldg(a.perm + w.pos + row) : 0;
         const float* stage = reinterpret_cast<const float*>(stage0 + (size_t)s * L.stage_bytes);
-        T2_WAIT(0, tc::mbar_wait(&full[s], (li / NS) & 1));
-        [[maybe_unused]] const long long tp0 = T2_PROF ? clock64() : 0;
+        tc::mbar_wait(&full[s], (li / NS) & 1);
         float xnorm;
         {
           f32x2_t nn0 = 0ull, nn1 = 0ull;
@@ -555,7 +533,6 @@ __global__ void __launch_bounds__(T2_THREADS(D), 1) gauss_label_tc2_kernel(const
         // of the 8 columns), |rows of U_k (x - mu_k)| >= 0.99 sqrt(q8) - s, and cluster k is NOT a candidate when
         // that exceeds sqrt(T), T = 2 (cc_k + 0.01 - thr); (a + b)^2 <= 2 a^2 + 2 b^2 turns it into
         //   q8 > 4.0816 (cc_k + 0.01 - thr) + 2.0408 s^2     (a NaN on either side keeps the candidate).
-        if (T2_PROF) prof[4] += clock64() - tp0;
         float thr = 0.f, A4 = 0.f;
         bool weird = false;
         int cnt = 0;
@@ -599,9 +576,8 @@ __global__ void __launch_bounds__(T2_THREADS(D), 1) gauss_label_tc2_kernel(const
         };
         for (int c = 0; c < nch; ++c, ++cc) {
           const int b = cc & 1;
-          T2_WAIT(1, tc::mbar_wait(&tfull[g * 2 + b], (cc >> 1) & 1));
+          tc::mbar_wait(&tfull[g * 2 + b], (cc >> 1) & 1);
           tc::tc_fence_after();
-          [[maybe_unused]] const long long tp1 = T2_PROF ? clock64() : 0;
           const uint32_t taddr = tmem_row + b * 128;
           const int ncl = c == 0 ? min(K, n0) : min(16, K - n0 - (c - 1) * 16);
           const int kbase = c == 0 ? 0 : n0 + (c - 1) * 16;
@@ -618,7 +594,7 @@ __global__ void __launch_bounds__(T2_THREADS(D), 1) gauss_label_tc2_kernel(const
             } else {
               tc::tmem_ld32(taddr, v);
               tc::tmem_ld32(taddr + 32, v1);          // first screen batch rides along
-              T2_WAIT(2, tc::tmem_ld_wait());
+              tc::tmem_ld_wait();
               qp = gauss_tc_screen_q(v);
             }
             const float2 cf = ccfro[key];
@@ -643,23 +619,16 @@ __global__ void __launch_bounds__(T2_THREADS(D), 1) gauss_label_tc2_kernel(const
             uint32_t v[32], v1[32];
             tc::tmem_ld32(taddr + col + b0 * 32, v);
             if (b0 + 1 < nb) tc::tmem_ld32(taddr + col + b0 * 32 + 32, v1);
-            T2_WAIT(2, tc::tmem_ld_wait());
+            tc::tmem_ld_wait();
             uint32_t h = screen4(v, c * 16 + b0 * 4);
             if (b0 + 1 < nb) h |= screen4(v1, c * 16 + b0 * 4 + 4) << 4;
-            if (T2_ABL & 1) {   // the same work once more (timing experiment)
-              asm volatile("" : "+r"(v[0]), "+r"(v1[0]));
-              h |= screen4(v, c * 16 + b0 * 4);
-              if (b0 + 1 < nb) h |= screen4(v1, c * 16 + b0 * 4 + 4) << 4;
-            }
             const int k0 = kbase + b0 * 4;
             if ((unsigned)(key - k0) < 8u) h &= ~(1u << (key - k0));
             if (h) append(h, k0);
           }
           tc::tc_fence_before();
           tc::mbar_arrive(&tempty[g * 2 + b]);
-          if (T2_PROF) prof[5] += clock64() - tp1;
         }
-        [[maybe_unused]] const long long tp2 = T2_PROF ? clock64() : 0;
         bool multi = valid && !weird && cnt > 0 && cnt < T2_CMAX;
         bool ovf = valid && (weird || cnt >= T2_CMAX);
         if (multi) {   // insert the pivot at its place (the list is ascending)
@@ -748,7 +717,6 @@ __global__ void __launch_bounds__(T2_THREADS(D), 1) gauss_label_tc2_kernel(const
           }
           ++npts_total;
         }
-        if (T2_PROF) prof[6] += clock64() - tp2;
       }
       {   // per-call counters (points, exact evaluations): read back asynchronously by the host's path choice
 #pragma unroll
@@ -803,7 +771,7 @@ __global__ void __launch_bounds__(T2_THREADS(D), 1) gauss_label_tc2_kernel(const
         cp_async_commit();
       }
       for (int li = 0; li < nt; ++li) {
-        T2_WAIT(0, cp_async_wait_group<PF - 1>());
+        cp_async_wait_group<PF - 1>();
         {   // centre this thread's chunks of the landed tile by the pivot's mean (rows beyond the tile stay zero)
           const int key = min(wc.key, K - 1);
           if (key != ckey) {
@@ -820,16 +788,6 @@ __global__ void __launch_bounds__(T2_THREADS(D), 1) gauss_label_tc2_kernel(const
             if (r < nrow) {
               v.x -= cen.x; v.y -= cen.y; v.z -= cen.z; v.w -= cen.w;
               *q = v;
-              if (T2_ABL & 2) {   // the same work once more (timing experiment)
-                asm volatile("" ::: "memory");
-                float4 u = *q;
-                u.x += cen.x; u.y += cen.y; u.z += cen.z; u.w += cen.w;
-                *q = u;
-                asm volatile("" ::: "memory");
-                u = *q;
-                u.x -= cen.x; u.y -= cen.y; u.z -= cen.z; u.w -= cen.w;
-                *q = u;
-              }
             }
           }
           t2_advance(wc, seq);
@@ -838,7 +796,7 @@ __global__ void __launch_bounds__(T2_THREADS(D), 1) gauss_label_tc2_kernel(const
         tc::mbar_arrive(&full[li % NS]);
         const int nx = li + PF;
         if (nx < nt) {
-          T2_WAIT(1, tc::mbar_wait(&empty[nx % NS], ((nx / NS) & 1) ^ 1));
+          tc::mbar_wait(&empty[nx % NS], ((nx / NS) & 1) ^ 1);
           issue(nx % NS);
           t2_advance(wl, seq);
           if (nx + 1 < nt) load_idx();
@@ -847,10 +805,6 @@ __global__ void __launch_bounds__(T2_THREADS(D), 1) gauss_label_tc2_kernel(const
       }
     }
   }
-#if T2_PROF
-  if (blockIdx.x == 0 && lane == 0 && (warp == 0 || warp == 2 || warp == 10))
-    printf("[t2 prof] warp %d tiles %d total %lld: wait0 %lld wait1 %lld wait2 %lld wait3 %lld | xnorm %lld chunks %lld post %lld\n", warp, nt, clock64() - t_start, prof[0], prof[1], prof[2], prof[3], prof[4], prof[5], prof[6]);
-#endif
   tc::tc_fence_before();
   __syncthreads();
   if (warp == 1) tc::tmem_dealloc(tmem_base, 512);

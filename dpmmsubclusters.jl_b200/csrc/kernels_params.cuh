@@ -29,14 +29,6 @@
 #include "kernels_pack.cuh"
 
 #define DPMM_STREAM_PARAMS 5u
-#ifndef PARAM_PROF
-#define PARAM_PROF 0
-#endif
-#if PARAM_PROF
-#define PP_MARK(i) do { __syncthreads(); if (blockIdx.x == 0 && threadIdx.x == 0) pp[i] = clock64(); } while (0)
-#else
-#define PP_MARK(i) do { } while (0)
-#endif
 #define NIW_HYPER_DOUBLES(D) (4 + (D) + (D) * (D))          // kappa, nu, logdet psi, lmvgamma(nu/2) | m | psi
 #define NIW_POST_DOUBLES(D) (8 + (D) + (D) * (D))           // kappa', nu', N, logml, logdet psi', ok, -, - | m' | Lhat
 
@@ -261,10 +253,6 @@ __global__ void __launch_bounds__(NIW_PACK_THREADS) niw_draw_kernel(const NiwDra
   const int t = blockIdx.x, tid = threadIdx.x, NT = NIW_PACK_THREADS;
   const double* P = a.post + (size_t)t * NIW_POST_DOUBLES(D);
   const bool prior = a.first != 0 || !(P[2] > 0.0);
-#if PARAM_PROF
-  __shared__ long long pp[12];
-#endif
-  PP_MARK(0);
   double kp, nup;
   const double* mpost;
   if (prior) {
@@ -286,7 +274,6 @@ __global__ void __launch_bounds__(NIW_PACK_THREADS) niw_draw_kernel(const NiwDra
     for (int e = tid; e < D * D; e += NT) Wk[(e / D) * LD + (e % D)] = P[8 + D + e];
     __syncthreads();
   }
-  PP_MARK(1);
   // ---- Bartlett factor B (lower) and the normals of the mean.  The D chi-square draws (rejection loops in
   //      Float64) go to the lanes of the last warp(s) together, so that no other warp diverges into them ----
   for (int e = tid; e < D * D + D; e += NT) {
@@ -306,7 +293,6 @@ __global__ void __launch_bounds__(NIW_PACK_THREADS) niw_draw_kernel(const NiwDra
     Bm[i * LD + i] = sqrt(2.0 * rng.gamma(0.5 * (nup - i)));
   }
   __syncthreads();
-  PP_MARK(2);
   // ---- L = M B with M = V^-T / sqrt(nu'), V = P Lhat P:  Lhat' X = P B / sqrt(nu'),  X = P L.
   //      Back substitution over the rows of the upper-triangular Lhat' in its column-oriented form (once x_i is
   //      final, every row k < i of the right-hand side loses Lhat[i][k] x_i).
@@ -342,11 +328,9 @@ __global__ void __launch_bounds__(NIW_PACK_THREADS) niw_draw_kernel(const NiwDra
     }
   }
   __syncthreads();
-  PP_MARK(4);
   __shared__ int ok_s;
   if (tid == 0) ok_s = 1;
   __syncthreads();
-  PP_MARK(5);
   for (int e = tid; e < D * D; e += NT) {
     const int i = e / D, j = e - i * D;
     const double v = j <= i ? Ls[i * LD + j] : 0.0;          // (entries above the diagonal are rounding residue)
@@ -382,11 +366,6 @@ __global__ void __launch_bounds__(NIW_PACK_THREADS) niw_draw_kernel(const NiwDra
     if (lane + 32 < D) a.mu[(size_t)t * D + lane + 32] = (float)(mpost[lane + 32] + y1 * rk);
     if (lane == 0) a.logdet[t] = okk ? (float)(-2.0 * lg) : __int_as_float(0x7fc00000);
   }
-  PP_MARK(6);
-#if PARAM_PROF
-  if (blockIdx.x == 0 && threadIdx.x == 0)
-    printf("[draw prof] load %lld bartlett %lld solve %lld mean %lld\n", pp[1] - pp[0], pp[2] - pp[1], pp[4] - pp[2], pp[6] - pp[4]);
-#endif
 }
 
 struct WeightsArgs {

@@ -47,37 +47,20 @@
 
 #define SS_D 32
 #define SS_TILE 128
-#ifndef SS_RAW
 #define SS_RAW 5                         // ring of raw tiles: landing -> split -> permuting pass
-#endif
-#ifndef SS_PF
 #define SS_PF 2                          // tiles of gather in flight
-#endif
-#ifndef SS_NG
 #define SS_NG 3                          // GEMM1 epilogue groups (4 warps each), tile li -> group li % SS_NG
-#endif
-#ifndef SS_GPHILOX
-#define SS_GPHILOX 0                     // 1: the gather warps evaluate the sub-label uniforms (measured: slower)
-#endif
-#ifndef SS_FLUSH
 #define SS_FLUSH 8                       // tiles per GEMM2 flush group (TMEM accumulates 1024 points between drains)
-#endif
-#ifndef SS_NTB
-#define SS_NTB (SS_NG == 3 ? 6 : SS_NG)  // GEMM1 accumulator buffers (64 TMEM columns each), tile li -> buffer li % SS_NTB
-#endif
-#define SS_THREADS (768 + (SS_NG - 2) * 128)
+#define SS_NTB 6                         // GEMM1 accumulator buffers (64 TMEM columns each), tile li -> buffer li % SS_NTB
+#define SS_THREADS 896
 #define SS_GATHER 256                    // gather threads: warps 0-3 and 19-22, 4 rows each
 #define SS_PANEL 16384                   // one [128][32] Float32 panel
 #define SS_PROWS 136                     // rows of a permuted panel: both runs padded to a multiple of 8
 #define SS_PPANEL (SS_PROWS * 128)
 #define SS_WSLOT (8192 + 8192 + 2048)    // Wh | Wl | bias k-step operand
-#define SS_TMEM_COLS (SS_NTB == 2 ? 256 : 512)  // GEMM1: SS_NTB x 64 columns, GEMM2: 2 x 64 columns
+#define SS_TMEM_COLS 512                 // GEMM1: SS_NTB x 64 columns, GEMM2: 2 x 64 columns
 #define SS_TMEM_G2 (SS_NTB * 64)         // first column of the GEMM2 accumulators
 #define SS_TLD 65
-#ifndef SS_DEBUG_SWITCHES
-#define SS_DEBUG_SWITCHES 0     // 1: the DPMM_SS_DEBUG ablation switches of tools/ss_debug_timing.py are live
-#endif
-#define SS_DBG (SS_DEBUG_SWITCHES ? a.dbg : 0)
 
 struct SubStatsArgs {
   const float* x;
@@ -100,11 +83,10 @@ struct SubStatsArgs {
   uint32_t call;
   int64_t goff;
   float* dump;             // optional [2][n]
-  int dbg;                 // development switches, compiled in with -DSS_DEBUG_SWITCHES=1 (timing experiments only)
 };
 
 struct SubStatsSmem {
-  size_t raw, split, perm, wslot, aaug, tbuf, tri, ubuf, dest, cnt, kcnt, bnd, pre, bars, slot, total;
+  size_t raw, split, perm, wslot, aaug, tbuf, tri, dest, cnt, kcnt, bnd, pre, bars, slot, total;
   __host__ __device__ explicit SubStatsSmem(int K) {
     size_t o = 0;
     raw = o;    o += (size_t)SS_RAW * SS_PANEL;
@@ -115,7 +97,6 @@ struct SubStatsSmem {
     tbuf = o;   o += 64 * SS_TLD * 4;
     tri = o;    o += 528 * 2;
     o = (o + 15) & ~(size_t)15;
-    ubuf = o;   o += SS_GPHILOX ? (size_t)SS_RAW * SS_TILE * 8 : 0;   // the sub-label uniforms of the tiles in the raw ring (f64)
     dest = o;   o += SS_NG * SS_TILE;
     cnt = o;    o += SS_NG * 4 * 4;
     kcnt = o;   o += 4 * 4;
@@ -128,52 +109,6 @@ struct SubStatsSmem {
   }
 };
 
-__device__ __forceinline__ void ss_wait(int dbg, uint64_t* bar, uint32_t parity) {
-  if (dbg & 64) {   // experiment: spin on test_wait instead of the suspending try_wait
-    uint32_t done = 0;
-    do {
-      asm volatile(
-          "{\n\t"
-          ".reg .pred p;\n\t"
-          "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-          "selp.u32 %0, 1, 0, p;\n\t"
-          "}"
-          : "=r"(done)
-          : "r"(tc::smem_u32(bar)), "r"(parity)
-          : "memory");
-    } while (!done);
-  } else {
-    tc::mbar_wait(bar, parity);
-  }
-}
-
-// Wait of a warp that is NOT on the critical path (gather, issuers, drain, staging): back off with nanosleep
-// between polls, so that its polling does not compete with the epilogue warps for issue slots and the
-// shared-memory pipe.
-#ifndef SS_SLEEP
-#define SS_SLEEP 0
-#endif
-__device__ __forceinline__ void ss_wait_lazy(uint64_t* bar, uint32_t parity, uint32_t ns) {
-#if SS_SLEEP
-  uint32_t done = 0;
-  for (;;) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t"
-        "}"
-        : "=r"(done)
-        : "r"(tc::smem_u32(bar)), "r"(parity)
-        : "memory");
-    if (done) break;
-    __nanosleep(ns);
-  }
-#else
-  tc::mbar_wait(bar, parity);
-#endif
-}
-
 __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const SubStatsArgs a) {
   extern __shared__ __align__(1024) uint8_t ss_smem[];
   const SubStatsSmem L(a.K);
@@ -185,7 +120,6 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
   float* T = reinterpret_cast<float*>(ss_smem + L.tbuf);
   uint16_t* tri = reinterpret_cast<uint16_t*>(ss_smem + L.tri);
   uint8_t* dest_s = ss_smem + L.dest;
-  double* ubuf = reinterpret_cast<double*>(ss_smem + L.ubuf);
   volatile int32_t* cnt_s = reinterpret_cast<int32_t*>(ss_smem + L.cnt);
   volatile int32_t* kcnt = reinterpret_cast<int32_t*>(ss_smem + L.kcnt);
   int32_t* B = reinterpret_cast<int32_t*>(ss_smem + L.bnd);
@@ -300,19 +234,12 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
           idx[j] = p < wl.end ? __ldg(a.perm + p) : -1;
         }
       };
-      // ... and the uniform of the sub-label draw of row r0 + 32 c (chunk lanes 0-3), so that the Philox rounds
-      // are off the epilogue warps' per-tile chain; the epilogue reads it after the tile's `landed` barrier
       auto issue = [&](int s) {
         uint8_t* dst = raw0 + (size_t)s * SS_PANEL + offr;
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           const bool ok = idx[j] >= 0;
-          if (!(SS_DBG & 16)) cp_async16(dst + j * 4096, a.x + (size_t)(ok ? idx[j] : 0) * SS_D + 4 * c, ok ? 16 : 0);
-        }
-        if (SS_GPHILOX && c < 4) {
-          const int ix = c == 0 ? idx[0] : (c == 1 ? idx[1] : (c == 2 ? idx[2] : idx[3]));
-          if (ix >= 0)
-            ubuf[s * SS_TILE + r0 + 32 * c] = dpmm_uniform(a.u_inj, ix, a.seed, DPMM_STREAM_SUBLABEL, a.call, (uint64_t)(a.goff + ix));
+          cp_async16(dst + j * 4096, a.x + (size_t)(ok ? idx[j] : 0) * SS_D + 4 * c, ok ? 16 : 0);
         }
       };
 #pragma unroll
@@ -338,20 +265,6 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
         cp_async_wait_group<SS_PF - 1>();
         uint8_t* src = raw0 + (size_t)(li % SS_RAW) * SS_PANEL + offr;
         float4 v[4];
-        if (SS_DBG & 512) {
-          tc::mbar_arrive(&landed[li % SS_RAW]);
-          ss_wait(SS_DBG, &sfree[b], ((li >> 1) & 1) ^ 1);
-          tc::fence_proxy_async();
-          tc::mbar_arrive(&ready[b]);
-          const int ln2 = li + SS_PF;
-          if (ln2 < nt) {
-            ss_wait(SS_DBG, &rfree[ln2 % SS_RAW], ((ln2 / SS_RAW) & 1) ^ 1);
-            stc_advance<SS_FLUSH>(wl, B);
-          }
-          cp_async_commit();
-          stc_advance<SS_FLUSH>(wc, B);
-          continue;
-        }
 #pragma unroll
         for (int j = 0; j < 4; ++j) v[j] = *reinterpret_cast<const float4*>(src + j * 4096);
         float4 lo[4];
@@ -365,7 +278,7 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
           lo[j].z = v[j].z - tc::trunc_tf32(v[j].z); lo[j].w = v[j].w - tc::trunc_tf32(v[j].w);
         }
         tc::mbar_arrive(&landed[li % SS_RAW]);             // this thread's chunks of z are in shared memory
-        ss_wait_lazy(&sfree[b], ((li >> 1) & 1) ^ 1, 32);     // GEMM1 of tile li - 2 has read the l panel
+        tc::mbar_wait(&sfree[b], ((li >> 1) & 1) ^ 1);     // GEMM1 of tile li - 2 has read the l panel
         uint8_t* lk = split0 + (size_t)b * SS_PANEL + offk;
 #pragma unroll
         for (int j = 0; j < 4; ++j) *reinterpret_cast<float4*>(lk + j * 4096) = lo[j];
@@ -374,7 +287,7 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
         // next gather: tile li + PF goes into the slot of tile li + PF - RAW once its permuting pass is done
         const int ln = li + SS_PF;
         if (ln < nt) {
-          ss_wait_lazy(&rfree[ln % SS_RAW], ((ln / SS_RAW) & 1) ^ 1, 64);
+          tc::mbar_wait(&rfree[ln % SS_RAW], ((ln / SS_RAW) & 1) ^ 1);
           issue(ln % SS_RAW);
           stc_advance<SS_FLUSH>(wl, B);
           if (ln + 1 < nt) load_idx();
@@ -407,11 +320,11 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
           if (wm.key != prevkey) {
             prevkey = wm.key;
             ++kj;
-            ss_wait_lazy(wfull, kj & 1, 32);
+            tc::mbar_wait(wfull, kj & 1);
           }
           const int tb = li % SS_NTB, tph = (li / SS_NTB) & 1;
-          ss_wait_lazy(&ready[b], (li >> 1) & 1, 32);
-          ss_wait_lazy(&d1empty[tb], tph ^ 1, 32);
+          tc::mbar_wait(&ready[b], (li >> 1) & 1);
+          tc::mbar_wait(&d1empty[tb], tph ^ 1);
           tc::tc_fence_after();
           uint64_t hd[4], ld[4];
 #pragma unroll
@@ -420,7 +333,6 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
             ld[ks] = l_desc + (uint64_t)(b * (SS_PANEL >> 4) + ks * 2);
           }
           const uint32_t tmem_d = tmem_u + tb * 64;
-          if (!(SS_DBG & 8)) {
           tc::umma_tf32_first_w(tmem_d, hd[0], whd[0], idesc1);
 #pragma unroll
           for (int ks = 1; ks < 4; ++ks) tc::umma_tf32_acc_w(tmem_d, hd[ks], whd[ks], idesc1);
@@ -429,7 +341,6 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
 #pragma unroll
           for (int ks = 0; ks < 4; ++ks) tc::umma_tf32_acc_w(tmem_d, hd[ks], wld[ks], idesc1);
           tc::umma_tf32_acc_w(tmem_d, aaug_desc, baug_desc, idesc1);   // Y -= b
-          }
           tc::umma_commit_w(&sfree[b]);
           tc::umma_commit_w(&d1full[tb]);
           if (wm.pos + SS_TILE >= wm.end) tc::umma_commit_w(wempty);   // last tile of the cluster
@@ -445,9 +356,9 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
         const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
         StcWalk wm;
         stc_walk_init(wm, B, P, nkeys, t0, t1);
-        // M = 64.  (Experiment switch 2048: M = 128 with two garbage atoms after the panels, whose products
-        // land in accumulator rows 64-127 that nobody reads -- measured 4 % slower, not faster.)
-        const uint32_t idesc2 = (SS_DBG & 2048) ? tc::idesc_tf32_mn_m128(32) : tc::idesc_tf32_mn_m64(32);
+        // M = 64.  (M = 128 with two garbage atoms after the panels, whose products land in accumulator rows
+        // 64-127 that nobody reads, was measured 4 % slower, not faster.)
+        const uint32_t idesc2 = tc::idesc_tf32_mn_m64(32);
         // A = [h | l] (two 32-row atoms, one panel apart), B = h: the same descriptor, one k-step = 8 rows = 1024 B
         const uint64_t pd0 = tc::smem_desc_mn128(tc::smem_u32(perm0), SS_PPANEL);
         const uint64_t pd1 = tc::smem_desc_mn128(tc::smem_u32(perm0 + 2 * SS_PPANEL), SS_PPANEL);
@@ -455,11 +366,11 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
         for (int li = 0; li < nt; ++li) {
           const int b = li & 1;
           const bool first = wm.gcount == 0, last = stc_is_last<SS_FLUSH>(wm);
-          ss_wait_lazy(&permd[b], (li >> 1) & 1, 32);
-          if (first) ss_wait_lazy(&d2empty[g2 & 1], ((g2 >> 1) & 1) ^ 1, 64);
+          tc::mbar_wait(&permd[b], (li >> 1) & 1);
+          if (first) tc::mbar_wait(&d2empty[g2 & 1], ((g2 >> 1) & 1) ^ 1);
           tc::tc_fence_after();
           const int nkl = __shfl_sync(0xffffffffu, kcnt[b * 2], 0), nkr = __shfl_sync(0xffffffffu, kcnt[b * 2 + 1], 0);
-          const int k0 = right ? nkl : 0, nk = (SS_DBG & 4) ? 0 : (right ? nkr : nkl);
+          const int k0 = right ? nkl : 0, nk = right ? nkr : nkl;
           const uint32_t tm = tmem_u + SS_TMEM_G2 + (g2 & 1) * 64 + right * 32;
           uint64_t pd = (b ? pd1 : pd0) + (uint64_t)(k0 * 64);
           int ks = 0;
@@ -512,43 +423,27 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
 
         }
         double u = 0.0;
-        if (!SS_GPHILOX && valid) u = dpmm_uniform(a.u_inj, idx, a.seed, DPMM_STREAM_SUBLABEL, a.call, (uint64_t)(a.goff + idx));
+        if (valid) u = dpmm_uniform(a.u_inj, idx, a.seed, DPMM_STREAM_SUBLABEL, a.call, (uint64_t)(a.goff + idx));
         const int tb = li % SS_NTB;
-        ss_wait(SS_DBG, &d1full[tb], (li / SS_NTB) & 1);
+        tc::mbar_wait(&d1full[tb], (li / SS_NTB) & 1);
         tc::tc_fence_after();
         uint32_t v0[32], v1[32];
         const uint32_t taddr = tmem_base + ((uint32_t)(sub * 32) << 16) + tb * 64;
-        float ql = 1.f, qr = 2.f;
-        if (!(SS_DBG & 128)) {
         tc::tmem_ld32(taddr, v0);
         tc::tmem_ld32(taddr + 32, v1);
         tc::tmem_ld_wait();
-        ql = gauss_tc_screen_q(v0), qr = gauss_tc_screen_q(v1);
-        }
+        const float ql = gauss_tc_screen_q(v0), qr = gauss_tc_screen_q(v1);
         tc::tc_fence_before();
         tc::mbar_arrive(&d1empty[tb]);
         int side = 2;
-        if (SS_GPHILOX) {
-          ss_wait(SS_DBG, &landed[li % SS_RAW], (li / SS_RAW) & 1);   // the uniforms of the tile (gather warps)
-          if (valid) u = ubuf[(li % SS_RAW) * SS_TILE + row];
-        }
         if (valid) {
           const float rl = gauss_finish(cl, ql, lwl), rr = gauss_finish(cr, qr, lwr);
           if (a.dump != nullptr) {
             a.dump[idx] = rl;
             a.dump[a.n + idx] = rr;
           }
-          side = (SS_DBG & 1) ? (row & 1) : dpmm_draw_two(rl, rr, u);
+          side = dpmm_draw_two(rl, rr, u);
           a.sub[idx] = (uint8_t)side;
-        }
-        if (SS_DBG & 1024) {
-          if (li >= 2) ss_wait(SS_DBG, &pfree[(li - 2) & 3], ((li - 2) >> 2) & 1);
-          if (gt == 0) { kcnt[b * 2] = 8; kcnt[b * 2 + 1] = 8; }
-          tc::fence_proxy_async();
-          tc::mbar_arrive(&permd[b]);
-          tc::mbar_arrive(&rfree[li % SS_RAW]);
-          stc_advance<SS_FLUSH>(we, B);
-          continue;
         }
         // ---- destination row of every point: left run first, right run from a multiple of 8 ----
         const uint32_t bl = __ballot_sync(0xffffffffu, side == 0), br = __ballot_sync(0xffffffffu, side == 1);
@@ -572,8 +467,8 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
         dest_g[row] = side == 0 ? (uint8_t)(offl + __popc(bl & lt_mask))
                                 : (side == 1 ? (uint8_t)(nl8 + offr_ + __popc(br & lt_mask)) : (uint8_t)dinv);
         if (gt == 0 && nl > 0) atomicAdd(a.lcount + key, nl);
-        if (!SS_GPHILOX) ss_wait(SS_DBG, &landed[li % SS_RAW], (li / SS_RAW) & 1);   // z of the tile (gathered and centred by the gather warps)
-        if (li >= 2) ss_wait(SS_DBG, &pfree[(li - 2) & 3], ((li - 2) >> 2) & 1);   // the GEMM2 that read this slot two tiles ago
+        tc::mbar_wait(&landed[li % SS_RAW], (li / SS_RAW) & 1);   // z of the tile (gathered and centred by the gather warps)
+        if (li >= 2) tc::mbar_wait(&pfree[(li - 2) & 3], ((li - 2) >> 2) & 1);   // the GEMM2 that read this slot two tiles ago
         asm volatile("bar.sync %0, 128;" ::"r"(1 + g) : "memory");
         if (gt == 0) {
           kcnt[b * 2] = nl8 >> 3;
@@ -663,24 +558,19 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
       for (int li = 0; li < nt; ++li) {
         if (stc_is_last<SS_FLUSH>(wd)) {
           const int buf = g2 & 1;
-          ss_wait_lazy(&d2full[buf], (g2 >> 1) & 1, 200);
+          tc::mbar_wait(&d2full[buf], (g2 >> 1) & 1);
           ++g2;
           tc::tc_fence_after();
           uint32_t v0[32], v1[32];
           const uint32_t taddr = tmem_base + SS_TMEM_G2 + buf * 64 + ((uint32_t)(sub * 32) << 16);
-          if (!(SS_DBG & 256)) {
           tc::tmem_ld32(taddr, v0);
           tc::tmem_ld32(taddr + 32, v1);
           tc::tmem_ld_wait();
-          }
           tc::tc_fence_before();
           tc::mbar_arrive(&d2empty[buf]);
-          if (SS_DBG & 256) { stc_advance<SS_FLUSH>(wd, B); continue; }
           // M = 64: accumulator row m lives in lane (m % 16) of sub-partition m / 16
-          // (M = 128, experiment switch: row m lives in TMEM lane m, rows 0-63 = sub-partitions 0 and 1)
-          const bool m64 = (SS_DBG & 2048) == 0;
-          if (m64 ? lane < 16 : sub < 2) {
-            float* trow = T + (m64 ? 16 * sub + lane : 32 * sub + lane) * SS_TLD;
+          if (lane < 16) {
+            float* trow = T + (16 * sub + lane) * SS_TLD;
 #pragma unroll
             for (int j = 0; j < 32; ++j) {
               trow[j] = __uint_as_float(v0[j]);
@@ -693,7 +583,7 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
             const int ij = tri[e - sd * 528], i = ij >> 8, j = ij & 255;
             const int co = 32 * sd;
             const float sv = (T[i * SS_TLD + co + j] + T[(32 + i) * SS_TLD + co + j]) + T[(32 + j) * SS_TLD + co + i];
-            if (sv != 0.f && !(SS_DBG & 32)) atomicAdd(a.acc + (size_t)(2 * wd.key + sd) * a.rec + 1 + SS_D + i * SS_D + j, (double)sv);
+            if (sv != 0.f) atomicAdd(a.acc + (size_t)(2 * wd.key + sd) * a.rec + 1 + SS_D + i * SS_D + j, (double)sv);
           }
           asm volatile("bar.sync 6, 128;" ::: "memory");
         }
@@ -710,7 +600,7 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
       for (int li = 0; li < nt; ++li) {
         if (wp.key != prevkey) {
           prevkey = wp.key;
-          ss_wait_lazy(wempty, (kj & 1) ^ 1, 200);   // every GEMM1 of the previous cluster has retired
+          tc::mbar_wait(wempty, (kj & 1) ^ 1);   // every GEMM1 of the previous cluster has retired
           const float4* src = reinterpret_cast<const float4*>(a.w + (size_t)wp.key * 2 * SS_D * SS_D);
           for (int e = lane; e < 512; e += 32) {
             const int r = e >> 3, cc = e & 7;   // row (side, i), 16-byte chunk

@@ -39,8 +39,7 @@ static int launch_gauss_label_p(dpmm_ctx* ctx, GaussLabelArgs a) {
     const size_t perwarp = ((size_t)32 * P * C::DS + (size_t)a.K * 32 * P) * 4;
     int W = fixed < (size_t)ctx->smem_optin ? (int)(((size_t)ctx->smem_optin - fixed) / perwarp) : 0;
     W = std::min(W, 12);
-    W = env_int("DPMM_LABEL_W", W);
-    if (W >= 6 && env_int("DPMM_LABEL_FORM", 1) == 1) {
+    if (W >= 6) {
       const size_t sm = fixed + (size_t)W * perwarp;
       auto kern = gauss_label_warp_kernel<D, P>;
       CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
@@ -72,10 +71,6 @@ static int launch_gauss_label_p(dpmm_ctx* ctx, GaussLabelArgs a) {
     if (ok) break;
   }
   if (!ok) return fail(ctx, DPMM_ELIMIT, "K too large for the label kernel's shared-memory slice");
-  // development overrides (tools/): DPMM_LABEL_T / DPMM_LABEL_KC
-  T = env_int("DPMM_LABEL_T", T);
-  KC = std::min(a.K, env_int("DPMM_LABEL_KC", KC));
-  if (bytes(T, KC) > budget1) return fail(ctx, DPMM_ELIMIT, "label kernel override exceeds shared memory");
   a.KC = KC;
   const int TP = T * P;
   a.ntiles = (a.n + TP - 1) / TP;
@@ -94,13 +89,6 @@ static int launch_gauss_label_p(dpmm_ctx* ctx, GaussLabelArgs a) {
 
 template <int D>
 static int launch_gauss_label(dpmm_ctx* ctx, GaussLabelArgs a) {
-#ifdef DPMM_EXPERIMENT
-  if constexpr (D == 32) {
-    const int p = env_int("DPMM_LABEL_P", LabelP<D>::P);
-    if (p == 1) return launch_gauss_label_p<D, 1>(ctx, a);
-    if (p == 4) return launch_gauss_label_p<D, 4>(ctx, a);
-  }
-#endif
   int rc = launch_gauss_label_p<D, LabelP<D>::P>(ctx, a);
   if constexpr (LabelP<D>::P > 1) {
     // the tile's slice of parr ([K][points]) is what limits K: one point per thread carries K up to DPMM_MAX_K
@@ -112,7 +100,7 @@ static int launch_gauss_label(dpmm_ctx* ctx, GaussLabelArgs a) {
 template <int D>
 static int launch_gauss_sublabel(dpmm_ctx* ctx, const SubLabelArgs& a, bool sample) {
   if constexpr (D % 4 == 0 && D >= 16 && D <= 48) {
-    if (sample && env_int("DPMM_SUBLABEL_P2", 1)) {
+    if (sample) {
       using C = GaussCfg<D>;
       const size_t sm = ((size_t)2 * 256 * C::DS + (size_t)SUBLABEL_SPAN * 2 * C::REC + a.K + 4) * 4;
       auto kern = gauss_sublabel2_kernel<D>;
