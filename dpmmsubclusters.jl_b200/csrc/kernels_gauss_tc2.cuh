@@ -38,7 +38,8 @@
 //   warps 2-5 / 6-9  epilogue (TMEM lane = point) of group 0/1, alternate tiles
 //   warps 10-13 gather: cp.async of the 128 rows of a tile into a 128B-swizzled K-major stage ring
 #pragma once
-#include "kernels_gauss_tc.cuh"
+#include "tcgen05.cuh"
+#include "kernels_gauss.cuh"   // gauss_finish
 #include "kernels_stats.cuh"   // cp_async16 / commit / wait_group
 
 #define T2_TILE 128

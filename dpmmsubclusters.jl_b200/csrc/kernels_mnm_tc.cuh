@@ -19,7 +19,7 @@
 // the pace until HBM does.
 #pragma once
 #include "common.cuh"
-#include "kernels_gauss_tc.cuh"  // tc:: PTX wrappers
+#include "tcgen05.cuh"
 
 #define MTC_TILE 128
 #define MTC_N 32                  // accumulator columns per tile (clusters, zero padded)

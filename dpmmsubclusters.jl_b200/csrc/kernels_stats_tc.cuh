@@ -26,7 +26,7 @@
 // range of the tile sequence, so there is no work list and no atomically fetched item; all roles walk
 // the same deterministic tile sequence.
 #pragma once
-#include "kernels_gauss_tc.cuh"
+#include "tcgen05.cuh"
 #include "kernels_stats.cuh"
 
 #define STC_D 32

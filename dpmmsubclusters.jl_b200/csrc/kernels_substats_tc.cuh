@@ -43,6 +43,7 @@
 // back-off in the waits of the non-critical warps (+2..+14 us), Philox on the gather warps (+15 us), three
 // tiles of gather in flight with a 5-slot ring (+9 us).
 #pragma once
+#include "kernels_gauss.cuh"   // gauss_finish
 #include "kernels_stats_tc.cuh"
 
 #define SS_D 32
