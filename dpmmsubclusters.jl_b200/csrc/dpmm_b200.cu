@@ -21,6 +21,7 @@
 #include "kernels_mnm_tc.cuh"
 #include "kernels_pack.cuh"
 #include "kernels_params.cuh"
+#include "kernels_params_mnm.cuh"
 #include "kernels_sort.cuh"
 #include "kernels_stats.cuh"
 #include "kernels_stats_tc.cuh"
@@ -49,16 +50,21 @@ static cudaError_t dev_grow_keep(T** p, size_t old_count, size_t new_count) {
   *p = q;
   return e;
 }
+// doubles per distribution of the posterior table
+static int post_doubles(const dpmm_ctx* c) {
+  return c->prior == DPMM_PRIOR_NIW ? NIW_POST_DOUBLES(c->D) : MNM_POST_DOUBLES(c->D);
+}
 static int ensure_tables(dpmm_ctx* ctx, int cap) {
   if (cap <= ctx->Kcap_tab) return 0;
   CK(cudaStreamSynchronize(ctx->stream));
   const int D = ctx->D, old = ctx->Kcap_tab;
-  const size_t rec3 = (size_t)3 * (1 + D + D * D), post3 = (size_t)3 * NIW_POST_DOUBLES(D);
+  const bool niw = ctx->prior == DPMM_PRIOR_NIW;
+  const size_t rec3 = (size_t)3 * (niw ? 1 + D + D * D : 1 + D), post3 = (size_t)3 * post_doubles(ctx);
   CK(dev_grow_keep(&ctx->ptab, old * rec3, cap * rec3));
   CK(dev_grow_keep(&ctx->ptab_alt, 0, cap * rec3));
   CK(dev_grow_keep(&ctx->post, old * post3, cap * post3));
   CK(dev_grow_keep(&ctx->post_alt, 0, cap * post3));
-  CK(dev_grow_keep(&ctx->lfac, (size_t)3 * old * D * D, (size_t)3 * cap * D * D));
+  if (niw) CK(dev_grow_keep(&ctx->lfac, (size_t)3 * old * D * D, (size_t)3 * cap * D * D));
   CK(dev_grow_keep(&ctx->pm_out, 0, (size_t)cap * 6 + (size_t)cap * cap + 2));
   CK(dev_grow_keep(&ctx->splittable_d, 0, (size_t)cap));
   CK(dev_grow_keep(&ctx->newof_d, 0, (size_t)cap));
@@ -585,7 +591,7 @@ extern "C" int dpmm_remove_empty(dpmm_ctx* ctx, const int64_t* pts_count, int32_
     CK(cudaStreamSynchronize(ctx->stream));
     memcpy(ctx->hstage, newof.data(), (size_t)kt_ * 4);
     CK(cudaMemcpyAsync(ctx->newof_d, ctx->hstage, (size_t)kt_ * 4, cudaMemcpyHostToDevice, ctx->stream));
-    const int rec3 = 3 * ctx->stats_rec, post3 = 3 * NIW_POST_DOUBLES(ctx->D);
+    const int rec3 = 3 * ctx->stats_rec, post3 = 3 * post_doubles(ctx);
     KernelTimer kt(ctx, TK_PARAMS, 2);
     table_gather_kernel<<<dim3(8, (unsigned)kt_), 256, 0, ctx->stream>>>(ctx->ptab, ctx->newof_d, kt_, rec3, ctx->ptab_alt);
     table_gather_kernel<<<dim3(8, (unsigned)kt_), 256, 0, ctx->stream>>>(ctx->post, ctx->newof_d, kt_, post3, ctx->post_alt);
@@ -817,6 +823,27 @@ extern "C" int dpmm_set_params_niw(dpmm_ctx* ctx, int32_t K, const float* mu, co
   return 0;
 }
 
+// Derive the sweep kernels' images from the [3K][D] log-probabilities in ctx->recs (the transposed table and, on the
+// tensor-core path, the TF32 split); logw / loglr are already in place.
+static int mnm_pack_launch(dpmm_ctx* ctx, int K) {
+  const int D = ctx->D;
+  const int KP = (K + MNM_KT - 1) / MNM_KT * MNM_KT;
+  const bool mtc = ctx->mtc_ok && K <= MTC_MAX_K;
+  MnmPackArgs pa{};
+  pa.D = D; pa.K = K; pa.KP = KP; pa.logp = ctx->recs; pa.logp_t = ctx->logp_t; pa.mtc_w = mtc ? ctx->mtc_w : nullptr;
+  const int64_t ne = std::max<int64_t>((int64_t)D * KP, mtc ? (int64_t)((D + 31) / 32) * MTC_N * 32 : 0);
+  {
+    KernelTimer kt(ctx, TK_PARAMS);
+    mnm_pack_kernel<<<(unsigned)std::min<int64_t>((ne + 255) / 256, (int64_t)ctx->sm_count * 4), 256, 0, ctx->stream>>>(pa);
+    CK(cudaGetLastError());
+  }
+  ctx->mtc_params = mtc;
+  ctx->K = K;
+  ctx->KP = KP;
+  ctx->params_set = true;
+  return 0;
+}
+
 extern "C" int dpmm_set_params_multinomial(dpmm_ctx* ctx, int32_t K, const float* log_p, const float* weights,
                                            const float* lr_weights) {
   NEED(ctx, DPMM_EINVAL, "ctx is NULL");
@@ -827,63 +854,22 @@ extern "C" int dpmm_set_params_multinomial(dpmm_ctx* ctx, int32_t K, const float
   int rc = ensure_k(ctx, K);
   if (rc) return rc;
   const int D = ctx->D;
-  const int KP = (K + MNM_KT - 1) / MNM_KT * MNM_KT;
   const size_t nrec = (size_t)3 * K;
-  const bool mtc = ctx->mtc_ok && K <= MTC_MAX_K;
-  const int NP = (D + 31) / 32;
-  const size_t wfl = mtc ? (size_t)3 * NP * MTC_N * 32 : 0;
-  const size_t bytes = (nrec * D + (size_t)D * KP + K + 2 * K + wfl) * sizeof(float);
+  const size_t bytes = (nrec * D + K + 2 * K) * sizeof(float);
   void* hs = nullptr;
   const int slot = upload_acquire(ctx, bytes, &hs);
   if (slot < 0) return slot;
   float* h_recs = (float*)hs;
-  float* h_t = h_recs + nrec * D;
-  float* h_logw = h_t + (size_t)D * KP;
+  float* h_logw = h_recs + nrec * D;
   float* h_loglr = h_logw + K;
-  float* h_ws = h_loglr + 2 * K;
   memcpy(h_recs, log_p, nrec * D * 4);
-  std::fill(h_t, h_t + (size_t)D * KP, 0.f);
-  for (int k = 0; k < K; ++k)
-    for (int d = 0; d < D; ++d) h_t[(size_t)d * KP + k] = log_p[(size_t)(3 * k) * D + d];
   common_weights(ctx, K, weights, lr_weights, h_logw, h_loglr);
-  ctx->mtc_params = false;
-  if (mtc) {
-    // alpha = a_hi + a_lo + a_lolo, every term exact in TF32 (10 explicit mantissa bits)
-    auto tf32 = [](float v) {
-      if (!std::isfinite(v)) return v;
-      uint32_t u;
-      memcpy(&u, &v, 4);
-      u += 0xFFFu + ((u >> 13) & 1u);
-      u &= 0xFFFFE000u;
-      float r;
-      memcpy(&r, &u, 4);
-      return r;
-    };
-    std::fill(h_ws, h_ws + wfl, 0.f);
-    for (int k = 0; k < K; ++k)
-      for (int dd = 0; dd < D; ++dd) {
-        const float al = log_p[(size_t)(3 * k) * D + dd];
-        const float hi = tf32(al);
-        const float r1 = std::isfinite(al) ? al - hi : 0.f;
-        const float lo = tf32(r1);
-        const float lolo = r1 - lo;
-        const int p = dd >> 5, c = dd & 31;
-        const float parts[3] = {hi, lo, lolo};
-        for (int sp = 0; sp < 3; ++sp) h_ws[(((size_t)sp * NP + p) * MTC_N + k) * 32 + c] = parts[sp];
-      }
-    CK(cudaMemcpyAsync(ctx->mtc_w, h_ws, wfl * 4, cudaMemcpyHostToDevice, ctx->stream));
-    ctx->mtc_params = true;
-  }
   CK(cudaMemcpyAsync(ctx->recs, h_recs, nrec * D * 4, cudaMemcpyHostToDevice, ctx->stream));
-  CK(cudaMemcpyAsync(ctx->logp_t, h_t, (size_t)D * KP * 4, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemcpyAsync(ctx->logw, h_logw, (size_t)K * 4, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemcpyAsync(ctx->loglr, h_loglr, (size_t)2 * K * 4, cudaMemcpyHostToDevice, ctx->stream));
   rc = upload_release(ctx, slot);
   if (rc) return rc;
-  ctx->K = K;
-  ctx->KP = KP;
-  ctx->params_set = true;
-  return 0;
+  return mnm_pack_launch(ctx, K);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1380,7 +1366,7 @@ extern "C" int dpmm_suff_stats(dpmm_ctx* ctx, const int64_t* indices, int32_t n_
 
 
 // ------------------------------------------------------------------------------------------------
-// device-side parameter step (NIW): SURVEY.md 8f-1
+// device-side parameter step (NIW and multinomial): SURVEY.md 8f-1
 // ------------------------------------------------------------------------------------------------
 extern "C" int dpmm_num_clusters(const dpmm_ctx* ctx) { return ctx ? keff(ctx) : 0; }
 
@@ -1427,10 +1413,46 @@ extern "C" int dpmm_set_hyper_niw(dpmm_ctx* ctx, double kappa, const double* m, 
   return ensure_tables(ctx, std::max(ctx->Kcap, 8));
 }
 
+extern "C" int dpmm_set_hyper_multinomial(dpmm_ctx* ctx, const float* alpha_prior, double alpha) {
+  NEED(ctx, DPMM_EINVAL, "ctx is NULL");
+  NEED(ctx->prior == DPMM_PRIOR_MULTINOMIAL, DPMM_ESTATE, "context was created with the NIW prior");
+  NEED(alpha_prior, DPMM_EINVAL, "alpha_prior is NULL");
+  NEED(alpha > 0, DPMM_EINVAL, "need alpha > 0");
+  CK(cudaSetDevice(ctx->device));
+  const int D = ctx->D;
+  std::vector<double> h(MNM_HYPER_DOUBLES(D));
+  double sa = 0.0;
+  for (int d = 0; d < D; ++d) {
+    NEED(std::isfinite(alpha_prior[d]) && alpha_prior[d] > 0.f, DPMM_EINVAL, "every alpha_prior[d] must be finite and > 0");
+    h[2 + d] = (double)alpha_prior[d];
+    sa += h[2 + d];
+  }
+  h[0] = sa;
+  h[1] = std::lgamma(sa);
+  if (!ctx->hyper_d) CK(cudaMalloc((void**)&ctx->hyper_d, h.size() * 8));
+  CK(cudaStreamSynchronize(ctx->stream));
+  CK(cudaMemcpy(ctx->hyper_d, h.data(), h.size() * 8, cudaMemcpyHostToDevice));
+  ctx->alpha = (double)(float)alpha;
+  ctx->dev_params = true;
+  return ensure_tables(ctx, std::max(ctx->Kcap, 8));
+}
+
+#define DPMM_NEED_HYPER(what) \
+  NEED(ctx->dev_params, DPMM_ESTATE, "dpmm_set_hyper_niw or dpmm_set_hyper_multinomial must precede " what)
+
 static size_t niw_post_smem(int D) { return ((size_t)D * (D + 1) + 2 * D) * sizeof(double); }
 
 // posterior + log marginal likelihood of the listed clusters (device list idx_d, or all m = K in order) from the table
 static int launch_post(dpmm_ctx* ctx, const int32_t* idx_d, int m, double* out) {
+  if (ctx->prior == DPMM_PRIOR_MULTINOMIAL) {
+    MnmPostArgs pa{};
+    pa.D = ctx->D; pa.rec = ctx->stats_rec; pa.hyper = ctx->hyper_d; pa.ptab = ctx->ptab; pa.idx_list = idx_d;
+    pa.post = ctx->post; pa.out = out;
+    KernelTimer kt(ctx, TK_PARAMS);
+    mnm_post_kernel<<<dim3((unsigned)m, 3), MNM_PARAM_THREADS, 0, ctx->stream>>>(pa);
+    CK(cudaGetLastError());
+    return 0;
+  }
   NiwPostArgs pa{};
   pa.D = ctx->D; pa.rec = ctx->stats_rec; pa.hyper = ctx->hyper_d; pa.ptab = ctx->ptab; pa.idx_list = idx_d;
   pa.post = ctx->post; pa.out = out;
@@ -1447,7 +1469,7 @@ extern "C" int dpmm_posterior_step(dpmm_ctx* ctx, const int64_t* indices, int32_
                                    double* merge_logml) {
   NEED(ctx, DPMM_EINVAL, "ctx is NULL");
   CK(cudaSetDevice(ctx->device));
-  NEED(ctx->dev_params, DPMM_ESTATE, "dpmm_set_hyper_niw must precede dpmm_posterior_step");
+  DPMM_NEED_HYPER("dpmm_posterior_step");
   const int rec = ctx->stats_rec;
   int m = 0;
   bool all = indices == nullptr;
@@ -1490,15 +1512,26 @@ extern "C" int dpmm_posterior_step(dpmm_ctx* ctx, const int64_t* indices, int32_
   if (want_merge) {
     NEED(k_merge <= ctx->Kcap_tab, DPMM_EINVAL, "k_merge exceeds the number of clusters");
     CK(cudaMemcpyAsync(ctx->splittable_d, splittable, (size_t)k_merge, cudaMemcpyHostToDevice, ctx->stream));
-    NiwMergeArgs ma{};
-    ma.D = ctx->D; ma.rec = rec; ma.K = k_merge; ma.hyper = ctx->hyper_d; ma.ptab = ctx->ptab;
-    ma.splittable = ctx->splittable_d; ma.out = merge_d;
-    const size_t sm = niw_post_smem(ctx->D);
-    if (sm > 48 * 1024) CK(cudaFuncSetAttribute(niw_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-    int rcf = side_fork(ctx);
-    if (rcf) return rcf;
-    ctx->launches += 1;
-    niw_merge_kernel<<<dim3((unsigned)k_merge, (unsigned)k_merge), 256, sm, ctx->side>>>(ma);
+    const dim3 grid((unsigned)k_merge, (unsigned)k_merge);
+    if (ctx->prior == DPMM_PRIOR_MULTINOMIAL) {
+      MnmMergeArgs ma{};
+      ma.D = ctx->D; ma.rec = rec; ma.K = k_merge; ma.hyper = ctx->hyper_d; ma.ptab = ctx->ptab;
+      ma.splittable = ctx->splittable_d; ma.out = merge_d;
+      int rcf = side_fork(ctx);
+      if (rcf) return rcf;
+      ctx->launches += 1;
+      mnm_merge_kernel<<<grid, MNM_PARAM_THREADS, 0, ctx->side>>>(ma);
+    } else {
+      NiwMergeArgs ma{};
+      ma.D = ctx->D; ma.rec = rec; ma.K = k_merge; ma.hyper = ctx->hyper_d; ma.ptab = ctx->ptab;
+      ma.splittable = ctx->splittable_d; ma.out = merge_d;
+      const size_t sm = niw_post_smem(ctx->D);
+      if (sm > 48 * 1024) CK(cudaFuncSetAttribute(niw_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+      int rcf = side_fork(ctx);
+      if (rcf) return rcf;
+      ctx->launches += 1;
+      niw_merge_kernel<<<grid, 256, sm, ctx->side>>>(ma);
+    }
     CK(cudaGetLastError());
   }
   int rc = launch_post(ctx, all ? nullptr : ctx->idx_list, m, ctx->pm_out);
@@ -1533,7 +1566,7 @@ extern "C" int dpmm_posterior_step(dpmm_ctx* ctx, const int64_t* indices, int32_
 extern "C" int dpmm_sample_params(dpmm_ctx* ctx, int32_t K, int32_t from_prior, int32_t unit_weights) {
   NEED(ctx, DPMM_EINVAL, "ctx is NULL");
   CK(cudaSetDevice(ctx->device));
-  NEED(ctx->dev_params, DPMM_ESTATE, "dpmm_set_hyper_niw must precede dpmm_sample_params");
+  DPMM_NEED_HYPER("dpmm_sample_params");
   NEED(K >= 1 && K <= DPMM_MAX_K, DPMM_ELIMIT, "K out of range");
   int rc = ensure_k(ctx, K);
   if (rc) return rc;
@@ -1544,7 +1577,7 @@ extern "C" int dpmm_sample_params(dpmm_ctx* ctx, int32_t K, int32_t from_prior, 
   ctx->pcall += 1;
   {   // the Dirichlet weights depend on the posterior table only: side stream, next to the draws and the packing
     WeightsArgs wa{};
-    wa.K = K; wa.D = D; wa.post = ctx->post; wa.stride = NIW_POST_DOUBLES(D); wa.alpha = ctx->alpha; wa.logw = ctx->logw;
+    wa.K = K; wa.D = D; wa.post = ctx->post; wa.stride = post_doubles(ctx); wa.alpha = ctx->alpha; wa.logw = ctx->logw;
     wa.loglr = ctx->loglr; wa.w_out = ctx->w_out; wa.lr_out = ctx->lr_out; wa.seed = ctx->seed; wa.call = ctx->pcall;
     wa.unit = unit_weights;
     rc = side_fork(ctx);
@@ -1552,6 +1585,19 @@ extern "C" int dpmm_sample_params(dpmm_ctx* ctx, int32_t K, int32_t from_prior, 
     ctx->launches += 1;
     dpmm_weights_kernel<<<1, 256, (size_t)(K + 1) * 8, ctx->side>>>(wa);
     CK(cudaGetLastError());
+  }
+  if (ctx->prior == DPMM_PRIOR_MULTINOMIAL) {
+    MnmDrawArgs da{};
+    da.D = D; da.hyper = ctx->hyper_d; da.post = ctx->post; da.logp = ctx->recs; da.seed = ctx->seed; da.call = ctx->pcall;
+    da.first = from_prior;
+    {
+      KernelTimer kt(ctx, TK_PARAMS);
+      mnm_draw_kernel<<<(unsigned)nrec, MNM_PARAM_THREADS, (size_t)D * sizeof(double), ctx->stream>>>(da);
+      CK(cudaGetLastError());
+    }
+    rc = mnm_pack_launch(ctx, K);
+    if (rc) return rc;
+    return side_join(ctx);
   }
   {
     NiwDrawArgs da{};
@@ -1571,7 +1617,7 @@ extern "C" int dpmm_sample_params(dpmm_ctx* ctx, int32_t K, int32_t from_prior, 
 extern "C" int dpmm_params_merge(dpmm_ctx* ctx, int64_t i, int64_t j) {
   NEED(ctx, DPMM_EINVAL, "ctx is NULL");
   CK(cudaSetDevice(ctx->device));
-  NEED(ctx->dev_params, DPMM_ESTATE, "dpmm_set_hyper_niw must precede dpmm_params_merge");
+  DPMM_NEED_HYPER("dpmm_params_merge");
   NEED(i >= 1 && j >= 1 && i != j && i <= ctx->Kcap_tab && j <= ctx->Kcap_tab, DPMM_EINVAL, "bad cluster pair");
   KernelTimer kt(ctx, TK_PARAMS);
   ptab_merge_kernel<<<1, 256, 0, ctx->stream>>>(ctx->ptab, ctx->stats_rec, (int)i - 1, (int)j - 1);
@@ -1583,6 +1629,7 @@ extern "C" int dpmm_get_params_niw(dpmm_ctx* ctx, int32_t K, float* mu, double* 
                                    float* lr_weights) {
   NEED(ctx, DPMM_EINVAL, "ctx is NULL");
   CK(cudaSetDevice(ctx->device));
+  NEED(ctx->prior == DPMM_PRIOR_NIW, DPMM_ESTATE, "context was created with the multinomial prior");
   NEED(ctx->dev_params && ctx->params_set && K == ctx->K, DPMM_ESTATE, "no device-sampled parameters for this K");
   const int D = ctx->D;
   const size_t nrec = (size_t)3 * K;
@@ -1590,6 +1637,18 @@ extern "C" int dpmm_get_params_niw(dpmm_ctx* ctx, int32_t K, float* mu, double* 
   if (mu) CK(cudaMemcpy(mu, ctx->raw_params, nrec * D * 4, cudaMemcpyDeviceToHost));
   if (logdet) CK(cudaMemcpy(logdet, ctx->raw_params + nrec * D + nrec * D * D, nrec * 4, cudaMemcpyDeviceToHost));
   if (lfac) CK(cudaMemcpy(lfac, ctx->lfac, nrec * D * D * 8, cudaMemcpyDeviceToHost));
+  if (weights) CK(cudaMemcpy(weights, ctx->w_out, (size_t)K * 4, cudaMemcpyDeviceToHost));
+  if (lr_weights) CK(cudaMemcpy(lr_weights, ctx->lr_out, (size_t)2 * K * 4, cudaMemcpyDeviceToHost));
+  return 0;
+}
+
+extern "C" int dpmm_get_params_multinomial(dpmm_ctx* ctx, int32_t K, float* log_p, float* weights, float* lr_weights) {
+  NEED(ctx, DPMM_EINVAL, "ctx is NULL");
+  CK(cudaSetDevice(ctx->device));
+  NEED(ctx->prior == DPMM_PRIOR_MULTINOMIAL, DPMM_ESTATE, "context was created with the NIW prior");
+  NEED(ctx->dev_params && ctx->params_set && K == ctx->K, DPMM_ESTATE, "no device-sampled parameters for this K");
+  CK(cudaStreamSynchronize(ctx->stream));
+  if (log_p) CK(cudaMemcpy(log_p, ctx->recs, (size_t)3 * K * ctx->D * 4, cudaMemcpyDeviceToHost));
   if (weights) CK(cudaMemcpy(weights, ctx->w_out, (size_t)K * 4, cudaMemcpyDeviceToHost));
   if (lr_weights) CK(cudaMemcpy(lr_weights, ctx->lr_out, (size_t)2 * K * 4, cudaMemcpyDeviceToHost));
   return 0;
@@ -1661,6 +1720,63 @@ extern "C" int dpmm_predict_niw(dpmm_ctx* ctx, int32_t K, const float* u, const 
   CKP(cudaStreamSynchronize(ctx->stream));
 #undef CKP
   for (int64_t i = 0; i < ctx->n; ++i) labels[i] = (int64_t)h[i] + 1;
+  cleanup();
+  return 0;
+}
+
+extern "C" int dpmm_predict_multinomial(dpmm_ctx* ctx, int32_t K, const double* logp, const float* logw,
+                                        int64_t* labels, float* probs) {
+  NEED(ctx && logp && logw && labels, DPMM_EINVAL, "NULL argument");
+  NEED(ctx->prior == DPMM_PRIOR_MULTINOMIAL, DPMM_ESTATE, "context was created with the NIW prior");
+  NEED(K >= 1 && K <= DPMM_MAX_K, DPMM_ELIMIT, "K out of range");
+  CK(cudaSetDevice(ctx->device));
+  const int D = ctx->D;
+  const int64_t n = ctx->n;
+  // as many clusters per tile as shared memory holds (a D = 1024 row takes 8 KB)
+  const int KC = std::max(1, std::min(K, ctx->smem_optin / (D * 8)));
+  const size_t sm = (size_t)KC * D * 8;
+  double* dlp = nullptr;
+  float* dlw = nullptr;
+  float* dscore = nullptr;
+  int32_t* dlab = nullptr;
+  auto cleanup = [&]() {
+    if (dlp) cudaFree(dlp);
+    if (dlw) cudaFree(dlw);
+    if (dscore) cudaFree(dscore);
+    if (dlab) cudaFree(dlab);
+  };
+#define CKP(call)                                                                                        \
+  do {                                                                                                   \
+    cudaError_t e__ = (call);                                                                            \
+    if (e__ != cudaSuccess) {                                                                            \
+      cleanup();                                                                                         \
+      return fail(ctx, DPMM_ECUDA, std::string(#call) + ": " + cudaGetErrorString(e__));                \
+    }                                                                                                    \
+  } while (0)
+  CKP(cudaMalloc((void**)&dlp, (size_t)K * D * 8));
+  CKP(cudaMalloc((void**)&dlw, (size_t)K * 4));
+  CKP(cudaMalloc((void**)&dscore, (size_t)n * K * 4));
+  CKP(cudaMalloc((void**)&dlab, (size_t)n * 4));
+  CKP(cudaMemcpyAsync(dlp, logp, (size_t)K * D * 8, cudaMemcpyHostToDevice, ctx->stream));
+  CKP(cudaMemcpyAsync(dlw, logw, (size_t)K * 4, cudaMemcpyHostToDevice, ctx->stream));
+  MnmScoreArgs sa{};
+  sa.x = ctx->x; sa.n = n; sa.D = D; sa.K = K; sa.KC = KC; sa.logp = dlp; sa.logw = dlw; sa.score = dscore;
+  if (sm > 48 * 1024) CKP(cudaFuncSetAttribute(mnm_score_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+  {
+    KernelTimer kt(ctx, TK_LABEL, 2);
+    const unsigned gx = (unsigned)std::min<int64_t>((n + 7) / 8, (int64_t)ctx->sm_count * 8);
+    mnm_score_kernel<<<dim3(gx, (unsigned)((K + KC - 1) / KC)), 256, sm, ctx->stream>>>(sa);
+    CKP(cudaGetLastError());
+    mnm_predict_finish_kernel<<<(unsigned)std::min<int64_t>((n + 255) / 256, (int64_t)ctx->sm_count * 8), 256, 0,
+                                ctx->stream>>>(dscore, n, K, dlab, probs != nullptr);
+    CKP(cudaGetLastError());
+  }
+  std::vector<int32_t> h((size_t)n);
+  CKP(cudaMemcpyAsync(h.data(), dlab, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  if (probs) CKP(cudaMemcpyAsync(probs, dscore, (size_t)n * K * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  CKP(cudaStreamSynchronize(ctx->stream));
+#undef CKP
+  for (int64_t i = 0; i < n; ++i) labels[i] = (int64_t)h[i] + 1;
   cleanup();
   return 0;
 }

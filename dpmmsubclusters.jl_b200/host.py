@@ -477,8 +477,12 @@ def _clusters_from_device(group, st, cfg):
     params = getattr(st, "params", None)
     if params is not None and params[0].shape[0] != K:
         params = None                                     # K changed after the parameters were fetched (mid-run checkpoint)
+    niw = isinstance(hyper, P.niw_hyperparams)
     if params is not None:
-        mu, lfac, logdet, w, lr = params
+        if niw:
+            mu, lfac, logdet, w, lr = params
+        else:
+            log_p, w, lr = params
     else:
         # no sampled parameters at hand: the posterior's centre stands in.  group_step re-draws every
         # distribution and weight before anything reads them (sample_clusters!, :659), so these never reach a sweep.
@@ -489,9 +493,15 @@ def _clusters_from_device(group, st, cfg):
     for k in range(K):
         cps = []
         for s_ in range(3):
-            ss = P.make_suff_stats(hyper, counts[k, s_], sum_x[k, s_], sum_xx[k, s_])
+            ss = P.make_suff_stats(hyper, counts[k, s_], sum_x[k, s_], None if sum_xx is None else sum_xx[k, s_])
             post = P.calc_posterior(hyper, ss)
-            if params is not None:
+            if not niw:
+                if params is not None:
+                    dist = P.multinomial_dist(log_p[k, s_].copy())
+                else:
+                    a = post.α.astype(np.float64)
+                    dist = P.multinomial_dist(np.log(a / a.sum()).astype(F32))
+            elif params is not None:
                 L = np.tril(lfac[k, s_])
                 inv = L @ L.T
                 with np.errstate(all="ignore"):
@@ -515,8 +525,9 @@ def dp_parallel(all_data, local_hyper_params=None, α_param=None, iters=100, ini
                 save_path=None, save_file_prefix="checkpoint_", model_save_interval=1000):
     """dp_parallel :121-157.  `sweep_factory`, `shard`, `comm`, `device`, `device_params` have no reference
     counterpart: they select the device / inject a test double / attach the multi-GPU communicator / choose
-    where the parameter step runs (default: on the device for the NIW prior, SURVEY 8f-1; False = the Python
-    mirror of the reference's master functions below)."""
+    where the parameter step runs (default: on the device for the NIW prior, SURVEY 8f-1, and on the host for the
+    multinomial prior, which takes the device with device_params=True; False = the Python mirror of the reference's
+    master functions below)."""
     if isinstance(all_data, (str, os.PathLike)):
         return dp_parallel_params_file(str(all_data), verbose=verbose, gt=gt, sweep_factory=sweep_factory, shard=shard,
                                        comm=comm, device=device, device_params=device_params)
@@ -549,8 +560,9 @@ def _run_from_settings(all_data, local_hyper_params, α_param, cfg, seed, sweep_
     sw = dp_model.group.sweep
     if comm is not None:
         sw.comm_init(*comm)
-    if device_params is None:
-        device_params = os.environ.get("DPMM_DEVICE_PARAMS", "1") != "0"
+    niw = isinstance(local_hyper_params, P.niw_hyperparams)
+    if device_params is None:                              # (multinomial: the host loop unless asked for explicitly)
+        device_params = niw and os.environ.get("DPMM_DEVICE_PARAMS", "1") != "0"
     first_iter = 1
     if restored is not None:                               # create_model_from_saved_data, ds.jl:89-92; :437-439
         grp, it = restored
@@ -559,7 +571,7 @@ def _run_from_settings(all_data, local_hyper_params, α_param, cfg, seed, sweep_
         dp_model.group.local_clusters = grp["local_clusters"]
         dp_model.group.weights = grp["weights"]
         first_iter = it + 1
-    if device_params and isinstance(local_hyper_params, P.niw_hyperparams) and hasattr(sw, "sample_params"):
+    if device_params and hasattr(sw, "sample_params"):
         from . import host_device as HD
         st, iter_count, nmi, ll, kh = HD.run_model_device(dp_model, cfg, rng, normalized_mutual_info, first_iter=first_iter,
                                                           resume=restored is not None)
@@ -642,14 +654,26 @@ def fit(all_data, *args, iters=100, init_clusters=1, seed=None, verbose=False, s
 
 def predict(dp_model, data, device=0, on_device=None):
     """predict / predict_points :23-40, :532-537: posterior-predictive hard labels + probabilities.
-    NIW models run on the GPU (dpmm_predict_niw: Student-t densities, argmax and softmax per point; the host
-    prepares the K factors); on_device=False, or a multinomial model, takes the NumPy formulas below."""
+    NIW models run on the GPU by default (dpmm_predict_niw: Student-t densities, argmax and softmax per point; the
+    host prepares the K factors); multinomial models do with on_device=True (dpmm_predict_multinomial: the host
+    prepares log(alpha'/sum alpha') in Float64).  on_device=False, or a multinomial model by default, takes the NumPy
+    formulas below."""
     data = np.asarray(data, F32)
     cl = dp_model.group.local_clusters
     posts = [c.cluster_params.cluster_params.posterior_hyperparams for c in cl]
     w = np.asarray(dp_model.group.weights, F32)
+    mnm = bool(posts) and isinstance(posts[0], P.multinomial_hyper)
     if on_device is None:
-        on_device = os.environ.get("DPMM_DEVICE_PREDICT", "1") != "0"
+        on_device = not mnm and os.environ.get("DPMM_DEVICE_PREDICT", "1") != "0"
+    if on_device and mnm and isinstance(dp_model.group.sweep, GpuSweep):
+        logp = np.stack([np.log(a / a.sum()) for a in (p.α.astype(np.float64) for p in posts)])   # posterior_predictive
+        with np.errstate(divide="ignore"):
+            lw = np.log(w)
+        g = GpuSweep(data, MULTINOMIAL, device=device)
+        try:
+            return g.predict_multinomial(logp, lw)
+        finally:
+            g.close()
     if on_device and posts and isinstance(posts[0], P.niw_hyperparams) and isinstance(dp_model.group.sweep, GpuSweep):
         D, K = data.shape[0], len(posts)
         u = np.zeros((K, D, D)); mu = np.zeros((K, D)); tc = np.zeros(K); dfs = np.zeros(K)

@@ -163,13 +163,18 @@ class GpuSweep:
                                           _ptr(sum_xx, C.c_double)))
         return counts, sum_x, sum_xx
 
-    # ---- device-side parameter step (NIW) ----
+    # ---- device-side parameter step ----
     def set_hyper_niw(self, kappa, m, nu, psi, alpha):
         m = np.ascontiguousarray(m, np.float64).reshape(-1)
         psi = np.ascontiguousarray(psi, np.float64)
         assert m.shape == (self.D,) and psi.shape == (self.D, self.D)
         self._ck(self.lib.dpmm_set_hyper_niw(self.h, float(kappa), _ptr(m, C.c_double), float(nu), _ptr(psi, C.c_double),
                                              float(alpha)))
+
+    def set_hyper_multinomial(self, alpha_prior, alpha):
+        a = np.ascontiguousarray(alpha_prior, np.float32).reshape(-1)
+        assert a.shape == (self.D,)
+        self._ck(self.lib.dpmm_set_hyper_multinomial(self.h, _ptr(a, C.c_float), float(alpha)))
 
     def posterior_step(self, indices=None, splittable=None, from_table=False, fetch=True):
         """Statistics (unless from_table) -> table -> posteriors.  Returns (counts [m,3] i64, logml [m,3] f64,
@@ -211,6 +216,15 @@ class GpuSweep:
                                               _ptr(w, C.c_float), _ptr(lr, C.c_float)))
         return mu, lf, ld, w, lr
 
+    def get_params_multinomial(self, K):
+        """(log_p [K,3,D] f32, weights [K] f32, lr [K,2] f32)."""
+        lp = np.empty((K, 3, self.D), np.float32)
+        w = np.empty(K, np.float32)
+        lr = np.empty((K, 2), np.float32)
+        self._ck(self.lib.dpmm_get_params_multinomial(self.h, int(K), _ptr(lp, C.c_float), _ptr(w, C.c_float),
+                                                      _ptr(lr, C.c_float)))
+        return lp, w, lr
+
     def predict_niw(self, u, mu, tconst, df, want_probs=True):
         """Posterior-predictive labels (and probabilities) of this context's points; see dpmm_predict_niw."""
         u = np.ascontiguousarray(u, np.float32); mu = np.ascontiguousarray(mu, np.float32)
@@ -221,6 +235,17 @@ class GpuSweep:
         probs = np.empty((self.n, K), np.float32) if want_probs else None
         self._ck(self.lib.dpmm_predict_niw(self.h, K, _ptr(u, C.c_float), _ptr(mu, C.c_float), _ptr(tconst, C.c_float),
                                            _ptr(df, C.c_float), _ptr(labels, C.c_int64), _ptr(probs, C.c_float)))
+        return labels, probs
+
+    def predict_multinomial(self, logp, logw, want_probs=True):
+        """Posterior-predictive labels (and probabilities) of this context's points; see dpmm_predict_multinomial."""
+        logp = np.ascontiguousarray(logp, np.float64); logw = np.ascontiguousarray(logw, np.float32)
+        K = logp.shape[0]
+        assert logp.shape == (K, self.D) and logw.shape == (K,)
+        labels = np.empty(self.n, np.int64)
+        probs = np.empty((self.n, K), np.float32) if want_probs else None
+        self._ck(self.lib.dpmm_predict_multinomial(self.h, K, _ptr(logp, C.c_double), _ptr(logw, C.c_float),
+                                                   _ptr(labels, C.c_int64), _ptr(probs, C.c_float)))
         return labels, probs
 
     # ---- smart splits (smart_cluster_init! local_clusters_actions.jl:555-623) ----

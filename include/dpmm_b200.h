@@ -125,17 +125,20 @@ int dpmm_suff_stats(dpmm_ctx* ctx, const int64_t* indices, int32_t n_indices, in
  * dpmm_suff_stats(indices = NULL) result.  With indices == NULL, n_indices must be 0 or exactly this. */
 int dpmm_num_clusters(const dpmm_ctx* ctx);
 
-/* ---- device-side parameter step (NIW; SURVEY 8f-1) --------------------------------------------
- * Optional: the host may keep sampling parameters itself (dpmm_set_params_niw).  With these calls the
- * per-iteration master work that scales with K D^3 runs next to the statistics:
- *   calc_posterior / log_marginal_likelihood   src/priors/niw.jl:20-31, 53-62
- *   sample_distribution                        src/priors/niw.jl:34-40
+/* ---- device-side parameter step (NIW and multinomial; SURVEY 8f-1) ----------------------------
+ * Optional: the host may keep sampling parameters itself (dpmm_set_params_*).  With these calls the
+ * per-iteration master work that scales with K D^3 (NIW) or K D (multinomial) runs next to the statistics:
+ *   calc_posterior / log_marginal_likelihood   src/priors/niw.jl:20-31, 53-62; multinomial_prior.jl:16-21, 34-39
+ *   sample_distribution                        src/priors/niw.jl:34-40; multinomial_prior.jl:23-25
  *   sample_cluster_params / sample_clusters!   src/shared_actions.jl:41-66, src/local_clusters_actions.jl:417-437
  *   should_merge! (the merged log marginal)    src/shared_actions.jl:21-38
  * The host keeps the Hastings accept / reject decisions on 3K scalars (+ the K x K merge table). */
 
 /* niw_hyperparams (niw.jl:6-11: kappa, m[D], nu, psi[D][D]) and the concentration alpha (ds.jl:9). */
 int dpmm_set_hyper_niw(dpmm_ctx* ctx, double kappa, const double* m, double nu, const double* psi, double alpha);
+/* multinomial_hyper (multinomial_prior.jl:6-8: alpha_prior float32 [D], every entry finite and > 0) and the
+ * concentration alpha > 0 (ds.jl:9).  DPMM_ESTATE on an NIW context. */
+int dpmm_set_hyper_multinomial(dpmm_ctx* ctx, const float* alpha_prior, double alpha);
 /* update_suff_stats_posterior! (local_clusters_actions.jl:206-254) kept on the device: statistics of the
  * listed clusters (NULL = all) -> all-reduce -> persistent table -> posterior hyper-parameters and log
  * marginal likelihoods of {cluster, left, right}.  from_table != 0: skip the statistics and re-evaluate the
@@ -149,7 +152,7 @@ int dpmm_posterior_step(dpmm_ctx* ctx, const int64_t* indices, int32_t n_indices
 /* sample_clusters! + broadcast_cluster_params (:417-437, :518-549) on the device: draw the 3K distributions
  * from the posterior table (from_prior != 0: from the prior), the sub-cluster weights Dirichlet(N_l + a/2,
  * N_r + a/2) and the mixture weights Dirichlet(N_1..N_K, a) (unit_weights != 0: 1/K, as
- * init_first_clusters!, dp-parallel-sampling.jl:77), and pack them for the sweep.  Replaces dpmm_set_params_niw. */
+ * init_first_clusters!, dp-parallel-sampling.jl:77), and pack them for the sweep.  Replaces dpmm_set_params_*. */
 int dpmm_sample_params(dpmm_ctx* ctx, int32_t k, int32_t from_prior, int32_t unit_weights);
 /* merge_clusters_to_splittable (shared_actions.jl:12-18) on the statistics table: cluster i <- {i + j, i, j},
  * cluster j <- empty (1-based).  Follow with dpmm_posterior_step(from_table = 1) for i. */
@@ -158,6 +161,9 @@ int dpmm_params_merge(dpmm_ctx* ctx, int64_t i, int64_t j);
  * invSigma = L L'), logdet float32 [3K] (log det Sigma), weights float32 [K], lr_weights float32 [K][2]. */
 int dpmm_get_params_niw(dpmm_ctx* ctx, int32_t k, float* mu, double* lfac, float* logdet, float* weights,
                         float* lr_weights);
+/* The parameters of the last dpmm_sample_params of a multinomial context: log_p float32 [3K][D]
+ * (multinomial_dist.alpha), weights float32 [K], lr_weights float32 [K][2].  Each output may be NULL. */
+int dpmm_get_params_multinomial(dpmm_ctx* ctx, int32_t k, float* log_p, float* weights, float* lr_weights);
 
 /* predict / predict_points (src/dp-parallel-sampling.jl:509-537, src/local_clusters_actions.jl:23-40) for the
  * points of THIS context under K NIW posterior predictives (multivariate Student-t, niw.jl:68-76):
@@ -167,6 +173,12 @@ int dpmm_get_params_niw(dpmm_ctx* ctx, int32_t k, float* mu, double* lfac, float
  * first argmax); probs: float32 [n][K] softmax over k, or NULL. */
 int dpmm_predict_niw(dpmm_ctx* ctx, int32_t k, const float* u, const float* mu, const float* tconst,
                      const float* df, int64_t* labels, float* probs);
+/* The same for K multinomial posterior predictives (multinomial_prior.jl:45-48):
+ *   parr[i,k] = fl32(logp_k' x_i) + logw[k]   (dot product in float64, the sum in float32)
+ * logp double [K][D] = log(alpha'_k / sum alpha'_k), logw float32 [K] = log of the mixture weights.  labels: int64 [n]
+ * (1-based first argmax, NaN counts as maximal); probs: float32 [n][K] softmax over k (NaN as -Inf), or NULL. */
+int dpmm_predict_multinomial(dpmm_ctx* ctx, int32_t k, const double* logp, const float* logw, int64_t* labels,
+                             float* probs);
 
 /* ---- relabelling after split / merge / compaction ------------------------------------------- */
 

@@ -127,7 +127,7 @@ apply_merge!(c::Ctx, idx::Vector{Int64}, new_idx::Vector{Int64}) = check(ccall((
 remove_empty!(c::Ctx, pts_count::Vector{Int64}) = check(ccall((:dpmm_remove_empty, lib), Cint,
     (Ptr{Cvoid}, Ptr{Int64}, Int32), c.ptr, pts_count, length(pts_count)), c.ptr)
 
-# ---- device-side parameter step (NIW; include/dpmm_b200.h "device-side parameter step") ------------------
+# ---- device-side parameter step (NIW and multinomial; include/dpmm_b200.h "device-side parameter step") ----
 # With these the master keeps only the Hastings decisions: posterior hyper-parameters, log marginal
 # likelihoods, the 3K posterior draws and the Dirichlet weights are produced next to the statistics.
 
@@ -138,6 +138,13 @@ function set_hyper!(c::Ctx, κ::Real, m::Vector{Float64}, ν::Real, ψ::Matrix{F
     GC.@preserve m ψ check(ccall((:dpmm_set_hyper_niw, lib), Cint,
         (Ptr{Cvoid}, Cdouble, Ptr{Cdouble}, Cdouble, Ptr{Cdouble}, Cdouble), c.ptr, κ, m, ν, ψ, α), c.ptr)
 end
+
+"""
+    set_hyper!(c, h::multinomial_hyper, α)   (multinomial_prior.jl:6-8, ds.jl:9)
+"""
+set_hyper!(c::Ctx, α_prior::Vector{Float32}, α::Real) =
+    GC.@preserve α_prior check(ccall((:dpmm_set_hyper_multinomial, lib), Cint,
+        (Ptr{Cvoid}, Ptr{Cfloat}, Cdouble), c.ptr, α_prior, α), c.ptr)
 
 """
     posterior_step(c, indices; splittable=nothing, from_table=false) -> (counts[3,m], logml[3,m], merge[K,K] or nothing)
@@ -175,6 +182,28 @@ function get_params(c::Ctx, K::Integer)
     GC.@preserve mu lf ld w lr check(ccall((:dpmm_get_params_niw, lib), Cint,
         (Ptr{Cvoid}, Int32, Ptr{Cfloat}, Ptr{Cdouble}, Ptr{Cfloat}, Ptr{Cfloat}, Ptr{Cfloat}), c.ptr, K, mu, lf, ld, w, lr), c.ptr)
     mu, lf, ld, w, lr
+end
+
+"(log_p[D,3,K] = multinomial_dist.α of the 3K distributions, weights[K], lr[2,K])"
+function get_params_multinomial(c::Ctx, K::Integer)
+    lp = Array{Float32}(undef, c.d, 3, K); w = Vector{Float32}(undef, K); lr = Array{Float32}(undef, 2, K)
+    GC.@preserve lp w lr check(ccall((:dpmm_get_params_multinomial, lib), Cint,
+        (Ptr{Cvoid}, Int32, Ptr{Cfloat}, Ptr{Cfloat}, Ptr{Cfloat}), c.ptr, K, lp, w, lr), c.ptr)
+    lp, w, lr
+end
+
+"""
+    predict_multinomial(c, logp::Matrix{Float64}, logw::Vector{Float32}) -> (labels[n], probs[K,n])
+
+predict_points (local_clusters_actions.jl:23-40) on this context's points: `logp[:, k] = log.(α′ₖ ./ sum(α′ₖ))`
+(multinomial_prior.jl:45-48), `logw = log.(weights)`.
+"""
+function predict_multinomial(c::Ctx, logp::Matrix{Float64}, logw::Vector{Float32})
+    K = length(logw)
+    labels = Vector{Int64}(undef, c.n); probs = Array{Float32}(undef, K, c.n)
+    GC.@preserve logp logw labels probs check(ccall((:dpmm_predict_multinomial, lib), Cint,
+        (Ptr{Cvoid}, Int32, Ptr{Cdouble}, Ptr{Cfloat}, Ptr{Int64}, Ptr{Cfloat}), c.ptr, K, logp, logw, labels, probs), c.ptr)
+    labels, probs
 end
 
 # ---- host-type shim ------------------------------------------------------------------------------------
