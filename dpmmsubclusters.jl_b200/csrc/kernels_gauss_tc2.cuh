@@ -10,7 +10,7 @@
 // few almost every point keeps its label, so the pivot is the cluster that decides the draw, and because it
 // is uniform over the tile everything below is warp-uniform:
 //
-//  0. CENTRE: the gather warps shift the tile by the pivot's mean in shared memory, z = x - mu_p.  The TF32
+//  0. CENTRE: the gather warps shift the tile by the pivot's mean, z = x - mu_p.  The TF32
 //     error of everything below is proportional to |z| (the spread of a cluster), not to |x|.
 //  1. PIVOT (tcgen05, kind::tf32): Y_p = Z U_p' for the full factor of the pivot (D columns).
 //     q~_p = |y|^2 carries a bounded TF32 error, so it yields a LOWER bound of r_p (see kernels_gauss_tc.cuh).
@@ -36,7 +36,8 @@
 // Warp roles (384 threads, one CTA per SM, contiguous range of the tile sequence per CTA):
 //   warps 0/1   control of point-group 0/1 (pivot image staging + tcgen05.mma issue)
 //   warps 2-5 / 6-9  epilogue (TMEM lane = point) of group 0/1, alternate tiles
-//   warps 10-13 gather: cp.async of the 128 rows of a tile into a 128B-swizzled K-major stage ring
+//   warps 10-13 gather: the 128 rows of a tile into a 128B-swizzled K-major stage ring, centred -- at D = 32 through
+//               registers (one store per row chunk), at D = 64 (warps 10-11) by cp.async and centring in place
 #pragma once
 #include "tcgen05.cuh"
 #include "kernels_gauss.cuh"   // gauss_finish
@@ -752,57 +753,117 @@ __global__ void __launch_bounds__(T2_THREADS(D), 1) gauss_label_tc2_kernel(const
           idx[j] = p < wl.end ? __ldg(a.perm + p) : -1;
         }
       };
-      auto issue = [&](int s) {
-        uint8_t* dst0 = stage0 + (size_t)s * L.stage_bytes + (c >> 3) * 16384;
+      if constexpr (D == 32) {
+        // The rows go straight into registers and are stored once, centred (no landing copy in shared memory):
+        // tile li + 2 is loaded into the register set tile li has just been stored from.  Rows past the end of
+        // the tile load as exact zeros and are stored uncentred.
+        static_assert(PF == 2, "one register set per tile in flight: va, vb");
+        auto load_rows = [&](float4 (&v)[NJ]) {
 #pragma unroll
-        for (int j = 0; j < NJ; ++j) {
-          const int r = r0 + RS * j;
-          const bool ok = idx[j] >= 0;
-          cp_async16(dst0 + r * 128 + (((c & 7) ^ (r & 7)) << 4), a.x + (size_t)(ok ? idx[j] : 0) * D + 4 * c, ok ? 16 : 0);
-        }
-      };
-      load_idx();
-#pragma unroll
-      for (int q = 0; q < PF; ++q) {
-        if (q < nt) {
-          issue(q % NS);
+          for (int j = 0; j < NJ; ++j) {
+            const bool ok = idx[j] >= 0;
+            v[j] = ldg_nc16(a.x + (size_t)(ok ? idx[j] : 0) * D + 4 * c, ok);
+          }
+        };
+        float4 va[NJ], vb[NJ];
+        load_idx();
+        load_rows(va);
+        t2_advance(wl, seq);
+        if (1 < nt) {
+          load_idx();
+          load_rows(vb);
           t2_advance(wl, seq);
-          if (q + 1 < nt) load_idx();
         }
-        cp_async_commit();
-      }
-      for (int li = 0; li < nt; ++li) {
-        cp_async_wait_group<PF - 1>();
-        {   // centre this thread's chunks of the landed tile by the pivot's mean (rows beyond the tile stay zero)
+        if (2 < nt) load_idx();
+        auto tile = [&](int li, float4 (&v)[NJ]) {
           const int key = min(wc.key, K - 1);
           if (key != ckey) {
             ckey = key;
             cen = __ldg(reinterpret_cast<const float4*>(a.mu + (size_t)key * D) + c);
           }
-          uint8_t* base = stage0 + (size_t)(li % NS) * L.stage_bytes + (c >> 3) * 16384;
           const int nrow = wc.end - wc.pos;
+          t2_advance(wc, seq);
+#pragma unroll
+          for (int j = 0; j < NJ; ++j) {
+            if (r0 + RS * j < nrow) {
+              v[j].x -= cen.x; v[j].y -= cen.y; v[j].z -= cen.z; v[j].w -= cen.w;
+            }
+          }
+          tc::mbar_wait(&empty[li % NS], ((li / NS) & 1) ^ 1);
+          uint8_t* base = stage0 + (size_t)(li % NS) * L.stage_bytes;
 #pragma unroll
           for (int j = 0; j < NJ; ++j) {
             const int r = r0 + RS * j;
-            float4* q = reinterpret_cast<float4*>(base + r * 128 + (((c & 7) ^ (r & 7)) << 4));
-            float4 v = *q;
-            if (r < nrow) {
-              v.x -= cen.x; v.y -= cen.y; v.z -= cen.z; v.w -= cen.w;
-              *q = v;
-            }
+            *reinterpret_cast<float4*>(base + r * 128 + ((c ^ (r & 7)) << 4)) = v[j];
           }
-          t2_advance(wc, seq);
+          tc::fence_proxy_async();
+          tc::mbar_arrive(&full[li % NS]);
+          const int nx = li + PF;
+          if (nx < nt) {
+            load_rows(v);
+            t2_advance(wl, seq);
+            if (nx + 1 < nt) load_idx();
+          }
+        };
+        for (int li = 0; li < nt; li += 2) {
+          tile(li, va);
+          if (li + 1 < nt) tile(li + 1, vb);
         }
-        tc::fence_proxy_async();
-        tc::mbar_arrive(&full[li % NS]);
-        const int nx = li + PF;
-        if (nx < nt) {
-          tc::mbar_wait(&empty[nx % NS], ((nx / NS) & 1) ^ 1);
-          issue(nx % NS);
-          t2_advance(wl, seq);
-          if (nx + 1 < nt) load_idx();
+      } else {
+        // D = 64: the registers of two tiles in flight do not fit beside the rest of the kernel; cp.async lands
+        // the rows in the stage, where they are centred in place
+        auto issue = [&](int s) {
+          uint8_t* dst0 = stage0 + (size_t)s * L.stage_bytes + (c >> 3) * 16384;
+#pragma unroll
+          for (int j = 0; j < NJ; ++j) {
+            const int r = r0 + RS * j;
+            const bool ok = idx[j] >= 0;
+            cp_async16(dst0 + r * 128 + (((c & 7) ^ (r & 7)) << 4), a.x + (size_t)(ok ? idx[j] : 0) * D + 4 * c, ok ? 16 : 0);
+          }
+        };
+        load_idx();
+#pragma unroll
+        for (int q = 0; q < PF; ++q) {
+          if (q < nt) {
+            issue(q % NS);
+            t2_advance(wl, seq);
+            if (q + 1 < nt) load_idx();
+          }
+          cp_async_commit();
         }
-        cp_async_commit();
+        for (int li = 0; li < nt; ++li) {
+          cp_async_wait_group<PF - 1>();
+          {   // centre this thread's chunks of the landed tile by the pivot's mean (rows beyond the tile stay zero)
+            const int key = min(wc.key, K - 1);
+            if (key != ckey) {
+              ckey = key;
+              cen = __ldg(reinterpret_cast<const float4*>(a.mu + (size_t)key * D) + c);
+            }
+            uint8_t* base = stage0 + (size_t)(li % NS) * L.stage_bytes + (c >> 3) * 16384;
+            const int nrow = wc.end - wc.pos;
+#pragma unroll
+            for (int j = 0; j < NJ; ++j) {
+              const int r = r0 + RS * j;
+              float4* q = reinterpret_cast<float4*>(base + r * 128 + (((c & 7) ^ (r & 7)) << 4));
+              float4 v = *q;
+              if (r < nrow) {
+                v.x -= cen.x; v.y -= cen.y; v.z -= cen.z; v.w -= cen.w;
+                *q = v;
+              }
+            }
+            t2_advance(wc, seq);
+          }
+          tc::fence_proxy_async();
+          tc::mbar_arrive(&full[li % NS]);
+          const int nx = li + PF;
+          if (nx < nt) {
+            tc::mbar_wait(&empty[nx % NS], ((nx / NS) & 1) ^ 1);
+            issue(nx % NS);
+            t2_advance(wl, seq);
+            if (nx + 1 < nt) load_idx();
+          }
+          cp_async_commit();
+        }
       }
     }
   }

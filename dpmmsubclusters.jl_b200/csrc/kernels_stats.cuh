@@ -142,6 +142,18 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void cp_async_wait_group() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+// 16 bytes of read-only global memory into registers, not allocated in L1 (as cp.async.cg); zeros when !ok, as
+// cp_async16 with src_bytes = 0.  Volatile so that it is issued where it is written: the loads of a tile are made
+// a tile or two ahead of their use, and the compiler must not sink them to it.
+__device__ __forceinline__ float4 ldg_nc16(const void* gmem_src, bool ok) {
+  float4 v;
+  asm volatile("{\n .reg .pred p;\n setp.ne.b32 p, %5, 0;\n"
+               " mov.f32 %0, 0f00000000; mov.f32 %1, 0f00000000; mov.f32 %2, 0f00000000; mov.f32 %3, 0f00000000;\n"
+               " @p ld.global.nc.L1::no_allocate.v4.f32 {%0, %1, %2, %3}, [%4];\n}"
+               : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w)
+               : "l"(gmem_src), "r"((int)ok));
+  return v;
+}
 
 // K5: NIW.  Warp w of a CTA owns upper block u = g*WPG + w % WPG of S (g = block group of the work
 // unit; G > 1 only when S has more than 16 upper blocks, i.e. D > 40) and point slice w / WPG; lane l

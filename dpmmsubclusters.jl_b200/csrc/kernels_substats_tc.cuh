@@ -8,8 +8,9 @@
 //   create_sufficient_statistics (NIW)                         src/priors/niw.jl:42-51
 //
 // A tile = 128 consecutive positions of ONE cluster k in the label-sorted permutation `perm`.  Its rows
-// are gathered with cp.async into a thread-private landing ring, shifted by the cluster's centre c_k
-// (x - c_k is exact in Float32, see niw_pack_center) and split z = h + l with h = tf32(z).
+// are loaded into registers (two tiles ahead), shifted there by the cluster's centre c_k (x - c_k is exact
+// in Float32, see niw_pack_center), split z = h + l with h = tf32(z), and stored once: z into the raw ring,
+// l into the split panel.
 //
 //   GEMM1 (contraction over FEATURES; h | l as K-major A operands, 128B swizzle, M = 128 points, N = 64):
 //       Y = h Wh' + l Wh' + h Wl' - b,   W = [U_left; U_right] = Wh + Wl,   b = U_s (mu_s - c_k)
@@ -36,20 +37,21 @@
 // instruction every ~7-10 cycles -- so three groups work on tiles li mod 3; GEMM1 has six accumulator buffers so
 // that its issuer runs ahead of them.)
 //
-// What bounds it (ncu, round 2, profiles/r2j_ncu_summary.md): the shared-memory data pipe.  Per 128-point tile
-// the CUDA cores move ~1400 wavefronts (gather landing 128, centre/split 128 + 256, permuting copy 128 + 272,
-// drain) and the tensor core reads ~1030 (GEMM1: 13 k-steps x (4 KB + 2 KB); GEMM2: 17 x (2 KB + 1 KB)):
-// lsu 54 % + tc 33 % of the pipe's peak.  Measured on the way and rejected: suspend-time hints and nanosleep
-// back-off in the waits of the non-critical warps (+2..+14 us), Philox on the gather warps (+15 us), three
-// tiles of gather in flight with a 5-slot ring (+9 us).
+// What bounds it (ncu, round 2, profiles/r2j_ncu_summary.md): the shared-memory data pipe, then at lsu 54 % +
+// tc 33 % of its peak.  Per 128-point tile the CUDA cores move ~1150 wavefronts (centre/split stores 128 + 128,
+// permuting copy 128 + 272, drain; before the register-path gather also a cp.async landing of 128 and its
+// read-back of 128) and the tensor core reads ~1030 (GEMM1: 13 k-steps x (4 KB + 2 KB); GEMM2: 17 x (2 KB + 1 KB)).
+// The register-path gather took C2 from 86.9 to 84.1 us (B200, 1000 W).  Measured on the way and rejected:
+// suspend-time hints and nanosleep back-off in the waits of the non-critical warps (+2..+14 us), Philox on the
+// gather warps (+15 us), three tiles of gather in flight with a 5-slot ring (+9 us).
 #pragma once
 #include "kernels_gauss.cuh"   // gauss_finish
 #include "kernels_stats_tc.cuh"
 
 #define SS_D 32
 #define SS_TILE 128
-#define SS_RAW 5                         // ring of raw tiles: landing -> split -> permuting pass
-#define SS_PF 2                          // tiles of gather in flight
+#define SS_RAW 5                         // ring of raw (centred) tiles: split -> GEMM1 and permuting pass
+#define SS_PF 2                          // tiles of gather in flight (one register set each)
 #define SS_NG 3                          // GEMM1 epilogue groups (4 warps each), tile li -> group li % SS_NG
 #define SS_FLUSH 8                       // tiles per GEMM2 flush group (TMEM accumulates 1024 points between drains)
 #define SS_NTB 6                         // GEMM1 accumulator buffers (64 TMEM columns each), tile li -> buffer li % SS_NTB
@@ -220,13 +222,16 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
       // ======================= gather + shift + split =======================
       const int gtid = warp < 4 ? tid : tid - 608 + 128;   // 0..255
       const int c = gtid & 7, r0 = gtid >> 3;   // 16-byte chunk, first row; rows r0 + 32 j
-      // raw ring and l panels: K-major rows of 128 bytes with the 128B swizzle.  The raw slot is centred in
-      // place and IS the h operand of GEMM1: the tensor core reads the TF32 bits of z, i.e. h = trunc(z).
+      // raw ring and l panels: K-major rows of 128 bytes with the 128B swizzle.  The raw slot holds z and IS the
+      // h operand of GEMM1: the tensor core reads the TF32 bits of z, i.e. h = trunc(z).
       const uint32_t offk = (uint32_t)(r0 * 128 + ((c ^ (r0 & 7)) << 4));
       const uint32_t offr = offk;
       StcWalk wl, wc;
       stc_walk_init(wl, B, P, nkeys, t0, t1);
       wc = wl;
+      // The rows go straight into registers (no landing copy in shared memory): tile li + SS_PF is loaded into the
+      // register set that tile li has just been stored from, and the indices of a tile are loaded one tile ahead
+      // of its rows.  Rows past the end of the cluster load as exact zeros.
       int idx[4];
       auto load_idx = [&]() {
 #pragma unroll
@@ -235,66 +240,67 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
           idx[j] = p < wl.end ? __ldg(a.perm + p) : -1;
         }
       };
-      auto issue = [&](int s) {
-        uint8_t* dst = raw0 + (size_t)s * SS_PANEL + offr;
+      auto load_rows = [&](float4 (&v)[4]) {
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           const bool ok = idx[j] >= 0;
-          cp_async16(dst + j * 4096, a.x + (size_t)(ok ? idx[j] : 0) * SS_D + 4 * c, ok ? 16 : 0);
+          v[j] = ldg_nc16(a.x + (size_t)(ok ? idx[j] : 0) * SS_D + 4 * c, ok);
         }
       };
-#pragma unroll
-      for (int li = 0; li < SS_PF; ++li) {
-        if (li < nt) {
-          load_idx();
-          issue(li);
-          stc_advance<SS_FLUSH>(wl, B);
-        }
-        cp_async_commit();
+      float4 va[4], vb[4];
+      load_idx();   // (nt > 0 here)
+      load_rows(va);
+      stc_advance<SS_FLUSH>(wl, B);
+      if (1 < nt) {
+        load_idx();
+        load_rows(vb);
+        stc_advance<SS_FLUSH>(wl, B);
       }
       if (SS_PF < nt) load_idx();
       auto load_center = [&](int key) { return __ldg(reinterpret_cast<const float4*>(a.cen + (size_t)key * SS_D) + c); };
       int ckey = wc.key;
       float4 cen = load_center(ckey);
-      for (int li = 0; li < nt; ++li) {
+      auto tile = [&](int li, float4 (&v)[4]) {
         const int b = li & 1;
         if (wc.key != ckey) {
           ckey = wc.key;
           cen = load_center(ckey);
         }
         const int npts = wc.end - wc.pos;   // rows >= npts are zero padding
-        cp_async_wait_group<SS_PF - 1>();
-        uint8_t* src = raw0 + (size_t)(li % SS_RAW) * SS_PANEL + offr;
-        float4 v[4];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) v[j] = *reinterpret_cast<const float4*>(src + j * 4096);
-        float4 lo[4];
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           if (r0 + 32 * j < npts) {
             v[j].x -= cen.x; v[j].y -= cen.y; v[j].z -= cen.z; v[j].w -= cen.w;
           }
-          *reinterpret_cast<float4*>(src + j * 4096) = v[j];   // z, in place
-          lo[j].x = v[j].x - tc::trunc_tf32(v[j].x); lo[j].y = v[j].y - tc::trunc_tf32(v[j].y);
-          lo[j].z = v[j].z - tc::trunc_tf32(v[j].z); lo[j].w = v[j].w - tc::trunc_tf32(v[j].w);
         }
+        tc::mbar_wait(&rfree[li % SS_RAW], ((li / SS_RAW) & 1) ^ 1);   // the permuting pass of tile li - SS_RAW is done
+        uint8_t* zk = raw0 + (size_t)(li % SS_RAW) * SS_PANEL + offr;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) *reinterpret_cast<float4*>(zk + j * 4096) = v[j];
         tc::mbar_arrive(&landed[li % SS_RAW]);             // this thread's chunks of z are in shared memory
         tc::mbar_wait(&sfree[b], ((li >> 1) & 1) ^ 1);     // GEMM1 of tile li - 2 has read the l panel
         uint8_t* lk = split0 + (size_t)b * SS_PANEL + offk;
 #pragma unroll
-        for (int j = 0; j < 4; ++j) *reinterpret_cast<float4*>(lk + j * 4096) = lo[j];
+        for (int j = 0; j < 4; ++j) {
+          float4 lo;
+          lo.x = v[j].x - tc::trunc_tf32(v[j].x); lo.y = v[j].y - tc::trunc_tf32(v[j].y);
+          lo.z = v[j].z - tc::trunc_tf32(v[j].z); lo.w = v[j].w - tc::trunc_tf32(v[j].w);
+          *reinterpret_cast<float4*>(lk + j * 4096) = lo;
+        }
         tc::fence_proxy_async();
         tc::mbar_arrive(&ready[b]);
-        // next gather: tile li + PF goes into the slot of tile li + PF - RAW once its permuting pass is done
         const int ln = li + SS_PF;
         if (ln < nt) {
-          tc::mbar_wait(&rfree[ln % SS_RAW], ((ln / SS_RAW) & 1) ^ 1);
-          issue(ln % SS_RAW);
+          load_rows(v);
           stc_advance<SS_FLUSH>(wl, B);
           if (ln + 1 < nt) load_idx();
         }
-        cp_async_commit();
         stc_advance<SS_FLUSH>(wc, B);
+      };
+      static_assert(SS_PF == 2, "one register set per tile in flight: va, vb");
+      for (int li = 0; li < nt; li += 2) {
+        tile(li, va);
+        if (li + 1 < nt) tile(li + 1, vb);
       }
     } else if (warp == 4) {
       // ======================= GEMM1 issuer =======================
