@@ -7,6 +7,7 @@
 #include "philox.cuh"
 
 #define DPMM_MAX_K 1024
+#define DPMM_MNM_MAX_D 16384   // multinomial vocabulary: the device draw keeps one row of D doubles in shared memory
 
 // ---------------------------------------------------------------------------------------------
 // Packed FP32 pairs.  On sm_100a the FMA pipe reaches its peak FP32 rate only with the packed

@@ -204,7 +204,7 @@ extern "C" const char* dpmm_last_error(const dpmm_ctx* ctx) { return ctx ? ctx->
 extern "C" int dpmm_limits(int32_t* out3) {
   if (!out3) return DPMM_EINVAL;
   out3[0] = 64;
-  out3[1] = 1024;
+  out3[1] = DPMM_MNM_MAX_D;
   out3[2] = DPMM_MAX_K;
   return 0;
 }
@@ -225,7 +225,7 @@ extern "C" int dpmm_create(dpmm_ctx** out, const float* x, int64_t n_local, int3
     NEED(d <= 64, DPMM_ELIMIT, "NIW: D must be <= 64");
     while (!niw_dim_supported(dpad)) ++dpad;
   } else
-    NEED(d <= 1024, DPMM_ELIMIT, "multinomial: D must be <= 1024");
+    NEED(d <= DPMM_MNM_MAX_D, DPMM_ELIMIT, "multinomial: D must be <= 16384");
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
     return fail(nullptr, DPMM_ECUDA, "no CUDA device: libdpmm_b200 has no CPU fallback");
@@ -929,6 +929,22 @@ static int launch_label_tc2(dpmm_ctx* ctx, int final_iter, int nkeys) {
   return 0;
 }
 
+template <int TP>
+static int launch_mnm_label_stream(dpmm_ctx* ctx, MnmLabelArgs& a) {
+  const size_t sm = MnmStreamCfg<TP>::smem_bytes(a.K);
+  NEED(sm <= (size_t)ctx->smem_optin, DPMM_ELIMIT, "internal: multinomial streaming label kernel does not fit shared memory");
+  a.ntiles = (a.n + TP - 1) / TP;
+  CK(cudaFuncSetAttribute(mnm_label_stream_kernel<TP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+  int occ = 1;
+  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, mnm_label_stream_kernel<TP>, 256, sm));
+  occ = std::max(occ, 1);
+  const int64_t grid = std::min<int64_t>(a.ntiles, (int64_t)ctx->sm_count * occ);
+  KernelTimer kt(ctx, TK_LABEL);
+  mnm_label_stream_kernel<TP><<<(unsigned)grid, 256, sm, ctx->stream>>>(a);
+  CK(cudaGetLastError());
+  return 0;
+}
+
 static int run_sample_labels(dpmm_ctx* ctx, int final_iter, float* dump) {
   NEED(ctx->params_set, DPMM_ESTATE, "set_params must precede sample_labels");
   const int K = ctx->K;
@@ -1014,17 +1030,24 @@ static int run_sample_labels(dpmm_ctx* ctx, int final_iter, float* dump) {
     int T = 128;
     auto bytes = [&](int T_) { return ((size_t)a.D * a.KP + (size_t)T_ * a.DS + (size_t)K * T_) * 4 + (size_t)K * 4; };
     while (T > 32 && bytes(T) > (size_t)ctx->smem_optin) T /= 2;
-    NEED(bytes(T) <= (size_t)ctx->smem_optin, DPMM_ELIMIT, "multinomial: D*K too large for the shared-memory table");
-    a.ntiles = (a.n + T - 1) / T;
-    const size_t sm = bytes(T);
-    CK(cudaFuncSetAttribute(mnm_label_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-    int occ = 1;
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, mnm_label_kernel, T, sm));
-    occ = std::max(occ, 1);
-    const int64_t grid = std::min<int64_t>(a.ntiles, (int64_t)ctx->sm_count * occ);
-    KernelTimer kt(ctx, TK_LABEL);
-    mnm_label_kernel<<<(unsigned)grid, T, sm, ctx->stream>>>(a);
-    CK(cudaGetLastError());
+    if (bytes(T) <= (size_t)ctx->smem_optin) {
+      a.ntiles = (a.n + T - 1) / T;
+      const size_t sm = bytes(T);
+      CK(cudaFuncSetAttribute(mnm_label_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+      int occ = 1;
+      CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, mnm_label_kernel, T, sm));
+      occ = std::max(occ, 1);
+      const int64_t grid = std::min<int64_t>(a.ntiles, (int64_t)ctx->sm_count * occ);
+      KernelTimer kt(ctx, TK_LABEL);
+      mnm_label_kernel<<<(unsigned)grid, T, sm, ctx->stream>>>(a);
+      CK(cudaGetLastError());
+    } else {
+      // the table does not fit shared memory: stream it in feature panels (largest point tile whose parr slice fits)
+      int rc = MnmStreamCfg<128>::smem_bytes(K) <= (size_t)ctx->smem_optin ? launch_mnm_label_stream<128>(ctx, a)
+             : MnmStreamCfg<64>::smem_bytes(K) <= (size_t)ctx->smem_optin  ? launch_mnm_label_stream<64>(ctx, a)
+                                                                            : launch_mnm_label_stream<32>(ctx, a);
+      if (rc) return rc;
+    }
   }
   ctx->hist_valid = true;
   ctx->scan_valid = use_t2;   // the overflow kernel's last block already scanned the new histogram (width K)
@@ -1143,6 +1166,8 @@ static int run_sublabels(dpmm_ctx* ctx, bool sample, float* dump) {
     KernelTimer kt(ctx, TK_SUBLABEL);
     if (sample && ctx->D <= 128)
       mnm_sublabel2_kernel<<<grid, T, 0, ctx->stream>>>(a);
+    else if (sample && ctx->D > 1024)
+      mnm_sublabel_staged_kernel<<<grid, MNM_SLS_T, 0, ctx->stream>>>(a);
     else if (sample)
       mnm_sublabel_kernel<true><<<grid, T, 0, ctx->stream>>>(a);
     else
@@ -1276,11 +1301,12 @@ static int stats_compute(dpmm_ctx* ctx, const int64_t* indices, int32_t n_indice
     rc = niw_launch_stats(ctx, sa);
     if (rc) return rc;
   } else {
+    const auto kern = D > 32 * MNM_STATS_NREG ? mnm_stats_kernel<true> : mnm_stats_kernel<false>;
     int occ = 1;
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, mnm_stats_kernel, 256, 0));
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 256, 0));
     occ = std::max(occ, 1);
     KernelTimer kt(ctx, TK_STATS);
-    mnm_stats_kernel<<<ctx->sm_count * occ, 256, 0, ctx->stream>>>(sa);
+    kern<<<ctx->sm_count * occ, 256, 0, ctx->stream>>>(sa);
     CK(cudaGetLastError());
   }
   // with a communicator and mapped peer memory the packed statistics go straight into this rank's exchange
@@ -1592,7 +1618,9 @@ extern "C" int dpmm_sample_params(dpmm_ctx* ctx, int32_t K, int32_t from_prior, 
     da.first = from_prior;
     {
       KernelTimer kt(ctx, TK_PARAMS);
-      mnm_draw_kernel<<<(unsigned)nrec, MNM_PARAM_THREADS, (size_t)D * sizeof(double), ctx->stream>>>(da);
+      const size_t sm = (size_t)D * sizeof(double);
+      if (sm > 48 * 1024) CK(cudaFuncSetAttribute(mnm_draw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+      mnm_draw_kernel<<<(unsigned)nrec, MNM_PARAM_THREADS, sm, ctx->stream>>>(da);
       CK(cudaGetLastError());
     }
     rc = mnm_pack_launch(ctx, K);

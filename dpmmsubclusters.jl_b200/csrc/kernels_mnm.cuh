@@ -105,6 +105,136 @@ __global__ void mnm_label_kernel(const MnmLabelArgs a) {
     if (hs[k] != 0) atomicAdd(&a.hist[k], hs[k]);
 }
 
+// K3 for the shapes whose [D][KP] table does not fit shared memory beside a 32-point tile (large D and / or
+// large K).  A persistent CTA of 256 threads owns tiles of TP points; clusters go in chunks of KC = 16384 / TP,
+// and D in panels of MNM_SP features, double-buffered with cp.async: the table panel [MNM_SP][KC] straight
+// from logp_t, the X panel transposed to [MNM_SP][TP + 4] by 4-byte copies (a warp reads 8 features of 4 points:
+// whole 32-byte sectors, conflict-free stores).  Every thread owns an 8 x 8 block of (point, cluster) dot
+// products, and each one is the same sequential fmaf chain over ascending d as in mnm_label_kernel, then
+// __fadd_rn(acc, logw[k]), so both kernels produce identical bits.  Ragged panels load zeros for both operands
+// (fmaf(0, 0, acc) == acc: acc starts at +0 and never holds -0).  The [K][TP] slice of parr stays in shared
+// memory, and each point's draw runs on its column with the same helpers and stream keys.
+#define MNM_SP 16
+template <int TP>
+struct MnmStreamCfg {
+  static constexpr int KC = 16384 / TP;      // clusters per chunk: TP x KC = 256 threads x 64 products
+  static constexpr int XS = TP + 4;          // X panel row stride
+  static constexpr int WY = TP / 32;         // warps along the point axis (4 lanes x 4 points x 2 halves each)
+  static constexpr int WX = 8 / WY;
+  static constexpr size_t stage_floats = (size_t)MNM_SP * (KC + XS);
+  static size_t smem_bytes(int K) { return (2 * stage_floats + (size_t)K * TP) * 4 + (size_t)K * 4; }
+};
+
+template <int TP>
+__global__ void __launch_bounds__(256) mnm_label_stream_kernel(const MnmLabelArgs a) {
+  using C = MnmStreamCfg<TP>;
+  constexpr int KC = C::KC, XS = C::XS;
+  extern __shared__ __align__(16) float smem[];
+  float* stage = smem;                          // 2 x ([MNM_SP][KC] table | [MNM_SP][XS] X)
+  float* rs = smem + 2 * C::stage_floats;       // [K][TP]
+  int* hs = reinterpret_cast<int*>(rs + (size_t)a.K * TP);
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int tx = (warp % C::WX) * 8 + (lane & 7);   // cluster group: k0 + 4 tx + {0..3} and k0 + KC/2 + 4 tx + {0..3}
+  const int ty = (warp / C::WX) * 4 + (lane >> 3);  // point group:   4 ty + {0..3} and TP/2 + 4 ty + {0..3}
+  const int D = a.D;
+  const int npan = (D + MNM_SP - 1) / MNM_SP;
+  const int nsteps = npan * ((a.K + KC - 1) / KC);
+  for (int k = tid; k < a.K; k += 256) hs[k] = 0;
+
+  for (int64_t tile = blockIdx.x; tile < a.ntiles; tile += gridDim.x) {
+    const int64_t base = tile * TP;
+    const int npts = (int)min((int64_t)TP, a.n - base);
+    auto issue = [&](int s) {
+      float* ts = stage + (size_t)(s & 1) * C::stage_floats;
+      float* xs = ts + MNM_SP * KC;
+      const int d0 = (s % npan) * MNM_SP, k0 = (s / npan) * KC;
+#pragma unroll
+      for (int r = 0; r < MNM_SP * KC / 4 / 256; ++r) {
+        const int e = tid + 256 * r;
+        const int d = e / (KC / 4), k = k0 + 4 * (e % (KC / 4));
+        const bool ok = d0 + d < D && k < a.KP;
+        cp_async16(ts + d * KC + 4 * (e % (KC / 4)), ok ? a.logp_t + (size_t)(d0 + d) * a.KP + k : a.logp_t, ok ? 16 : 0);
+      }
+#pragma unroll
+      for (int r = 0; r < TP * MNM_SP / 256; ++r) {
+        const int d = (r & 1) * 8 + (lane & 7);
+        const int p = ((r >> 1) * 8 + warp) * 4 + (lane >> 3);
+        const bool ok = p < npts && d0 + d < D;
+        cp_async4(xs + d * XS + p, ok ? a.x + (base + p) * D + d0 + d : a.x, ok ? 4 : 0);
+      }
+      cp_async_commit();
+    };
+    float acc[8][8];
+    issue(0);
+    for (int s = 0; s < nsteps; ++s) {
+      if (s % npan == 0) {
+#pragma unroll
+        for (int i = 0; i < 8; ++i)
+#pragma unroll
+          for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
+      }
+      if (s + 1 < nsteps) {
+        issue(s + 1);
+        cp_async_wait_group<1>();
+      } else {
+        cp_async_wait_all();
+      }
+      __syncthreads();
+      const float* ts = stage + (size_t)(s & 1) * C::stage_floats;
+      const float* xs = ts + MNM_SP * KC;
+#pragma unroll
+      for (int d = 0; d < MNM_SP; ++d) {
+        const float4 x0 = *reinterpret_cast<const float4*>(xs + d * XS + 4 * ty);
+        const float4 x1 = *reinterpret_cast<const float4*>(xs + d * XS + TP / 2 + 4 * ty);
+        const float4 t0 = *reinterpret_cast<const float4*>(ts + d * KC + 4 * tx);
+        const float4 t1 = *reinterpret_cast<const float4*>(ts + d * KC + KC / 2 + 4 * tx);
+        const float xv[8] = {x0.x, x0.y, x0.z, x0.w, x1.x, x1.y, x1.z, x1.w};
+        const float tv[8] = {t0.x, t0.y, t0.z, t0.w, t1.x, t1.y, t1.z, t1.w};
+#pragma unroll
+        for (int i = 0; i < 8; ++i)
+#pragma unroll
+          for (int j = 0; j < 8; ++j) acc[i][j] = fmaf(tv[j], xv[i], acc[i][j]);
+      }
+      if (s % npan == npan - 1) {
+        const int k0 = (s / npan) * KC;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          const int k = k0 + (j < 4 ? 4 * tx + j : KC / 2 + 4 * tx + j - 4);
+          if (k < a.K) {
+            const float lw = __ldg(a.logw + k);
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+              const int p = i < 4 ? 4 * ty + i : TP / 2 + 4 * ty + i - 4;
+              rs[(size_t)k * TP + p] = __fadd_rn(acc[i][j], lw);
+            }
+          }
+        }
+      }
+      __syncthreads();   // the buffer just read is the next issue's target
+    }
+    if (tid < npts) {
+      const int64_t i = base + tid;
+      float* col = rs + tid;
+      if (a.dump != nullptr)
+        for (int k = 0; k < a.K; ++k) a.dump[(size_t)k * a.n + i] = col[(size_t)k * TP];
+      int lab;
+      if (a.final_iter) {
+        lab = dpmm_draw_argmax(col, TP, a.K);
+      } else if (a.sampler == 1) {
+        lab = dpmm_draw_gumbel(col, TP, a.K, a.seed, a.call, (uint64_t)(a.goff + i));
+      } else {
+        const double u = dpmm_uniform(a.u_inj, i, a.seed, DPMM_STREAM_LABEL, a.call, (uint64_t)(a.goff + i));
+        lab = dpmm_draw_inverse_cdf_screened(col, TP, a.K, u);
+      }
+      a.labels[i] = lab;
+      atomicAdd(&hs[lab], 1);
+    }
+    __syncthreads();   // rs is rewritten by the next tile
+  }
+  for (int k = tid; k < a.K; k += 256)
+    if (hs[k] != 0) atomicAdd(&a.hist[k], hs[k]);
+}
+
 // Sub-label draw over the label-sorted permutation (+ left/right partition); a.recs = log_p [3K][D].
 template <bool SAMPLE>
 __global__ void mnm_sublabel_kernel(const SubLabelArgs a) {
@@ -143,6 +273,60 @@ __global__ void mnm_sublabel_kernel(const SubLabelArgs a) {
     }
   }
   sublabel_partition(a, active, k, side, idx, s_cnt, s_base, s_first);
+}
+
+// Sub-label draw, D > 1024: the positions and the per-point arithmetic of mnm_sublabel_kernel<true> (128
+// label-sorted positions per CTA, sl / sr sequential fmaf over ascending d), but the 128 rows go through a
+// [128][65] shared-memory tile 64 features at a time, every row segment read by a whole warp as two 128-byte
+// lines, instead of each thread walking its own row.
+#define MNM_SLS_T 128
+__global__ void __launch_bounds__(MNM_SLS_T) mnm_sublabel_staged_kernel(const SubLabelArgs a) {
+  __shared__ float xs[MNM_SLS_T][65];
+  __shared__ int32_t s_idx[MNM_SLS_T];
+  __shared__ int s_cnt[2 * MNM_SLS_T];
+  __shared__ int s_base[2 * MNM_SLS_T];
+  __shared__ int s_first[2];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int D = a.D;
+  const int64_t pos = (int64_t)blockIdx.x * MNM_SLS_T + tid;
+  const bool active = pos < a.n;
+  int32_t idx = active ? a.perm[pos] : -1;
+  const int k = active ? a.labels[idx] : 0;
+  s_idx[tid] = idx;
+  const float* al = a.recs + (size_t)(3 * k + 1) * D;
+  const float* ar = a.recs + (size_t)(3 * k + 2) * D;
+  float sl = 0.f, sr = 0.f;
+  for (int d0 = 0; d0 < D; d0 += 64) {
+    __syncthreads();   // s_idx written / the previous panel consumed
+    const bool ok0 = d0 + lane < D, ok1 = d0 + 32 + lane < D;
+#pragma unroll 8
+    for (int p = warp; p < MNM_SLS_T; p += MNM_SLS_T / 32) {
+      const int32_t q = s_idx[p];
+      const float* xr = a.x + (size_t)max(q, 0) * D + d0 + lane;
+      xs[p][lane] = (q >= 0 && ok0) ? __ldg(xr) : 0.f;
+      xs[p][32 + lane] = (q >= 0 && ok1) ? __ldg(xr + 32) : 0.f;
+    }
+    __syncthreads();
+    const int dn = min(64, D - d0);
+    for (int d = 0; d < dn; ++d) {
+      const float xv = xs[tid][d];
+      sl = fmaf(__ldg(al + d0 + d), xv, sl);
+      sr = fmaf(__ldg(ar + d0 + d), xv, sr);
+    }
+  }
+  int side = 0;
+  if (active) {
+    const float rl = __fadd_rn(sl, __ldg(a.loglr + 2 * k));
+    const float rr = __fadd_rn(sr, __ldg(a.loglr + 2 * k + 1));
+    if (a.dump != nullptr) {
+      a.dump[idx] = rl;
+      a.dump[a.n + idx] = rr;
+    }
+    const double u = dpmm_uniform(a.u_inj, idx, a.seed, DPMM_STREAM_SUBLABEL, a.call, (uint64_t)(a.goff + idx));
+    side = dpmm_draw_two(rl, rr, u);
+    a.sub[idx] = (uint8_t)side;
+  }
+  sublabel_partition(a, active, k, side, active ? idx : 0, s_cnt, s_base, s_first);
 }
 
 // Sub-label draw, D <= 128: a warp evaluates its 32 label-sorted positions one point at a time with

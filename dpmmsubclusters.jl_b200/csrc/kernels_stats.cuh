@@ -367,63 +367,70 @@ __global__ void __launch_bounds__(256) niw_stats_small_kernel(const StatsArgs a)
 // segments straight from global memory (no staging), with MNM_STATS_UNROLL points in flight per
 // warp, and the per-lane Float32 partial sums (exact: small integer counts) are added to the key's
 // Float64 accumulator once per item.
-#define MNM_STATS_NREG 32      // features per lane: supports D <= 1024
+#define MNM_STATS_NREG 32      // features per lane: slices of 1024 features
 #define MNM_STATS_UNROLL 8
+template <bool SLICED>
 __global__ void __launch_bounds__(256) mnm_stats_kernel(const StatsArgs a) {
-  const int D = a.D;
   const int lane = threadIdx.x & 31;
-  const int nreg = (D + 31) >> 5;
-  const int n_items = *a.n_items;
+  // SLICED (D > 1024): a work unit is (item, slice of 32 x MNM_STATS_NREG features)
+  const int nslices = SLICED ? (a.D + 32 * MNM_STATS_NREG - 1) / (32 * MNM_STATS_NREG) : 1;
+  const int n_units = *a.n_items * nslices;
   for (;;) {
-    int it = 0;
-    if (lane == 0) it = atomicAdd(a.next_item, 1);
-    it = __shfl_sync(0xffffffffu, it, 0);
-    if (it >= n_items) break;
-    const StatsItem item = a.items[it];
-    float acc[MNM_STATS_NREG];
+    int u = 0;
+    if (lane == 0) u = atomicAdd(a.next_item, 1);
+    u = __shfl_sync(0xffffffffu, u, 0);
+    if (u >= n_units) break;
+    const StatsItem item = a.items[u / nslices];
+    {
+      const int d0 = (u % nslices) * 32 * MNM_STATS_NREG;
+      const int D = SLICED ? min(a.D - d0, 32 * MNM_STATS_NREG) : a.D;
+      const float* x = a.x + d0;
+      const int nreg = (D + 31) >> 5;
+      float acc[MNM_STATS_NREG];
 #pragma unroll
-    for (int r = 0; r < MNM_STATS_NREG; ++r) acc[r] = 0.f;
-    int idx_n[MNM_STATS_UNROLL];
+      for (int r = 0; r < MNM_STATS_NREG; ++r) acc[r] = 0.f;
+      int idx_n[MNM_STATS_UNROLL];
 #pragma unroll
-    for (int j = 0; j < MNM_STATS_UNROLL; ++j) idx_n[j] = (item.begin + j < item.end) ? __ldg(a.perm2 + item.begin + j) : -1;
-    for (int p0 = item.begin; p0 < item.end; p0 += MNM_STATS_UNROLL) {
-      int idx[MNM_STATS_UNROLL];
+      for (int j = 0; j < MNM_STATS_UNROLL; ++j) idx_n[j] = (item.begin + j < item.end) ? __ldg(a.perm2 + item.begin + j) : -1;
+      for (int p0 = item.begin; p0 < item.end; p0 += MNM_STATS_UNROLL) {
+        int idx[MNM_STATS_UNROLL];
 #pragma unroll
-      for (int j = 0; j < MNM_STATS_UNROLL; ++j) {
-        idx[j] = idx_n[j];                                   // indices were fetched one batch ahead
-        const int pn = p0 + MNM_STATS_UNROLL + j;
-        idx_n[j] = (pn < item.end) ? __ldg(a.perm2 + pn) : -1;
-      }
-      if (nreg <= 4) {  // common case (D <= 128): all loads of the batch in flight at once
-        float v[MNM_STATS_UNROLL][4];
+        for (int j = 0; j < MNM_STATS_UNROLL; ++j) {
+          idx[j] = idx_n[j];                                   // indices were fetched one batch ahead
+          const int pn = p0 + MNM_STATS_UNROLL + j;
+          idx_n[j] = (pn < item.end) ? __ldg(a.perm2 + pn) : -1;
+        }
+        if (nreg <= 4) {  // common case (D <= 128): all loads of the batch in flight at once
+          float v[MNM_STATS_UNROLL][4];
 #pragma unroll
-        for (int j = 0; j < MNM_STATS_UNROLL; ++j)
+          for (int j = 0; j < MNM_STATS_UNROLL; ++j)
 #pragma unroll
-          for (int r = 0; r < 4; ++r) {
-            const int d = lane + 32 * r;
-            v[j][r] = (idx[j] >= 0 && d < D) ? __ldg(a.x + (size_t)idx[j] * D + d) : 0.f;
-          }
-#pragma unroll
-        for (int j = 0; j < MNM_STATS_UNROLL; ++j)
-#pragma unroll
-          for (int r = 0; r < 4; ++r) acc[r] += v[j][r];
-      } else {
-#pragma unroll
-        for (int j = 0; j < MNM_STATS_UNROLL; ++j)
-          if (idx[j] >= 0) {
-#pragma unroll
-            for (int r = 0; r < MNM_STATS_NREG; ++r) {
+            for (int r = 0; r < 4; ++r) {
               const int d = lane + 32 * r;
-              if (r < nreg && d < D) acc[r] += __ldg(a.x + (size_t)idx[j] * D + d);
+              v[j][r] = (idx[j] >= 0 && d < D) ? __ldg(x + (size_t)idx[j] * a.D + d) : 0.f;
             }
-          }
-      }
-    }
-    double* dst = a.acc + (size_t)item.key * a.rec + 1;
 #pragma unroll
-    for (int r = 0; r < MNM_STATS_NREG; ++r) {
-      const int d = lane + 32 * r;
-      if (r < nreg && d < D && acc[r] != 0.f) atomicAdd(dst + d, (double)acc[r]);
+          for (int j = 0; j < MNM_STATS_UNROLL; ++j)
+#pragma unroll
+            for (int r = 0; r < 4; ++r) acc[r] += v[j][r];
+        } else {
+#pragma unroll
+          for (int j = 0; j < MNM_STATS_UNROLL; ++j)
+            if (idx[j] >= 0) {
+#pragma unroll
+              for (int r = 0; r < MNM_STATS_NREG; ++r) {
+                const int d = lane + 32 * r;
+                if (r < nreg && d < D) acc[r] += __ldg(x + (size_t)idx[j] * a.D + d);
+              }
+            }
+        }
+      }
+      double* dst = a.acc + (size_t)item.key * a.rec + 1 + d0;
+#pragma unroll
+      for (int r = 0; r < MNM_STATS_NREG; ++r) {
+        const int d = lane + 32 * r;
+        if (r < nreg && d < D && acc[r] != 0.f) atomicAdd(dst + d, (double)acc[r]);
+      }
     }
   }
 }

@@ -51,7 +51,9 @@ typedef struct dpmm_ctx dpmm_ctx;
  * shard.  x: host float32 [d x n_local] column-major, copied to the device.  global_offset = index
  * (0-based) of this shard's first point in the whole data set: the counter-based RNG is keyed by the
  * global point index so results do not depend on how many GPUs the points are spread over.
- * device: CUDA ordinal.  seed: replaces `@everywhere Random.seed!(seed)` (:37-39). */
+ * device: CUDA ordinal.  seed: replaces `@everywhere Random.seed!(seed)` (:37-39).
+ * d: 1..64 for the NIW prior, 1..16384 for the multinomial prior; larger d returns
+ * DPMM_ELIMIT.  Every multinomial d samples with any K up to DPMM_MAX_K. */
 int dpmm_create(dpmm_ctx** out, const float* x, int64_t n_local, int32_t d, int32_t prior_kind,
                 int32_t device, uint64_t seed, int64_t global_offset);
 int dpmm_destroy(dpmm_ctx* ctx);
@@ -59,7 +61,7 @@ const char* dpmm_last_error(const dpmm_ctx* ctx);
 /* Use an externally owned cudaStream_t (e.g. the host framework's current stream) for all work. */
 int dpmm_set_stream(dpmm_ctx* ctx, void* cuda_stream);
 int dpmm_sync(dpmm_ctx* ctx);
-/* out[0]=max D (NIW), out[1]=max D (multinomial), out[2]=max K. */
+/* out[0]=max D (NIW, 64), out[1]=max D (multinomial, 16384), out[2]=max K (1024, any D of either prior). */
 int dpmm_limits(int32_t* out3);
 
 /* ---- labels: initialisation, gather, resume ------------------------------------------------- */
