@@ -62,6 +62,7 @@ SIGNATURES = {
     "dpmm_set_uniforms": (C.c_int, [_p, _f64p, _f64p, _u8p]),
     "dpmm_debug_loglik": (C.c_int, [_p, _i32, _f32p]),
     "dpmm_debug_tc_stats": (C.c_int, [_p, _i64p]),
+    "dpmm_debug_sort": (C.c_int, [_p, C.POINTER(C.c_int32), _i64p]),
     "dpmm_debug_fused_stats": (C.c_int, [_p, _i64p]),
     "dpmm_timing_enable": (C.c_int, [_p, _i32]),
     "dpmm_timing_kinds": (C.c_int, []),

@@ -259,6 +259,33 @@ __device__ __forceinline__ int dpmm_draw_two(float rl, float rr, double u) {
   return dpmm_draw_inverse_cdf(m, 1, 2, u);
 }
 
+// ---------------------------------------------------------------------------------------------
+// Programmatic dependent launch (PDL).  The sweep's kernels are launched with launch_pdl(): a kernel may start while
+// its predecessor on the stream still runs, does only CTA-local set-up (mbarriers, shared-memory tables, tensor memory)
+// and then waits in pdl_wait() until the predecessor has completed and its writes are visible.  Every global load or
+// store of such a kernel comes after pdl_wait().  pdl_launch_dependents() lets the next kernel be scheduled; the
+// kernels here issue it right after their own wait, so at most two grids of the chain overlap.  Both are no-ops in a
+// kernel launched without the attribute.
+// ---------------------------------------------------------------------------------------------
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
+template <typename... KArgs, typename... Args>
+inline cudaError_t launch_pdl(bool pdl, void (*kern)(KArgs...), dim3 grid, unsigned block, size_t smem,
+                              cudaStream_t stream, Args... args) {
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = grid;
+  cfg.blockDim = dim3(block);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = stream;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = pdl ? 1 : 0;
+  return cudaLaunchKernelEx(&cfg, kern, args...);
+}
+
 __device__ __forceinline__ double dpmm_uniform(const double* inj, int64_t local_i, uint64_t seed,
                                                uint32_t stream, uint32_t call, uint64_t gidx) {
   if (inj != nullptr) return inj[local_i];

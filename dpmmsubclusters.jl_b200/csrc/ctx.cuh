@@ -105,7 +105,7 @@ struct dpmm_ctx {
   float* t2_bias = nullptr;
   float* t2_fro8 = nullptr;
   int32_t* t2_ctr = nullptr;
-  int32_t* ctr_sets = nullptr;   // [2][4]: tc_stats / t2_ctr point into the set of the current label call
+  int32_t* ctr_sets = nullptr;   // [2][T2_CTR_SET]: tc_stats / t2_ctr point into the set of the current label call
   int ctr_cur = 0;
   bool ctr_clean = false;        // the set the next tensor-core label call takes is known to be zero
   bool t2_ok = false;       // shape supported
@@ -114,7 +114,8 @@ struct dpmm_ctx {
   // adaptive path choice: counters of the last tensor-core label call (points, exact evaluations, overflow points)
   // land in pinned memory behind an event; a call that finds more exact work than the FMA kernel would do for all K
   // clusters sends the next calls to the FMA kernel for a while (early iterations, heavily overlapping clusters)
-  int32_t* t2_hstat = nullptr;       // pinned [4]
+  int32_t* t2_hstat = nullptr;       // mapped pinned [4], written by the overflow kernel's last block
+  int32_t* t2_hstat_dev = nullptr;   // its device address
   cudaEvent_t t2_hstat_ev = nullptr;
   bool t2_hstat_pending = false;
   int t2_cooldown = 0;
@@ -131,7 +132,17 @@ struct dpmm_ctx {
   bool tc_params = false;   // tc_* describe the current parameters
   float* logp_t = nullptr;  // multinomial [D][KP]
   int KP = 0;
-  int32_t* hist = nullptr;
+  // label histograms: two buffers of Kcap entries.  A tensor-core label call fills one (ctx->hist from then on) while
+  // its overflow kernel clears the other for the next call, so no memset sits between the sweeps
+  int32_t* hist_mem = nullptr;
+  int32_t* hist = nullptr;        // the buffer of the current labels
+  int hist_cur = 0;
+  int hist_spare_clean = 0;       // entries of the other buffer known to be zero
+  // moved-point counter of the last tensor-core label call, while perm still sorts the labels that call started from
+  // and nothing else changed them: the sort after it then skips the scatter when the counter is 0
+  const int32_t* t2_moved = nullptr;
+  int risk_zeroed_k = 0;          // K > 0: the label scatter cleared the risk slot outbuf[3 K rec] (no memset before the finalise)
+  int pdl_tmem = -1;              // tensor memory may be allocated before the grid dependency (sweep_pdl_ok); -1: not checked yet
   int32_t* seg_off = nullptr;
   int32_t* scat_cursor = nullptr;
   int32_t* lr_cursor = nullptr;

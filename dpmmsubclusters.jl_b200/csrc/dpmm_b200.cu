@@ -122,7 +122,11 @@ static int ensure_k(dpmm_ctx* ctx, int K) {
     CK(dev_realloc(&ctx->ss_b, (size_t)cap * 2 * D));
     CK(dev_realloc(&ctx->ss_c, (size_t)cap * D));
   }
-  CK(dev_realloc(&ctx->hist, (size_t)cap));
+  CK(dev_realloc(&ctx->hist_mem, (size_t)2 * cap));
+  ctx->hist = ctx->hist_mem;
+  ctx->hist_cur = ctx->hist_spare_clean = 0;
+  ctx->t2_moved = nullptr;
+  ctx->risk_zeroed_k = 0;
   CK(dev_realloc(&ctx->seg_off, (size_t)cap + 1));
   CK(dev_realloc(&ctx->scat_cursor, (size_t)cap));
   CK(dev_realloc(&ctx->lr_cursor, (size_t)2 * cap));
@@ -307,8 +311,8 @@ extern "C" int dpmm_create(dpmm_ctx** out, const float* x, int64_t n_local, int3
   if (ctx->tc_ok || (prior_kind == DPMM_PRIOR_NIW && (dpad == 32 || dpad == 64) && n_local >= T2_TILE)) {
     // two alternating counter sets [exact evaluations: points, evaluations | overflow count | pad]: the overflow
     // kernel of a call clears the set of the next one, so no memset launches sit between the sweeps
-    CKC(cudaMalloc((void**)&ctx->ctr_sets, 8 * sizeof(int32_t)));
-    CKC(cudaMemset(ctx->ctr_sets, 0, 8 * sizeof(int32_t)));
+    CKC(cudaMalloc((void**)&ctx->ctr_sets, 2 * T2_CTR_SET * sizeof(int32_t)));
+    CKC(cudaMemset(ctx->ctr_sets, 0, 2 * T2_CTR_SET * sizeof(int32_t)));
     ctx->tc_stats = ctx->ctr_sets;
     ctx->t2_ctr = ctx->ctr_sets + 2;
   }
@@ -377,7 +381,7 @@ extern "C" int dpmm_destroy(dpmm_ctx* ctx) {
   }
   for (auto e : ctx->ev_pool) cudaEventDestroy(e);
   void* ptrs[] = {ctx->x, ctx->labels, ctx->sub, ctx->perm, ctx->perm2, ctx->u_label, ctx->u_sub, ctx->r_bits,
-                  ctx->raw_params, ctx->recs, ctx->cst, ctx->logw, ctx->loglr, ctx->logp_t, ctx->t2_piv, ctx->t2_scr, ctx->t2_u, ctx->t2_bias, ctx->t2_fro8, ctx->ctr_sets, ctx->tc_w, ctx->tc_b, ctx->tc_mu, ctx->tc_fro, ctx->ss_w, ctx->ss_b, ctx->ss_c, ctx->lcount, ctx->mtc_w, ctx->hist, ctx->seg_off,
+                  ctx->raw_params, ctx->recs, ctx->cst, ctx->logw, ctx->loglr, ctx->logp_t, ctx->t2_piv, ctx->t2_scr, ctx->t2_u, ctx->t2_bias, ctx->t2_fro8, ctx->ctr_sets, ctx->tc_w, ctx->tc_b, ctx->tc_mu, ctx->tc_fro, ctx->ss_w, ctx->ss_b, ctx->ss_c, ctx->lcount, ctx->mtc_w, ctx->hist_mem, ctx->seg_off,
                   ctx->scat_cursor, ctx->lr_cursor, ctx->lut_l, ctx->lut_r, ctx->rule, ctx->wanted,
                   ctx->idx_list, ctx->acc, ctx->centers, ctx->outbuf, ctx->items, ctx->item_ctr, ctx->hyper_d, ctx->ptab,
                   ctx->ptab_alt, ctx->post, ctx->post_alt, ctx->lfac, ctx->pm_out, ctx->splittable_d, ctx->newof_d,
@@ -877,6 +881,32 @@ extern "C" int dpmm_set_params_multinomial(dpmm_ctx* ctx, int32_t K, const float
 // ------------------------------------------------------------------------------------------------
 static int ensure_sorted(dpmm_ctx* ctx);
 
+// The sweep's kernels are chained with programmatic dependent launch (common.cuh).  The label and fused kernels allocate
+// tensor memory before their grid dependency, i.e. possibly while CTAs of the previous kernel still run.  That is safe
+// when no two CTAs that hold tensor memory can share an SM, which their register footprints decide (C2: 448 x 128 and
+// 896 x 72 registers of 64 Ki): checked here once from the compiled kernels; if it does not hold, these two kernels are
+// launched without the attribute.  Timed launches (KernelTimer events between the kernels) are plain as well.
+static bool sweep_pdl_ok(dpmm_ctx* ctx) {
+  if (ctx->pdl_tmem < 0) {
+    const struct { const void* f; int threads; } ks[] = {{(const void*)gauss_label_tc2_kernel<32>, T2_THREADS(32)},
+                                                        {(const void*)gauss_label_tc2_kernel<64>, T2_THREADS(64)},
+                                                        {(const void*)niw_substats_tc_kernel, SS_THREADS}};
+    int regs_sm = 0;
+    bool ok = cudaDeviceGetAttribute(&regs_sm, cudaDevAttrMaxRegistersPerMultiprocessor, ctx->device) == cudaSuccess;
+    int foot[3];
+    for (int i = 0; i < 3 && ok; ++i) {
+      cudaFuncAttributes fa;
+      ok = cudaFuncGetAttributes(&fa, ks[i].f) == cudaSuccess;
+      foot[i] = fa.numRegs * ks[i].threads;
+    }
+    for (int i = 0; i < 3 && ok; ++i)
+      for (int j = 0; j < 3; ++j) ok &= foot[i] + foot[j] > regs_sm;
+    cudaGetLastError();
+    ctx->pdl_tmem = ok ? 1 : 0;
+  }
+  return ctx->pdl_tmem == 1 && !ctx->timing;
+}
+
 template <int D>
 static int launch_label_tc2(dpmm_ctx* ctx, int final_iter, int nkeys) {
   const int K = ctx->K;
@@ -887,27 +917,39 @@ static int launch_label_tc2(dpmm_ctx* ctx, int final_iter, int nkeys) {
   a.urows = ctx->t2_u; a.mu = ctx->tc_mu; a.cst = ctx->cst; a.logw = ctx->logw; a.fro = ctx->tc_fro;
   // this call's counter set (the other one was cleared by the previous call's overflow kernel)
   ctx->ctr_cur ^= 1;
-  ctx->tc_stats = ctx->ctr_sets + 4 * ctx->ctr_cur;
+  ctx->tc_stats = ctx->ctr_sets + T2_CTR_SET * ctx->ctr_cur;
   ctx->t2_ctr = ctx->tc_stats + 2;
   a.labels = ctx->labels; a.hist = ctx->hist; a.ovf_list = ctx->perm2; a.ovf_count = ctx->t2_ctr;
   a.u_inj = ctx->u_label; a.seed = ctx->seed; a.call = ctx->call; a.goff = ctx->goff; a.final_iter = final_iter;
   a.stats = ctx->tc_stats;
+  a.moved = ctx->tc_stats + 4;
   const size_t sm = GaussTc2Smem(D, K, a.KS, a.nch, nkeys).total;
   CK(cudaFuncSetAttribute(gauss_label_tc2_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-  if (!ctx->ctr_clean) CK(cudaMemsetAsync(ctx->ctr_sets, 0, 8 * sizeof(int32_t), ctx->stream));   // another path used them
+  if (!ctx->ctr_clean) CK(cudaMemsetAsync(ctx->ctr_sets, 0, 2 * T2_CTR_SET * sizeof(int32_t), ctx->stream));   // another path used them
+  if (ctx->t2_hstat == nullptr) {
+    CK(cudaHostAlloc((void**)&ctx->t2_hstat, 4 * sizeof(int32_t), cudaHostAllocMapped));
+    CK(cudaHostGetDevicePointer((void**)&ctx->t2_hstat_dev, ctx->t2_hstat, 0));
+    CK(cudaEventCreateWithFlags(&ctx->t2_hstat_ev, cudaEventDisableTiming));
+  }
   const int64_t grid = std::min<int64_t>((ctx->n + T2_TILE - 1) / T2_TILE, (int64_t)ctx->sm_count);
   {
     KernelTimer kt(ctx, TK_LABEL);
-    gauss_label_tc2_kernel<D><<<(unsigned)grid, T2_THREADS(D), sm, ctx->stream>>>(a);
-    CK(cudaGetLastError());
+    CK(launch_pdl(sweep_pdl_ok(ctx), gauss_label_tc2_kernel<D>, (unsigned)grid, T2_THREADS(D), sm, ctx->stream, a));
   }
   // the (normally empty) overflow list: points with a NaN / Inf screen value or more than 7 candidates
   GaussListArgs l{};
   l.x = ctx->x; l.K = K; l.list = ctx->perm2; l.count = ctx->t2_ctr; l.urows = ctx->t2_u; l.mu = ctx->tc_mu;
   l.cst = ctx->cst; l.logw = ctx->logw; l.labels = ctx->labels; l.hist = ctx->hist; l.u_inj = ctx->u_label;
   l.seed = ctx->seed; l.call = ctx->call; l.goff = ctx->goff; l.final_iter = final_iter; l.stats = a.stats;
-  l.zero_next = ctx->ctr_sets + 4 * (ctx->ctr_cur ^ 1);
+  l.moved = a.moved;
+  l.zero_next = ctx->ctr_sets + T2_CTR_SET * (ctx->ctr_cur ^ 1);
   ctx->ctr_clean = true;
+  // the histogram buffer of the previous labels is not read again: it becomes the next call's, cleared here
+  l.zero_hist = ctx->hist_mem + (size_t)(ctx->hist_cur ^ 1) * ctx->Kcap;
+  l.zero_hist_n = K;
+  ctx->hist_spare_clean = K;
+  // the counters go to mapped host memory; the event behind the kernel says they have arrived (never waited for)
+  l.hstat = ctx->t2_hstat_dev;
   // the last block of the overflow kernel scans the new label histogram (label_scan_kernel's job) when the scan's
   // width is the K of this call: one launch fewer between the label kernel and the sort
   l.ticket = ctx->tc_stats + 3; l.scan_k = K; l.seg_off = ctx->seg_off; l.scat_cursor = ctx->scat_cursor; l.lr_cursor = ctx->lr_cursor;
@@ -915,15 +957,8 @@ static int launch_label_tc2(dpmm_ctx* ctx, int final_iter, int nkeys) {
   if (lsm > 48 * 1024) CK(cudaFuncSetAttribute(gauss_label_list_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lsm));
   {
     KernelTimer kt(ctx, TK_LABEL_OVF);
-    gauss_label_list_kernel<D><<<(unsigned)ctx->sm_count * 2, 256, lsm, ctx->stream>>>(l);
-    CK(cudaGetLastError());
+    CK(launch_pdl(!ctx->timing, gauss_label_list_kernel<D>, (unsigned)ctx->sm_count * 2, 256, lsm, ctx->stream, l));
   }
-  // counters -> pinned memory (read by the next call's path choice, never waited for)
-  if (ctx->t2_hstat == nullptr) {
-    CK(cudaMallocHost((void**)&ctx->t2_hstat, 4 * sizeof(int32_t)));
-    CK(cudaEventCreateWithFlags(&ctx->t2_hstat_ev, cudaEventDisableTiming));
-  }
-  CK(cudaMemcpyAsync(ctx->t2_hstat, ctx->tc_stats, 12, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaEventRecord(ctx->t2_hstat_ev, ctx->stream));
   ctx->t2_hstat_pending = true;
   return 0;
@@ -978,7 +1013,13 @@ static int run_sample_labels(dpmm_ctx* ctx, int final_iter, float* dump) {
     int rc = ensure_sorted(ctx);
     if (rc) return rc;
   }
-  CK(cudaMemsetAsync(ctx->hist, 0, (size_t)K * 4, ctx->stream));
+  if (use_t2 && ctx->hist_spare_clean >= K) {   // cleared by the previous tensor-core call's overflow kernel
+    ctx->hist_cur ^= 1;
+    ctx->hist = ctx->hist_mem + (size_t)ctx->hist_cur * ctx->Kcap;
+    ctx->hist_spare_clean = 0;
+  } else {
+    CK(cudaMemsetAsync(ctx->hist, 0, (size_t)K * 4, ctx->stream));
+  }
   if (use_t2) {
     int rc = ctx->D == 32 ? launch_label_tc2<32>(ctx, final_iter, nkeys) : launch_label_tc2<64>(ctx, final_iter, nkeys);
     if (rc) return rc;
@@ -1051,6 +1092,7 @@ static int run_sample_labels(dpmm_ctx* ctx, int final_iter, float* dump) {
   }
   ctx->hist_valid = true;
   ctx->scan_valid = use_t2;   // the overflow kernel's last block already scanned the new histogram (width K)
+  ctx->t2_moved = use_t2 ? ctx->tc_stats + 4 : nullptr;   // (perm sorts the labels this call started from)
   ctx->sorted = false;
   ctx->partitioned = ctx->stats_cached = false;
   ctx->label_bound = K;
@@ -1077,17 +1119,22 @@ static int ensure_sorted(dpmm_ctx* ctx) {
     label_scan_kernel<<<1, 1024, 0, ctx->stream>>>(ctx->hist, K, ctx->seg_off, ctx->scat_cursor, ctx->lr_cursor);
     CK(cudaGetLastError());
   }
+  // the tensor-core label call that produced these labels counted the points that changed label: with none, perm
+  // (sorted for the labels that call started from) is still a valid sort and the scatter kernel skips its work
+  const int32_t* moved = ctx->hist_valid && ctx->scan_valid ? ctx->t2_moved : nullptr;
+  ctx->t2_moved = nullptr;
   ctx->scan_valid = false;   // the scatter below consumes the cursors
   {
     const int T = 256;
     const unsigned grid = (unsigned)((ctx->n + (int64_t)T * SCATTER_PPT - 1) / ((int64_t)T * SCATTER_PPT));
-    // the fused sub-label + statistics kernel (NIW, D = 32) wants its accumulators cleared: done here
+    // the fused sub-label + statistics kernel (NIW, D = 32) wants its accumulators cleared, and the statistics finalise
+    // that follows it the risk slot of outbuf: done here
     const bool pre = ctx->prior == DPMM_PRIOR_NIW && ctx->D == SS_D && ctx->tc_ok && ctx->lcount != nullptr;
-    label_scatter_kernel<<<grid, T, (size_t)K * 8, ctx->stream>>>(ctx->labels, ctx->n, K, ctx->scat_cursor, ctx->perm,
-                                                                  pre ? ctx->acc : nullptr, pre ? (int64_t)2 * K * ctx->stats_rec : 0,
-                                                                  pre ? ctx->lcount : nullptr, pre ? K : 0);
-    CK(cudaGetLastError());
+    CK(launch_pdl(!ctx->timing, label_scatter_kernel, grid, T, (size_t)K * 8, ctx->stream, (const int32_t*)ctx->labels,
+                  ctx->n, K, ctx->scat_cursor, ctx->perm, pre ? ctx->acc : nullptr, pre ? (int64_t)2 * K * ctx->stats_rec : (int64_t)0,
+                  pre ? ctx->lcount : nullptr, pre ? K : 0, pre ? ctx->outbuf + (size_t)K * 3 * ctx->stats_rec : nullptr, moved));
     ctx->acc_cleared = pre;
+    ctx->risk_zeroed_k = pre ? K : 0;
   }
   ctx->sorted = true;
   ctx->partitioned = ctx->stats_cached = false;
@@ -1132,8 +1179,7 @@ static int run_sublabels(dpmm_ctx* ctx, bool sample, float* dump) {
     CK(cudaFuncSetAttribute(niw_substats_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     {
       KernelTimer kt(ctx, TK_SUBLABEL);
-      niw_substats_tc_kernel<<<ctx->sm_count, SS_THREADS, smem, ctx->stream>>>(f);
-      CK(cudaGetLastError());
+      CK(launch_pdl(sweep_pdl_ok(ctx), niw_substats_tc_kernel, (unsigned)ctx->sm_count, SS_THREADS, smem, ctx->stream, f));
     }
     ctx->partitioned = false;
     ctx->stats_cached = true;
@@ -1319,13 +1365,13 @@ static int stats_compute(dpmm_ctx* ctx, const int64_t* indices, int32_t n_indice
     KernelTimer kt(ctx, TK_STATS_AUX);
     const int T = 256;
     dim3 grid((unsigned)std::min((rec + T - 1) / T, 64), (unsigned)m);
-    CK(cudaMemsetAsync(fin + (size_t)m * 3 * rec, 0, 8, ctx->stream));
-    stats_finalize_kernel<<<grid, T, 0, ctx->stream>>>(ctx->acc, ctx->seg_off, ctx->lr_cursor, all ? nullptr : ctx->idx_list, m, D, rec,
-                                                       ctx->prior == DPMM_PRIOR_NIW ? 1 : 0, fin,
-                                                       (stats_tc || stats_tc64 || cached) ? ctx->centers : nullptr,
-                                                       cached ? ctx->lcount : nullptr,
-                                                       cached ? fin + (size_t)m * 3 * rec : nullptr);
-    CK(cudaGetLastError());
+    // the risk slot: cleared by the label scatter that preceded the fused kernel, or here
+    if (!(fin == ctx->outbuf && m == ctx->risk_zeroed_k)) CK(cudaMemsetAsync(fin + (size_t)m * 3 * rec, 0, 8, ctx->stream));
+    ctx->risk_zeroed_k = 0;
+    CK(launch_pdl(!ctx->timing, stats_finalize_kernel, grid, T, 0, ctx->stream, (const double*)ctx->acc, (const int32_t*)ctx->seg_off,
+                  (const int32_t*)ctx->lr_cursor, (const int32_t*)(all ? nullptr : ctx->idx_list), m, D, rec,
+                  ctx->prior == DPMM_PRIOR_NIW ? 1 : 0, fin, (const float*)((stats_tc || stats_tc64 || cached) ? ctx->centers : nullptr),
+                  (const int32_t*)(cached ? ctx->lcount : nullptr), cached ? fin + (size_t)m * 3 * rec : nullptr));
   }
   if (use_ipc) {
     IpcReduceArgs ia{};
@@ -1877,6 +1923,24 @@ extern "C" int dpmm_debug_tc_stats(dpmm_ctx* ctx, int64_t* out3) {
   if (ctx->t2_ctr != nullptr) {
     CK(cudaMemcpy(h, ctx->t2_ctr, 4, cudaMemcpyDeviceToHost));
     out3[2] = h[0];
+  }
+  return 0;
+}
+
+extern "C" int dpmm_debug_sort(dpmm_ctx* ctx, int32_t* perm, int64_t* moved) {
+  NEED(ctx && moved, DPMM_EINVAL, "NULL argument");
+  CK(cudaSetDevice(ctx->device));
+  moved[0] = 0;
+  if (perm != nullptr) {
+    int rc = ensure_sorted(ctx);
+    if (rc) return rc;
+  }
+  CK(cudaStreamSynchronize(ctx->stream));
+  if (perm != nullptr) CK(cudaMemcpy(perm, ctx->perm, (size_t)ctx->n * 4, cudaMemcpyDeviceToHost));
+  if (ctx->ctr_sets != nullptr) {
+    int32_t h = 0;
+    CK(cudaMemcpy(&h, ctx->tc_stats + 4, 4, cudaMemcpyDeviceToHost));
+    moved[0] = h;
   }
   return 0;
 }

@@ -44,6 +44,8 @@
 #include "kernels_stats.cuh"   // cp_async16 / commit / wait_group
 
 #define T2_TILE 128
+// per-call counter set: [0] points, [1] exact evaluations, [2] overflow points, [3] scan ticket, [4] moved points
+#define T2_CTR_SET 8
 #define T2_PRODUCERS(D) ((D) == 32 ? 128 : 64)   // gather threads (warps 10-13 / 10-11): D = 64 needs the registers
 #define T2_THREADS(D) (320 + T2_PRODUCERS(D))
 #define T2_CMAX 8          // exact evaluations per point handled in the kernel (pivot included)
@@ -81,6 +83,7 @@ struct GaussTc2Args {
   int64_t goff;
   int final_iter;
   int32_t* stats;          // optional [2]: points, exact evaluations
+  int32_t* moved;          // [1] += points whose new label differs from their old one (the pivot)
 };
 
 struct GaussTc2Smem {
@@ -366,7 +369,12 @@ __global__ void __launch_bounds__(T2_THREADS(D), 1) gauss_label_tc2_kernel(const
     tc::mbar_init(&wdone[1], 1);
     tc::fence_barrier_init();
   }
+  // Tensor memory is allocated before the grid dependency, possibly while CTAs of the previous kernel still run: safe
+  // because no CTA that holds tensor memory can share an SM with this one (their register files do not fit together;
+  // checked on the host by sweep_pdl_ok, which otherwise launches this kernel without PDL).
   if (warp == 1) tc::tmem_alloc(tmem_ptr, 512);
+  pdl_wait();
+  pdl_launch_dependents();   // (the overflow kernel's CTAs cannot share an SM with this one: they queue behind it)
   for (int j = tid; j <= nkeys; j += T2_THREADS(D)) B[j] = __ldg(a.seg_off + j);
   {   // screen images: already in the shared-memory layout
     const int nf4 = nch * (KS / 8) * 256;
@@ -716,6 +724,9 @@ __global__ void __launch_bounds__(T2_THREADS(D), 1) gauss_label_tc2_kernel(const
           } else {
             a.labels[idx] = lab;
             atomicAdd(&hs[lab], 1);
+            // (the tile's sort key is the old label of its points; the compiler aggregates this atomic over the warp,
+            // and a counter kept across the tile loop would cost the loop spill traffic)
+            if (lab != w.key) atomicAdd(a.moved, 1);
           }
           ++npts_total;
         }
@@ -895,7 +906,11 @@ struct GaussListArgs {
   int64_t goff;
   int final_iter;
   int32_t* stats;          // optional [2]: [1] += K per listed point
-  int32_t* zero_next;      // optional [4]: the counter set of the NEXT call, cleared here (no memset launches)
+  int32_t* moved;          // [1] += listed points whose label changed
+  int32_t* zero_next;      // optional [T2_CTR_SET]: the counter set of the NEXT call, cleared here (no memset launches)
+  int32_t* zero_hist;      // optional [zero_hist_n]: the histogram buffer of the NEXT call, cleared here
+  int zero_hist_n;
+  int32_t* hstat;          // optional [3]: mapped host memory, receives stats[0], stats[1], *count from the last block
   // optional: the last block to finish turns the completed label histogram into the segment offsets and cursors of the
   // sort (what label_scan_kernel does), saving its launch.  ticket: zero on entry, reset on exit.
   int32_t* ticket;
@@ -909,8 +924,11 @@ template <int D>
 __global__ void __launch_bounds__(256) gauss_label_list_kernel(const GaussListArgs a) {
   extern __shared__ float gl_rs[];   // [8][K]
   const int lane = threadIdx.x & 31, wl = threadIdx.x >> 5;
+  pdl_wait();
+  pdl_launch_dependents();
   const int nlist = *a.count;
-  if (a.zero_next != nullptr && blockIdx.x == 0 && threadIdx.x < 4) a.zero_next[threadIdx.x] = 0;
+  if (a.zero_next != nullptr && blockIdx.x == 0 && threadIdx.x < T2_CTR_SET) a.zero_next[threadIdx.x] = 0;
+  for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < a.zero_hist_n; k += gridDim.x * blockDim.x) a.zero_hist[k] = 0;
   float* rs = gl_rs + (size_t)wl * a.K;
   for (int e = blockIdx.x * 8 + wl; e < nlist; e += gridDim.x * 8) {
     const int32_t idx = a.list[e];
@@ -929,6 +947,7 @@ __global__ void __launch_bounds__(256) gauss_label_list_kernel(const GaussListAr
         const double u = dpmm_uniform(a.u_inj, idx, a.seed, DPMM_STREAM_LABEL, a.call, (uint64_t)(a.goff + idx));
         lab = dpmm_draw_inverse_cdf(rs, 1, a.K, u);
       }
+      if (a.moved != nullptr && a.labels[idx] != lab) atomicAdd(a.moved, 1);
       a.labels[idx] = lab;
       atomicAdd(a.hist + lab, 1);
       if (a.stats != nullptr) atomicAdd(&a.stats[1], a.K);
@@ -975,6 +994,12 @@ __global__ void __launch_bounds__(256) gauss_label_list_kernel(const GaussListAr
       if (threadIdx.x == 0) {
         a.seg_off[a.scan_k] = carry;
         *a.ticket = 0;
+        if (a.hstat != nullptr) {   // the host's path choice reads these once the event behind this kernel has fired
+          a.hstat[0] = __ldcg(a.stats + 0);
+          a.hstat[1] = __ldcg(a.stats + 1);
+          a.hstat[2] = __ldcg(a.count);
+          __threadfence_system();
+        }
       }
     }
   }

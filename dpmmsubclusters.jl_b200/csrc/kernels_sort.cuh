@@ -70,13 +70,21 @@ __global__ void label_scan_kernel(const int32_t* __restrict__ hist, int K, int32
 // and reserves one contiguous range per (CTA, label) with a single global atomic.
 #define SCATTER_PPT 8
 // `zero` / `zero2` (optional): buffers the NEXT kernel expects cleared (the statistics accumulators and left
-// counts of the fused sub-label + statistics kernel) -- cleared here instead of by two memset launches.
+// counts of the fused sub-label + statistics kernel) -- cleared here instead of by two memset launches; `zero3`
+// (optional): one more double, the risk counter of the statistics finalise that follows the fused kernel.
+// `moved` (optional): the number of points whose label changed since `perm` was last sorted.  When it is 0, perm
+// is still a valid sort of the labels (the order inside a bucket is arbitrary anyway: ranks come from atomics) and
+// the cursors, which only the scatter consumes, keep their scan: the kernel only clears the buffers above.
 __global__ void label_scatter_kernel(const int32_t* __restrict__ labels, int64_t n, int K,
                                      int32_t* cursor, int32_t* perm, double* zero, int64_t nzero,
-                                     int32_t* zero2, int nzero2) {
+                                     int32_t* zero2, int nzero2, double* zero3, const int32_t* moved) {
   extern __shared__ int sm[];
+  pdl_wait();
+  pdl_launch_dependents();
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < nzero; e += (int64_t)gridDim.x * blockDim.x) zero[e] = 0.0;
   for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < nzero2; e += gridDim.x * blockDim.x) zero2[e] = 0;
+  if (zero3 != nullptr && blockIdx.x == 0 && threadIdx.x == 0) *zero3 = 0.0;
+  if (moved != nullptr && *moved == 0) return;
   int* cnt = sm;
   int* basev = sm + K;
   const int T = blockDim.x, tid = threadIdx.x;

@@ -447,6 +447,8 @@ __global__ void stats_finalize_kernel(const double* __restrict__ acc, const int3
                                       const int32_t* __restrict__ lr_cursor, const int32_t* __restrict__ idx_list,
                                       int m, int D, int rec, int niw, double* out, const float* __restrict__ centers,
                                       const int32_t* __restrict__ lcount, double* risk) {
+  pdl_wait();
+  pdl_launch_dependents();
   const int a = blockIdx.y;
   if (a >= m) return;
   const int k = idx_list != nullptr ? idx_list[a] : a;   // no list: every cluster in order

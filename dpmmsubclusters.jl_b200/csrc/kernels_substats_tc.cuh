@@ -148,8 +148,7 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int nkeys = a.K;
 
-  // ---- cluster boundaries, triangle index table, constant operands ----
-  for (int j = tid; j <= nkeys; j += SS_THREADS) B[j] = __ldg(a.seg_off + j);
+  // ---- triangle index table, constant operands, barriers, tensor memory: CTA-local, before the grid dependency ----
   for (int e = tid; e < 1024; e += SS_THREADS) {
     const int i = e >> 5, j = e & 31;
     if (j >= i) tri[i * 32 - (i * (i - 1)) / 2 + (j - i)] = (uint16_t)((i << 8) | j);
@@ -159,9 +158,6 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
     float* baug = reinterpret_cast<float*>(wslot + 16384);
     for (int e = tid; e < 512; e += SS_THREADS) baug[e] = 0.f;
   }
-  if (blockIdx.x == 0)
-    for (int e = tid; e < 2 * nkeys * SS_D; e += SS_THREADS)
-      a.centers[e] = __ldg(a.cen + (size_t)(e >> 6) * SS_D + (e & 31));
   if (tid == 0) {
     for (int b = 0; b < SS_NTB; ++b) {
       tc::mbar_init(&d1full[b], 1);
@@ -185,6 +181,17 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
     tc::mbar_init(wempty, 1);
     tc::fence_barrier_init();
   }
+  // Allocated before the grid dependency, possibly while CTAs of the previous kernel still run: safe because no CTA
+  // that holds tensor memory can share an SM with this one (896 threads use nearly the whole register file; checked
+  // on the host by sweep_pdl_ok, which otherwise launches this kernel without PDL).
+  if (warp == 4) tc::tmem_alloc(tmem_slot, SS_TMEM_COLS);
+  pdl_wait();
+  pdl_launch_dependents();   // (the finalise kernel's CTAs cannot share an SM with this one: they queue behind it)
+  // ---- cluster boundaries, centres ----
+  for (int j = tid; j <= nkeys; j += SS_THREADS) B[j] = __ldg(a.seg_off + j);
+  if (blockIdx.x == 0)
+    for (int e = tid; e < 2 * nkeys * SS_D; e += SS_THREADS)
+      a.centers[e] = __ldg(a.cen + (size_t)(e >> 6) * SS_D + (e & 31));
   __syncthreads();
   for (int r = tid; r < SS_TILE; r += SS_THREADS) {   // bias k-step A operand: (1, 1, 0, ...) per row
     float* p = aaug + (r >> 3) * 64 + (r & 7) * 4;
@@ -206,7 +213,6 @@ __global__ void __launch_bounds__(SS_THREADS, 1) niw_substats_tc_kernel(const Su
       carry += __shfl_sync(0xffffffffu, v, 31);
     }
   }
-  if (warp == 4) tc::tmem_alloc(tmem_slot, SS_TMEM_COLS);
   tc::fence_proxy_async();
   tc::tc_fence_before();
   __syncthreads();

@@ -316,6 +316,14 @@ class GpuSweep:
         self._ck(self.lib.dpmm_debug_tc_stats(self.h, _ptr(out, C.c_int64)))
         return (int(out[0]), int(out[1]), int(out[2])) if overflow else (int(out[0]), int(out[1]))
 
+    def sort_state(self):
+        """(perm: point indices in the order of the current label sort, points whose label changed in the last
+        tensor-core label call)."""
+        perm = np.empty(self.n, np.int32)
+        moved = np.zeros(1, np.int64)
+        self._ck(self.lib.dpmm_debug_sort(self.h, _ptr(perm, C.c_int32), _ptr(moved, C.c_int64)))
+        return perm, int(moved[0])
+
     def fused_stats(self):
         """(fused sub-label+statistics launches, suff_stats calls served from them, exact recomputations)."""
         out = np.zeros(3, np.int64)

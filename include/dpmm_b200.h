@@ -227,6 +227,10 @@ int dpmm_debug_loglik(dpmm_ctx* ctx, int32_t which, float* out);
  * out[2] = points of that call finished by the full-K overflow kernel (NaN screen values or more than
  * 7 candidate clusters; D = 32 / 64 path). */
 int dpmm_debug_tc_stats(dpmm_ctx* ctx, int64_t* out3);
+/* Label sort diagnostics: perm (n_local entries, or NULL) receives the point indices in the order of the current
+ * label sort (sorting first if needed), moved[0] the number of points whose label changed in the last dpmm_sample_labels
+ * that ran on the D = 32 / 64 tensor-core path (the sort after such a call skips its scatter when it is 0). */
+int dpmm_debug_sort(dpmm_ctx* ctx, int32_t* perm, int64_t* moved);
 /* Fused sub-label + statistics path diagnostics (NIW, D = 32): out[0] = launches of the fused kernel by
  * dpmm_sample_sublabels, out[1] = dpmm_suff_stats calls served from its accumulators, out[2] = calls that
  * fell back to the separate statistics kernel because a run lay far from its cluster's centre. */
