@@ -24,6 +24,7 @@ _f32p, _f64p, _i64p, _u8p = (C.POINTER(C.c_float), C.POINTER(C.c_double), C.POIN
 # name -> (restype, argtypes); exactly the symbols include/dpmm_b200.h declares
 SIGNATURES = {
     "dpmm_create": (C.c_int, [C.POINTER(_p), _f32p, _i64, _i32, _i32, _i32, _u64, _i64]),
+    "dpmm_create_sparse": (C.c_int, [C.POINTER(_p), _i64p, _i64p, _f32p, _i64, _i32, _i32, _u64, _i64]),
     "dpmm_destroy": (C.c_int, [_p]),
     "dpmm_last_error": (C.c_char_p, [_p]),
     "dpmm_set_stream": (C.c_int, [_p, _p]),

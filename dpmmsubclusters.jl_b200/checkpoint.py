@@ -28,7 +28,12 @@ FORMAT = 1
 
 # ------------------------------------------------------------------------------------------- data ----------
 def load_data(path, prefix="", swapDimension=True):
-    """utils.jl:5-14."""
+    """utils.jl:5-14.  Also reads `path + prefix + ".npz"` written by scipy.sparse.save_npz when there is no ".npy":
+    an N x D sparse matrix like the reference's array, returned as CSC (D x N when swapDimension)."""
+    if not os.path.exists(path + prefix + ".npy") and os.path.exists(path + prefix + ".npz"):
+        import scipy.sparse as sps
+        m = sps.load_npz(path + prefix + ".npz")
+        return sps.csc_matrix(m.T if swapDimension else m)
     arr = np.load(path + prefix + ".npy")
     if np.issubdtype(arr.dtype, np.floating):
         arr = np.where(np.isnan(arr), 0.0, arr)

@@ -71,7 +71,13 @@ struct dpmm_ctx {
   int sampler = 0;
   std::string err;
 
-  float* x = nullptr;
+  float* x = nullptr;              // dense points [n][D]; NULL for a sparse context
+  // sparse context (dpmm_create_sparse, multinomial): the points as compressed rows, see kernels_mnm_sparse.cuh
+  bool sparse = false;
+  int64_t nnz = 0;
+  int64_t* sp_ptr = nullptr;       // [n + 1]
+  int32_t* sp_idx = nullptr;       // [nnz]
+  float* sp_val = nullptr;         // [nnz]
   int32_t* labels = nullptr;
   uint8_t* sub = nullptr;
   int32_t* perm = nullptr;

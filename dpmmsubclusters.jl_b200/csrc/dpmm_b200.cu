@@ -18,6 +18,7 @@
 #include "kernels_gauss_tc2.cuh"
 #include "kernels_ipc.cuh"
 #include "kernels_mnm.cuh"
+#include "kernels_mnm_sparse.cuh"
 #include "kernels_mnm_tc.cuh"
 #include "kernels_pack.cuh"
 #include "kernels_params.cuh"
@@ -357,6 +358,101 @@ extern "C" int dpmm_create(dpmm_ctx** out, const float* x, int64_t n_local, int3
   return 0;
 }
 
+extern "C" int dpmm_create_sparse(dpmm_ctx** out, const int64_t* colptr, const int64_t* rowval, const float* nzval,
+                                  int64_t n_local, int32_t d, int32_t device, uint64_t seed, int64_t global_offset) {
+  dpmm_ctx* ctx = nullptr;
+  if (!out) return fail(nullptr, DPMM_EINVAL, "out is NULL");
+  *out = nullptr;
+  NEED(colptr != nullptr && n_local > 0 && d > 0, DPMM_EINVAL, "colptr must be non-NULL with n_local > 0 and d > 0");
+  NEED(n_local < ((int64_t)1 << 31) - 4096, DPMM_ELIMIT, "n_local must fit in int32 (shard the points over more GPUs)");
+  NEED(d <= DPMM_MNM_MAX_D, DPMM_ELIMIT, "multinomial: D must be <= 16384");
+  NEED(colptr[0] == 1, DPMM_EINVAL, "colptr[0] must be 1 (1-based compressed columns)");
+  const int64_t nnz = colptr[n_local] - 1;
+  NEED(nnz >= 0, DPMM_EINVAL, "colptr[n_local] must be >= 1 (nnz = colptr[n_local] - 1)");
+  NEED(nnz == 0 || (rowval != nullptr && nzval != nullptr), DPMM_EINVAL, "rowval and nzval must be non-NULL when nnz > 0");
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+    return fail(nullptr, DPMM_ECUDA, "no CUDA device: libdpmm_b200 has no CPU fallback");
+  NEED(device >= 0 && device < ndev, DPMM_EINVAL, "bad device ordinal");
+  ctx = new dpmm_ctx();
+  ctx->device = device;
+  ctx->n = n_local;
+  ctx->D = ctx->D_user = d;
+  ctx->prior = DPMM_PRIOR_MULTINOMIAL;
+  ctx->seed = seed;
+  ctx->goff = global_offset;
+  ctx->sparse = true;
+  ctx->nnz = nnz;
+  ctx->chunk = 256;
+  int64_t* dcol = nullptr;
+  int64_t* drow = nullptr;
+  unsigned long long* dbad = nullptr;
+  auto bail = [&](int code) {
+    if (dcol) cudaFree(dcol);
+    if (drow) cudaFree(drow);
+    if (dbad) cudaFree(dbad);
+    g_err = ctx->err;
+    dpmm_destroy(ctx);
+    return code;
+  };
+#define CKC(call)                                                                        \
+  do {                                                                                   \
+    cudaError_t e__ = (call);                                                            \
+    if (e__ != cudaSuccess) {                                                            \
+      ctx->err = std::string(#call) + ": " + cudaGetErrorString(e__);                    \
+      return bail(DPMM_ECUDA);                                                           \
+    }                                                                                    \
+  } while (0)
+  CKC(cudaSetDevice(device));
+  cudaDeviceProp prop;
+  CKC(cudaGetDeviceProperties(&prop, device));
+  if (prop.major < 10) {
+    ctx->err = "device is not sm_100-class (Blackwell); this library ships sm_100a code only";
+    return bail(DPMM_ECUDA);
+  }
+  ctx->sm_count = prop.multiProcessorCount;
+  ctx->smem_optin = (int)prop.sharedMemPerBlockOptin;
+  ctx->smem_per_sm = (int)prop.sharedMemPerMultiprocessor;
+  CKC(cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
+  CKC(cudaMalloc((void**)&ctx->sp_ptr, (size_t)(n_local + 1) * sizeof(int64_t)));
+  CKC(cudaMalloc((void**)&ctx->sp_idx, (size_t)std::max<int64_t>(nnz, 1) * sizeof(int32_t)));
+  CKC(cudaMalloc((void**)&ctx->sp_val, (size_t)std::max<int64_t>(nnz, 1) * sizeof(float)));
+  CKC(cudaMalloc((void**)&ctx->labels, (size_t)n_local * sizeof(int32_t)));
+  CKC(cudaMalloc((void**)&ctx->sub, (size_t)n_local));
+  CKC(cudaMalloc((void**)&ctx->perm, (size_t)n_local * sizeof(int32_t)));
+  CKC(cudaMalloc((void**)&ctx->perm2, (size_t)n_local * sizeof(int32_t)));
+  CKC(cudaMalloc((void**)&ctx->item_ctr, 2 * sizeof(int32_t)));
+  CKC(cudaMalloc((void**)&dcol, (size_t)(n_local + 1) * sizeof(int64_t)));
+  CKC(cudaMalloc((void**)&drow, (size_t)std::max<int64_t>(nnz, 1) * sizeof(int64_t)));
+  CKC(cudaMalloc((void**)&dbad, sizeof(unsigned long long)));
+  CKC(cudaMemcpyAsync(dcol, colptr, (size_t)(n_local + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream));
+  if (nnz > 0) {
+    CKC(cudaMemcpyAsync(drow, rowval, (size_t)nnz * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream));
+    CKC(cudaMemcpyAsync(ctx->sp_val, nzval, (size_t)nnz * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+  }
+  CKC(cudaMemsetAsync(dbad, 0xff, sizeof(unsigned long long), ctx->stream));
+  mnm_sparse_convert_kernel<<<(unsigned)std::min<int64_t>((n_local + 255) / 256, (int64_t)ctx->sm_count * 8), 256, 0,
+                              ctx->stream>>>(dcol, drow, n_local, nnz, d, ctx->sp_ptr, ctx->sp_idx, dbad);
+  CKC(cudaGetLastError());
+  unsigned long long bad = 0;
+  CKC(cudaMemcpyAsync(&bad, dbad, sizeof(bad), cudaMemcpyDeviceToHost, ctx->stream));
+  CKC(cudaMemsetAsync(ctx->labels, 0, (size_t)n_local * sizeof(int32_t), ctx->stream));
+  CKC(cudaMemsetAsync(ctx->sub, 0, (size_t)n_local, ctx->stream));
+  CKC(cudaStreamSynchronize(ctx->stream));
+#undef CKC
+  if (bad != ~0ull) {
+    static const char* const why[3] = {"colptr decreases or leaves [1, nnz + 1]", "a row index outside [1, d]",
+                                       "row indices not strictly increasing (unsorted or duplicate)"};
+    ctx->err = "sparse input: column " + std::to_string(bad / 4 + 1) + " (1-based) is invalid: " + why[bad % 4];
+    return bail(DPMM_EINVAL);
+  }
+  cudaFree(dcol);
+  cudaFree(drow);
+  cudaFree(dbad);
+  *out = ctx;
+  return 0;
+}
+
 extern "C" int dpmm_destroy(dpmm_ctx* ctx) {
   if (!ctx) return 0;
   cudaSetDevice(ctx->device);
@@ -380,7 +476,7 @@ extern "C" int dpmm_destroy(dpmm_ctx* ctx) {
     cudaEventDestroy(t.b);
   }
   for (auto e : ctx->ev_pool) cudaEventDestroy(e);
-  void* ptrs[] = {ctx->x, ctx->labels, ctx->sub, ctx->perm, ctx->perm2, ctx->u_label, ctx->u_sub, ctx->r_bits,
+  void* ptrs[] = {ctx->x, ctx->sp_ptr, ctx->sp_idx, ctx->sp_val, ctx->labels, ctx->sub, ctx->perm, ctx->perm2, ctx->u_label, ctx->u_sub, ctx->r_bits,
                   ctx->raw_params, ctx->recs, ctx->cst, ctx->logw, ctx->loglr, ctx->logp_t, ctx->t2_piv, ctx->t2_scr, ctx->t2_u, ctx->t2_bias, ctx->t2_fro8, ctx->ctr_sets, ctx->tc_w, ctx->tc_b, ctx->tc_mu, ctx->tc_fro, ctx->ss_w, ctx->ss_b, ctx->ss_c, ctx->lcount, ctx->mtc_w, ctx->hist_mem, ctx->seg_off,
                   ctx->scat_cursor, ctx->lr_cursor, ctx->lut_l, ctx->lut_r, ctx->rule, ctx->wanted,
                   ctx->idx_list, ctx->acc, ctx->centers, ctx->outbuf, ctx->items, ctx->item_ctr, ctx->hyper_d, ctx->ptab,
@@ -980,6 +1076,40 @@ static int launch_mnm_label_stream(dpmm_ctx* ctx, MnmLabelArgs& a) {
   return 0;
 }
 
+// K3 on sparse points (kernels_mnm_sparse.cuh): the largest point tile whose [K][TP] parr slice fits shared memory,
+// with the [D][KP] table staged there too when it fits beside the slice
+template <int W, int KR>
+static int launch_mnm_sparse_label_w(dpmm_ctx* ctx, MnmSparseLabelArgs& a) {
+  const size_t base = ((size_t)a.K * a.TP + a.K) * 4, tab = (size_t)a.D * a.KP * 4;
+  a.tab_smem = base + tab <= (size_t)ctx->smem_optin;
+  const size_t sm = base + (a.tab_smem ? tab : 0);
+  CK(cudaFuncSetAttribute(mnm_sparse_label_kernel<W, KR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+  int occ = 1;
+  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, mnm_sparse_label_kernel<W, KR>, MNM_SP_THREADS, sm));
+  occ = std::max(occ, 1);
+  const int64_t grid = std::min<int64_t>(a.ntiles, (int64_t)ctx->sm_count * occ);
+  KernelTimer kt(ctx, TK_LABEL);
+  mnm_sparse_label_kernel<W, KR><<<(unsigned)grid, MNM_SP_THREADS, sm, ctx->stream>>>(a);
+  CK(cudaGetLastError());
+  return 0;
+}
+static int launch_mnm_sparse_label(dpmm_ctx* ctx, int final_iter, float* dump) {
+  const int K = ctx->K;
+  MnmSparseLabelArgs a{};
+  a.sp = MnmSparse{ctx->sp_ptr, ctx->sp_idx, ctx->sp_val};
+  a.n = ctx->n; a.D = ctx->D; a.K = K; a.KP = ctx->KP; a.logp_t = ctx->logp_t; a.logw = ctx->logw;
+  a.labels = ctx->labels; a.hist = ctx->hist; a.u_inj = ctx->u_label; a.seed = ctx->seed; a.call = ctx->call;
+  a.goff = ctx->goff; a.final_iter = final_iter; a.sampler = ctx->sampler; a.dump = dump;
+  a.TP = 256;
+  while (a.TP > 32 && ((size_t)K * a.TP + K) * 4 > (size_t)ctx->smem_optin) a.TP /= 2;
+  a.ntiles = (a.n + a.TP - 1) / a.TP;
+  if (K > 32) return launch_mnm_sparse_label_w<32, 4>(ctx, a);
+  if (K > 16) return launch_mnm_sparse_label_w<32, 1>(ctx, a);
+  if (K > 8) return launch_mnm_sparse_label_w<16, 1>(ctx, a);
+  if (K > 4) return launch_mnm_sparse_label_w<8, 1>(ctx, a);
+  return launch_mnm_sparse_label_w<4, 1>(ctx, a);
+}
+
 static int run_sample_labels(dpmm_ctx* ctx, int final_iter, float* dump) {
   NEED(ctx->params_set, DPMM_ESTATE, "set_params must precede sample_labels");
   const int K = ctx->K;
@@ -1048,6 +1178,9 @@ static int run_sample_labels(dpmm_ctx* ctx, int final_iter, float* dump) {
     a.labels = ctx->labels; a.hist = ctx->hist; a.u_inj = ctx->u_label; a.seed = ctx->seed; a.call = ctx->call;
     a.goff = ctx->goff; a.final_iter = final_iter; a.sampler = ctx->sampler; a.dump = dump;
     int rc = niw_launch_label(ctx, a);
+    if (rc) return rc;
+  } else if (ctx->sparse) {
+    int rc = launch_mnm_sparse_label(ctx, final_iter, dump);
     if (rc) return rc;
   } else if (ctx->mtc_params && dump == nullptr && env_int("DPMM_LABEL_TC", 1) != 0) {
     // K3 on tcgen05: exact TF32 3-way split GEMM of counts x log-probabilities
@@ -1210,7 +1343,10 @@ static int run_sublabels(dpmm_ctx* ctx, bool sample, float* dump) {
     const int T = 128;
     const unsigned grid = (unsigned)((a.n + T - 1) / T);
     KernelTimer kt(ctx, TK_SUBLABEL);
-    if (sample && ctx->D <= 128)
+    if (sample && ctx->sparse)
+      mnm_sparse_sublabel_kernel<<<(unsigned)((a.n + MNM_SPS_T - 1) / MNM_SPS_T), MNM_SPS_T, 0, ctx->stream>>>(
+          a, MnmSparse{ctx->sp_ptr, ctx->sp_idx, ctx->sp_val});
+    else if (sample && ctx->D <= 128)
       mnm_sublabel2_kernel<<<grid, T, 0, ctx->stream>>>(a);
     else if (sample && ctx->D > 1024)
       mnm_sublabel_staged_kernel<<<grid, MNM_SLS_T, 0, ctx->stream>>>(a);
@@ -1346,6 +1482,15 @@ static int stats_compute(dpmm_ctx* ctx, const int64_t* indices, int32_t n_indice
   } else if (ctx->prior == DPMM_PRIOR_NIW) {
     rc = niw_launch_stats(ctx, sa);
     if (rc) return rc;
+  } else if (ctx->sparse) {
+    const size_t smem = (size_t)D * 4;
+    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(mnm_sparse_stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int occ = 1;
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, mnm_sparse_stats_kernel, 256, smem));
+    occ = std::max(occ, 1);
+    KernelTimer kt(ctx, TK_STATS);
+    mnm_sparse_stats_kernel<<<ctx->sm_count * occ, 256, smem, ctx->stream>>>(sa, MnmSparse{ctx->sp_ptr, ctx->sp_idx, ctx->sp_val});
+    CK(cudaGetLastError());
   } else {
     const auto kern = D > 32 * MNM_STATS_NREG ? mnm_stats_kernel<true> : mnm_stats_kernel<false>;
     int occ = 1;
@@ -1835,11 +1980,16 @@ extern "C" int dpmm_predict_multinomial(dpmm_ctx* ctx, int32_t K, const double* 
   CKP(cudaMemcpyAsync(dlw, logw, (size_t)K * 4, cudaMemcpyHostToDevice, ctx->stream));
   MnmScoreArgs sa{};
   sa.x = ctx->x; sa.n = n; sa.D = D; sa.K = K; sa.KC = KC; sa.logp = dlp; sa.logw = dlw; sa.score = dscore;
-  if (sm > 48 * 1024) CKP(cudaFuncSetAttribute(mnm_score_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+  if (sm > 48 * 1024) CKP(cudaFuncSetAttribute(ctx->sparse ? (const void*)mnm_sparse_score_kernel : (const void*)mnm_score_kernel,
+                                               cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
   {
     KernelTimer kt(ctx, TK_LABEL, 2);
     const unsigned gx = (unsigned)std::min<int64_t>((n + 7) / 8, (int64_t)ctx->sm_count * 8);
-    mnm_score_kernel<<<dim3(gx, (unsigned)((K + KC - 1) / KC)), 256, sm, ctx->stream>>>(sa);
+    if (ctx->sparse)
+      mnm_sparse_score_kernel<<<dim3(gx, (unsigned)((K + KC - 1) / KC)), 256, sm, ctx->stream>>>(
+          sa, MnmSparse{ctx->sp_ptr, ctx->sp_idx, ctx->sp_val});
+    else
+      mnm_score_kernel<<<dim3(gx, (unsigned)((K + KC - 1) / KC)), 256, sm, ctx->stream>>>(sa);
     CKP(cudaGetLastError());
     mnm_predict_finish_kernel<<<(unsigned)std::min<int64_t>((n + 255) / 256, (int64_t)ctx->sm_count * 8), 256, 0,
                                 ctx->stream>>>(dscore, n, K, dlab, probs != nullptr);

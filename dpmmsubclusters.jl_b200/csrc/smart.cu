@@ -106,6 +106,7 @@ extern "C" int dpmm_smart_project(dpmm_ctx* ctx, int64_t cluster, const double* 
   NEED(ctx, DPMM_EINVAL, "ctx is NULL");
   NEED(v && mu && lo_hi && count, DPMM_EINVAL, "NULL argument");
   NEED(cluster >= 1 && cluster <= DPMM_MAX_K, DPMM_EINVAL, "cluster index out of range");
+  NEED(ctx->x != nullptr, DPMM_ESTATE, "smart splits project the dense points: a sparse context has none");
   CK(cudaSetDevice(ctx->device));
   if (!ctx->smart) ctx->smart = new SmartState();
   SmartState* s = ctx->smart;

@@ -16,12 +16,19 @@ import time
 from dataclasses import dataclass, field
 
 import numpy as np
+import scipy.sparse as sps
 from scipy.special import gammaln
 
 from . import priors as P
 from .sweep import GpuSweep, NIW, MULTINOMIAL
 
 F32 = np.float32
+
+
+def _points(x):
+    """The points as the sweep takes them: scipy.sparse matrices pass through (multinomial prior only; the sweep converts
+    them to 1-based CSC once), everything else becomes a Float32 array."""
+    return x if sps.issparse(x) else np.asarray(x, F32)
 
 
 # ---------------------------------------------------------------- data structures (src/ds.jl) ----
@@ -407,7 +414,7 @@ def calculate_posterior(model):
 def init_model_from_data(all_data, hyper_params, α, cfg, seed, sweep_factory, shard):
     """init_model_from_data :36-53: `distribute(all_data)` + random labels become dpmm_create +
     dpmm_init_labels.  `shard` = (global_offset, n_total) when the points are one shard of many."""
-    all_data = np.asarray(all_data, F32)
+    all_data = _points(all_data)
     kind = NIW if isinstance(hyper_params, P.niw_hyperparams) else MULTINOMIAL
     goff, n_total = shard if shard is not None else (0, all_data.shape[1])
     sweep_seed = int(seed) if seed is not None else int(np.random.default_rng().integers(2 ** 62))
@@ -535,6 +542,8 @@ def dp_parallel(all_data, local_hyper_params=None, α_param=None, iters=100, ini
         raise NotImplementedError("the outlier component is out of scope (DESIGN.md 6)")
     if save_model and save_path is None:
         raise ValueError("save_model=True needs save_path (global_params.jl:37 in the reference)")
+    if sps.issparse(all_data) and isinstance(local_hyper_params, P.niw_hyperparams):
+        raise ValueError("sparse points are supported for the multinomial prior only")
     if smart_splits and not isinstance(local_hyper_params, P.niw_hyperparams):
         raise ValueError("smart splits are Gaussian only (dp-parallel-sampling.jl:111)")
     if (comm is not None or shard is not None) and seed is None:
@@ -602,7 +611,7 @@ def dp_parallel_params_file(model_params, verbose=True, gt=None, **kw):
     cfg.global_params = model_params
     if gp["hyper_params"] is None:
         raise ValueError("the parameter file must define hyper_params")
-    data = np.asarray(load_data(cfg.data_path, prefix=cfg.data_prefix), F32)      # init_model :24-25
+    data = _points(load_data(cfg.data_path, prefix=cfg.data_prefix))              # init_model :24-25
     return _run_from_settings(data, gp["hyper_params"], gp["α"], cfg, gp["random_seed"], kw.get("sweep_factory"),
                               kw.get("shard"), kw.get("comm"), kw.get("device", 0), kw.get("device_params"))
 
@@ -627,7 +636,7 @@ def run_model_from_checkpoint(filename, verbose=True, gt=None, data=None, **kw):
         seed = (gparams or {}).get("random_seed")
     if data is None:
         data = load_data(cfg.data_path, prefix=cfg.data_prefix)                   # :435
-    data = np.asarray(data, F32)
+    data = _points(data)
     return _run_from_settings(data, mh.distribution_hyper_params, mh.α, cfg, seed, kw.get("sweep_factory"), kw.get("shard"),
                               kw.get("comm"), kw.get("device", 0), kw.get("device_params"), restored=(grp, it))
 
@@ -637,8 +646,10 @@ def fit(all_data, *args, iters=100, init_clusters=1, seed=None, verbose=False, s
     """fit(all_data, [local_hyper_params,] α_param; ...) :215-293.  Returns the reference's tuple:
     (labels, clusters, weights, iter_count, nmi_score_history, likelihood_history, cluster_count_history,
      sub_labels, dp_model)."""
-    all_data = np.asarray(all_data, F32)
+    all_data = _points(all_data)
     if len(args) == 1:
+        if sps.issparse(all_data):
+            raise ValueError("sparse points need the multinomial prior: pass multinomial_hyper(...) and α")
         D = all_data.shape[0]
         hyper = P.niw_hyperparams(1.0, np.zeros(D), D + 3, np.eye(D))        # :272-274
         α = args[0]
@@ -657,8 +668,8 @@ def predict(dp_model, data, device=0, on_device=None):
     NIW models run on the GPU by default (dpmm_predict_niw: Student-t densities, argmax and softmax per point; the
     host prepares the K factors); multinomial models do with on_device=True (dpmm_predict_multinomial: the host
     prepares log(alpha'/sum alpha') in Float64).  on_device=False, or a multinomial model by default, takes the NumPy
-    formulas below."""
-    data = np.asarray(data, F32)
+    formulas below.  Sparse data (scipy.sparse, D x N) runs on a sparse context on the device and as x' logp in NumPy."""
+    data = _points(data)
     cl = dp_model.group.local_clusters
     posts = [c.cluster_params.cluster_params.posterior_hyperparams for c in cl]
     w = np.asarray(dp_model.group.weights, F32)

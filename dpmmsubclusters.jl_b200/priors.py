@@ -13,6 +13,7 @@ from __future__ import annotations
 from dataclasses import dataclass
 
 import numpy as np
+import scipy.sparse as sps
 from scipy.special import gammaln
 
 F32 = np.float32
@@ -168,6 +169,8 @@ def posterior_predictive(x, post):
     """posterior_predictive! niw.jl:68-76 (multivariate Student-t log-density) and
     multinomial_prior.jl:45-48.  x is D x n; returns Float64[n].  Host-only (predict)."""
     if isinstance(post, niw_hyperparams):
+        if sps.issparse(x):
+            raise ValueError("sparse points are supported for the multinomial prior only")
         ν, ψ, κ, m = post.ν, post.ψ, post.κ, post.m
         D = m.shape[0]
         df = ν - D + 1
@@ -178,4 +181,8 @@ def posterior_predictive(x, post):
         return (gammaln((df + D) / 2) - gammaln(df / 2) - 0.5 * D * np.log(df * np.pi)
                 - 0.5 * np.linalg.slogdet(Sig)[1] - 0.5 * (df + D) * np.log1p(q / df))
     a = post.α.astype(np.float64)
+    if sps.issparse(x):   # zero counts contribute nothing (stored or not), as in the sparse device kernels
+        xt = sps.csr_matrix(x.T, dtype=np.float64, copy=True)
+        xt.eliminate_zeros()
+        return np.asarray(xt @ np.log(a / a.sum())).reshape(-1)
     return np.log(a / a.sum()) @ np.asarray(x, np.float64)

@@ -10,6 +10,7 @@ from __future__ import annotations
 import ctypes as C
 
 import numpy as np
+import scipy.sparse as sps
 
 from . import _lib as L
 
@@ -25,11 +26,24 @@ def _i64(a):
     return np.ascontiguousarray(np.asarray(a, dtype=np.int64))
 
 
+def csc_1based(x):
+    """The arrays of a Julia SparseMatrixCSC{Float32,Int64} for a scipy.sparse matrix x of shape (D, N): column j is
+    point j; duplicates summed, row indices sorted within each column, 1-based int64 colptr / rowval, float32 nzval."""
+    x = sps.csc_matrix(x, dtype=np.float32, copy=True)
+    x.sum_duplicates()          # (also sorts the row indices of every column)
+    return (x.indptr.astype(np.int64) + 1, x.indices.astype(np.int64) + 1, np.ascontiguousarray(x.data, np.float32))
+
+
 class GpuSweep:
-    """The worker side of the sampler on one B200 (src/local_clusters_actions.jl *_worker!)."""
+    """The worker side of the sampler on one B200 (src/local_clusters_actions.jl *_worker!).  x: D x N points, dense
+    (any array-like) or, for the multinomial prior, any scipy.sparse matrix (dpmm_create_sparse)."""
 
     def __init__(self, x, prior_kind, seed=0, global_offset=0, device=0):
         self.lib = L.load()
+        self.sparse = sps.issparse(x)
+        if self.sparse:
+            self._init_sparse(x, prior_kind, seed, global_offset, device)
+            return
         x = np.asarray(x, dtype=np.float32)
         if x.ndim != 2:
             raise ValueError("x must be D x N")
@@ -42,6 +56,22 @@ class GpuSweep:
         h = C.c_void_p()
         rc = self.lib.dpmm_create(C.byref(h), _ptr(xt, C.c_float), self.n, self.D, self.prior_kind, int(device),
                                   C.c_uint64(int(seed) & (2 ** 64 - 1)), int(global_offset))
+        L.check(rc, None)
+        self.h = h
+
+    def _init_sparse(self, x, prior_kind, seed, global_offset, device):
+        if int(prior_kind) != MULTINOMIAL:
+            raise ValueError("sparse points are supported for the multinomial prior only")
+        if len(x.shape) != 2:
+            raise ValueError("x must be D x N")
+        self.D, self.n = int(x.shape[0]), int(x.shape[1])
+        self.prior_kind = MULTINOMIAL
+        self.K = 0
+        colptr, rowval, nzval = csc_1based(x)
+        h = C.c_void_p()
+        rc = self.lib.dpmm_create_sparse(C.byref(h), _ptr(colptr, C.c_int64), _ptr(rowval, C.c_int64), _ptr(nzval, C.c_float),
+                                         self.n, self.D, int(device), C.c_uint64(int(seed) & (2 ** 64 - 1)),
+                                         int(global_offset))
         L.check(rc, None)
         self.h = h
 

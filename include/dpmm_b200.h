@@ -17,7 +17,8 @@
  *     102-109 -- a stream gives the same semantics).  Calls that return data synchronise.
  *   - labels and sub-labels cross the boundary as 1-based int64 (Julia Int64, ds.jl:54-55);
  *     cluster indices in index lists are 1-based int64 as well.
- *   - points are float32, D x N column-major (each point = D contiguous floats, ds.jl:53).
+ *   - points are float32, D x N column-major (each point = D contiguous floats, ds.jl:53), or, for the
+ *     multinomial prior, sparse compressed columns (dpmm_create_sparse).
  *   - host buffers are borrowed for the duration of the call only (x is copied at create).
  *   - there is NO CPU fallback: without a CUDA device every call fails with DPMM_ECUDA.
  */
@@ -56,6 +57,22 @@ typedef struct dpmm_ctx dpmm_ctx;
  * DPMM_ELIMIT.  Every multinomial d samples with any K up to DPMM_MAX_K. */
 int dpmm_create(dpmm_ctx** out, const float* x, int64_t n_local, int32_t d, int32_t prior_kind,
                 int32_t device, uint64_t seed, int64_t global_offset);
+/* init_model_from_data for ONE shard of sparse counts: the three arrays of a Julia SparseMatrixCSC{Float32,Int64}
+ * of size d x n_local (column j = point j), 1-based as Julia stores them.  Multinomial prior only.
+ *   colptr int64 [n_local + 1]  colptr[0] == 1, non-decreasing; nnz = colptr[n_local] - 1 >= 0
+ *   rowval int64 [nnz]          1..d, strictly increasing within a column
+ *   nzval  float32 [nnz]
+ * Empty columns and nnz = 0 are valid.  n_local, d, colptr[0] and nnz are checked on the host (d > 16384:
+ * DPMM_ELIMIT); the arrays are then copied to the device and checked there while they are converted to the internal
+ * layout (compressed rows: int64 offsets, int32 feature indices, float32 counts): a violation returns DPMM_EINVAL
+ * naming the first invalid column.  global_offset, device and seed as for dpmm_create.
+ * A sparse context has every entry point of a dense multinomial context holding the same matrix except the smart-split
+ * projection (dpmm_smart_project: DPMM_ESTATE).  Its log-likelihoods are the sequential Float32 fmaf chain over the
+ * stored entries in ascending feature order: bit for bit what the dense kernels compute over all D features, with
+ * one deliberate difference: a -Inf log-probability against a zero count (stored or not) contributes nothing, where
+ * the dense product gives NaN (0 * -Inf).  That is also what Julia's sparse `alpha' * x` gives for absent entries. */
+int dpmm_create_sparse(dpmm_ctx** out, const int64_t* colptr, const int64_t* rowval, const float* nzval,
+                       int64_t n_local, int32_t d, int32_t device, uint64_t seed, int64_t global_offset);
 int dpmm_destroy(dpmm_ctx* ctx);
 const char* dpmm_last_error(const dpmm_ctx* ctx);
 /* Use an externally owned cudaStream_t (e.g. the host framework's current stream) for all work. */

@@ -6,6 +6,8 @@
 # worker side of the sampler to the GPU; INTEGRATION.md lists the call sites.
 module DPMMSubClustersB200
 
+using SparseArrays: SparseMatrixCSC
+
 const lib = get(ENV, "DPMM_B200_LIB", "libdpmm_b200.so")
 
 const PRIOR_NIW = Cint(0)
@@ -37,6 +39,25 @@ function create(points::Matrix{Float32}, prior::Cint; device::Integer = 0, seed:
         (Ref{Ptr{Cvoid}}, Ptr{Cfloat}, Int64, Int32, Int32, Int32, UInt64, Int64),
         out, points, n, d, prior, device, UInt64(seed), global_offset))
     c = Ctx(out[], n, d, prior)
+    finalizer(x -> (x.ptr == C_NULL || ccall((:dpmm_destroy, lib), Cint, (Ptr{Cvoid},), x.ptr); x.ptr = C_NULL), c)
+    return c
+end
+
+"""
+    create(points::SparseMatrixCSC{Float32,Int64}; device=0, seed=0, global_offset=0)
+
+Sparse counts for the multinomial prior (dpmm_create_sparse): `colptr`, `rowval` and `nzval` go to the library as Julia
+stores them (1-based); the library validates them on the device.  Not exercised by this repository's tests (no Julia
+here); the same C entry point is tested from Python (`tests/test_gpu_mnm_sparse.py`).
+"""
+function create(points::SparseMatrixCSC{Float32,Int64}; device::Integer = 0, seed::Integer = 0, global_offset::Integer = 0)
+    out = Ref{Ptr{Cvoid}}(C_NULL)
+    d, n = size(points)
+    colptr, rowval, nzval = points.colptr, points.rowval, points.nzval
+    GC.@preserve colptr rowval nzval check(ccall((:dpmm_create_sparse, lib), Cint,
+        (Ref{Ptr{Cvoid}}, Ptr{Int64}, Ptr{Int64}, Ptr{Cfloat}, Int64, Int32, Int32, UInt64, Int64),
+        out, colptr, rowval, nzval, n, d, device, UInt64(seed), global_offset))
+    c = Ctx(out[], n, d, PRIOR_MULTINOMIAL)
     finalizer(x -> (x.ptr == C_NULL || ccall((:dpmm_destroy, lib), Cint, (Ptr{Cvoid},), x.ptr); x.ptr = C_NULL), c)
     return c
 end
