@@ -191,12 +191,12 @@ struct dpmm_ctx {
   // device-side parameter step (NIW): hyper-parameters, persistent statistics / posterior tables, factors
   bool dev_params = false;
   double alpha = 0.0;
-  double* hyper_d = nullptr;     // [NIW_HYPER_DOUBLES]
-  double* ptab = nullptr;        // [Kcap][3][stats_rec]
+  double* hyper_d = nullptr;     // [NIW_HYPER_DOUBLES(D_user)]
+  double* ptab = nullptr;        // [Kcap][3][stats_rec]   (records at D)
   double* ptab_alt = nullptr;
-  double* post = nullptr;        // [Kcap][3][NIW_POST_DOUBLES]
+  double* post = nullptr;        // [Kcap][3][NIW_POST_DOUBLES(D_user)]
   double* post_alt = nullptr;
-  double* lfac = nullptr;        // [3 Kcap][D][D]
+  double* lfac = nullptr;        // [3 Kcap][D][D]   (padded features: identity rows / columns)
   double* pm_out = nullptr;      // [Kcap*3*2 + Kcap*Kcap + 2] results of the posterior step for the host
   uint8_t* splittable_d = nullptr;
   int32_t* newof_d = nullptr;

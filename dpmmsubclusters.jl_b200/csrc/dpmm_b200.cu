@@ -51,9 +51,9 @@ static cudaError_t dev_grow_keep(T** p, size_t old_count, size_t new_count) {
   *p = q;
   return e;
 }
-// doubles per distribution of the posterior table
+// doubles per distribution of the posterior table (NIW: at the caller's D, also in a zero-padded context)
 static int post_doubles(const dpmm_ctx* c) {
-  return c->prior == DPMM_PRIOR_NIW ? NIW_POST_DOUBLES(c->D) : MNM_POST_DOUBLES(c->D);
+  return c->prior == DPMM_PRIOR_NIW ? NIW_POST_DOUBLES(c->D_user) : MNM_POST_DOUBLES(c->D);
 }
 static int ensure_tables(dpmm_ctx* ctx, int cap) {
   if (cap <= ctx->Kcap_tab) return 0;
@@ -1587,15 +1587,14 @@ extern "C" int dpmm_suff_stats(dpmm_ctx* ctx, const int64_t* indices, int32_t n_
 // ------------------------------------------------------------------------------------------------
 extern "C" int dpmm_num_clusters(const dpmm_ctx* ctx) { return ctx ? keff(ctx) : 0; }
 
+// The hyper-parameters, the posterior table and the draws are at the caller's D; only the statistics records and
+// what the sweep reads (lfac, the raw mu) keep the zero-padded context width ctx->D.
 extern "C" int dpmm_set_hyper_niw(dpmm_ctx* ctx, double kappa, const double* m, double nu, const double* psi, double alpha) {
   NEED(ctx && m && psi, DPMM_EINVAL, "NULL argument");
   NEED(ctx->prior == DPMM_PRIOR_NIW, DPMM_ESTATE, "context was created with the multinomial prior");
-  NEED(ctx->D == ctx->D_user, DPMM_ELIMIT,
-       "the device-side parameter step needs an instantiated feature dimension (1-8, 12, 16, 24, 32, 48, 64); "
-       "sample the parameters on the host (dpmm_set_params_niw) for other D");
-  NEED(kappa > 0 && nu > ctx->D - 1 && alpha > 0, DPMM_EINVAL, "need kappa > 0, nu > D - 1, alpha > 0");
+  NEED(kappa > 0 && nu > ctx->D_user - 1 && alpha > 0, DPMM_EINVAL, "need kappa > 0, nu > D - 1, alpha > 0");
   CK(cudaSetDevice(ctx->device));
-  const int D = ctx->D;
+  const int D = ctx->D_user;
   std::vector<double> h(NIW_HYPER_DOUBLES(D));
   // logdet psi by a host Cholesky of the symmetrised matrix (one-time, D <= 64)
   std::vector<double> A((size_t)D * D);
@@ -1657,7 +1656,7 @@ extern "C" int dpmm_set_hyper_multinomial(dpmm_ctx* ctx, const float* alpha_prio
 #define DPMM_NEED_HYPER(what) \
   NEED(ctx->dev_params, DPMM_ESTATE, "dpmm_set_hyper_niw or dpmm_set_hyper_multinomial must precede " what)
 
-static size_t niw_post_smem(int D) { return ((size_t)D * (D + 1) + 2 * D) * sizeof(double); }
+static size_t niw_post_smem(int D) { return ((size_t)D * (D + 1) + 2 * D) * sizeof(double); }   // D: the caller's
 
 // posterior + log marginal likelihood of the listed clusters (device list idx_d, or all m = K in order) from the table
 static int launch_post(dpmm_ctx* ctx, const int32_t* idx_d, int m, double* out) {
@@ -1671,9 +1670,9 @@ static int launch_post(dpmm_ctx* ctx, const int32_t* idx_d, int m, double* out) 
     return 0;
   }
   NiwPostArgs pa{};
-  pa.D = ctx->D; pa.rec = ctx->stats_rec; pa.hyper = ctx->hyper_d; pa.ptab = ctx->ptab; pa.idx_list = idx_d;
-  pa.post = ctx->post; pa.out = out;
-  const size_t sm = niw_post_smem(ctx->D);
+  pa.D = ctx->D_user; pa.ld = ctx->D; pa.rec = ctx->stats_rec; pa.hyper = ctx->hyper_d; pa.ptab = ctx->ptab;
+  pa.idx_list = idx_d; pa.post = ctx->post; pa.out = out;
+  const size_t sm = niw_post_smem(ctx->D_user);
   if (sm > 48 * 1024) CK(cudaFuncSetAttribute(niw_post_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
   KernelTimer kt(ctx, TK_PARAMS);
   niw_post_kernel<<<dim3((unsigned)m, 3), 256, sm, ctx->stream>>>(pa);
@@ -1740,9 +1739,9 @@ extern "C" int dpmm_posterior_step(dpmm_ctx* ctx, const int64_t* indices, int32_
       mnm_merge_kernel<<<grid, MNM_PARAM_THREADS, 0, ctx->side>>>(ma);
     } else {
       NiwMergeArgs ma{};
-      ma.D = ctx->D; ma.rec = rec; ma.K = k_merge; ma.hyper = ctx->hyper_d; ma.ptab = ctx->ptab;
+      ma.D = ctx->D_user; ma.ld = ctx->D; ma.rec = rec; ma.K = k_merge; ma.hyper = ctx->hyper_d; ma.ptab = ctx->ptab;
       ma.splittable = ctx->splittable_d; ma.out = merge_d;
-      const size_t sm = niw_post_smem(ctx->D);
+      const size_t sm = niw_post_smem(ctx->D_user);
       if (sm > 48 * 1024) CK(cudaFuncSetAttribute(niw_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
       int rcf = side_fork(ctx);
       if (rcf) return rcf;
@@ -1819,10 +1818,12 @@ extern "C" int dpmm_sample_params(dpmm_ctx* ctx, int32_t K, int32_t from_prior, 
     return side_join(ctx);
   }
   {
+    const int Du = ctx->D_user;
     NiwDrawArgs da{};
-    da.D = D; da.mu = ctx->raw_params; da.logdet = ctx->raw_params + nrec * D + nrec * D * D; da.hyper = ctx->hyper_d;
-    da.post = ctx->post; da.lfac = ctx->lfac; da.seed = ctx->seed; da.call = ctx->pcall; da.first = from_prior;
-    const size_t sm = ((size_t)3 * D * (D + 1) + 2 * D) * sizeof(double);
+    da.D = Du; da.ld = D; da.mu = ctx->raw_params; da.logdet = ctx->raw_params + nrec * D + nrec * D * D;
+    da.hyper = ctx->hyper_d; da.post = ctx->post; da.lfac = ctx->lfac; da.seed = ctx->seed; da.call = ctx->pcall;
+    da.first = from_prior;
+    const size_t sm = ((size_t)3 * Du * (Du + 1) + 2 * Du) * sizeof(double);
     if (sm > 48 * 1024) CK(cudaFuncSetAttribute(niw_draw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
     KernelTimer kt(ctx, TK_PARAMS);
     niw_draw_kernel<<<(unsigned)nrec, NIW_PACK_THREADS, sm, ctx->stream>>>(da);
@@ -1850,12 +1851,26 @@ extern "C" int dpmm_get_params_niw(dpmm_ctx* ctx, int32_t K, float* mu, double* 
   CK(cudaSetDevice(ctx->device));
   NEED(ctx->prior == DPMM_PRIOR_NIW, DPMM_ESTATE, "context was created with the multinomial prior");
   NEED(ctx->dev_params && ctx->params_set && K == ctx->K, DPMM_ESTATE, "no device-sampled parameters for this K");
-  const int D = ctx->D;
+  const int D = ctx->D, Du = ctx->D_user;
   const size_t nrec = (size_t)3 * K;
   CK(cudaStreamSynchronize(ctx->stream));
-  if (mu) CK(cudaMemcpy(mu, ctx->raw_params, nrec * D * 4, cudaMemcpyDeviceToHost));
+  if (Du == D) {
+    if (mu) CK(cudaMemcpy(mu, ctx->raw_params, nrec * D * 4, cudaMemcpyDeviceToHost));
+    if (lfac) CK(cudaMemcpy(lfac, ctx->lfac, nrec * D * D * 8, cudaMemcpyDeviceToHost));
+  } else {   // zero-padded context: the caller's [Du] / [Du][Du] blocks out of the [D] / [D][D] storage
+    if (mu) {
+      std::vector<float> h(nrec * D);
+      CK(cudaMemcpy(h.data(), ctx->raw_params, nrec * D * 4, cudaMemcpyDeviceToHost));
+      for (size_t t = 0; t < nrec; ++t) memcpy(mu + t * Du, &h[t * D], (size_t)Du * 4);
+    }
+    if (lfac) {
+      std::vector<double> h(nrec * D * D);
+      CK(cudaMemcpy(h.data(), ctx->lfac, nrec * D * D * 8, cudaMemcpyDeviceToHost));
+      for (size_t t = 0; t < nrec; ++t)
+        for (int i = 0; i < Du; ++i) memcpy(lfac + (t * Du + i) * Du, &h[(t * D + i) * D], (size_t)Du * 8);
+    }
+  }
   if (logdet) CK(cudaMemcpy(logdet, ctx->raw_params + nrec * D + nrec * D * D, nrec * 4, cudaMemcpyDeviceToHost));
-  if (lfac) CK(cudaMemcpy(lfac, ctx->lfac, nrec * D * D * 8, cudaMemcpyDeviceToHost));
   if (weights) CK(cudaMemcpy(weights, ctx->w_out, (size_t)K * 4, cudaMemcpyDeviceToHost));
   if (lr_weights) CK(cudaMemcpy(lr_weights, ctx->lr_out, (size_t)2 * K * 4, cudaMemcpyDeviceToHost));
   return 0;

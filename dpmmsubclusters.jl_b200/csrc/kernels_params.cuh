@@ -104,8 +104,9 @@ __device__ inline bool cta_cholesky(double* A, int D, int LD) {
 
 // Posterior of the statistics (N, sx, S) = sum over `nsrc` source records, written into shared memory:
 // A[D][LD] <- psi' (index-reversed when `reversed`), mp[D] <- m'.  Returns kappa', nu' through pointers.
-__device__ inline void niw_posterior_to_smem(const double* hyper, int D, int LD, const double* const* src, int nsrc,
-                                             bool reversed, double* A, double* mp, double* sxs, double& N,
+// D is the model's dimension; the records hold sx[ld] and S[ld][ld] (ld >= D: a zero-padded context's width).
+__device__ inline void niw_posterior_to_smem(const double* hyper, int D, int ld, int LD, const double* const* src,
+                                             int nsrc, bool reversed, double* A, double* mp, double* sxs, double& N,
                                              double& kp, double& nup) {
   const int tid = threadIdx.x, NT = blockDim.x;
   const double kappa = hyper[0], nu = hyper[1];
@@ -127,7 +128,7 @@ __device__ inline void niw_posterior_to_smem(const double* hyper, int D, int LD,
     double v;
     if (N > 0.0) {
       double S = 0.0;
-      for (int q = 0; q < nsrc; ++q) S += 0.5 * (src[q][1 + D + e] + src[q][1 + D + j * D + i]);
+      for (int q = 0; q < nsrc; ++q) S += 0.5 * (src[q][1 + ld + i * ld + j] + src[q][1 + ld + j * ld + i]);
       v = (nu * 0.5 * (psi[e] + psi[j * D + i]) + kappa * m0[i] * m0[j] - kp * mp[i] * mp[j] + S) / nup;
     } else {
       v = 0.5 * (psi[e] + psi[j * D + i]);
@@ -161,8 +162,10 @@ __device__ inline double niw_logml_cta(const double* hyper, int D, int LD, const
          (nup / 2.0) * (D * log(nup) + logdet) + (D / 2.0) * log(kappa / kp);
 }
 
+// D: the model's dimension (the caller's), at which the hyper-parameters and the posterior table are laid out;
+// ld: the context's (padded) dimension, the stride of the statistics records (rec = 1 + ld + ld^2).
 struct NiwPostArgs {
-  int D, rec;
+  int D, ld, rec;
   const double* hyper;
   const double* ptab;        // [K][3][rec]
   const int32_t* idx_list;   // [m] or nullptr (a = k)
@@ -180,7 +183,7 @@ __global__ void __launch_bounds__(256) niw_post_kernel(const NiwPostArgs a) {
   const int k = a.idx_list != nullptr ? a.idx_list[ai] : ai;
   const double* src[1] = {a.ptab + ((size_t)k * 3 + s) * a.rec};
   double N, kp, nup;
-  niw_posterior_to_smem(a.hyper, D, LD, src, 1, true, A, mp, sxs, N, kp, nup);
+  niw_posterior_to_smem(a.hyper, D, a.ld, LD, src, 1, true, A, mp, sxs, N, kp, nup);
   const bool ok = cta_cholesky(A, D, LD);
   double* P = a.post + ((size_t)k * 3 + s) * NIW_POST_DOUBLES(D);
   for (int e = threadIdx.x; e < D * D; e += blockDim.x) P[8 + D + e] = A[(e / D) * LD + (e % D)];
@@ -196,7 +199,7 @@ __global__ void __launch_bounds__(256) niw_post_kernel(const NiwPostArgs a) {
 }
 
 struct NiwMergeArgs {
-  int D, rec, K;
+  int D, ld, rec, K;         // D, ld, rec as in NiwPostArgs
   const double* hyper;
   const double* ptab;
   const uint8_t* splittable;   // [K]
@@ -223,20 +226,22 @@ __global__ void __launch_bounds__(256) niw_merge_kernel(const NiwMergeArgs a) {
   double* sxs = mp + D;
   const double* src[2] = {si, sj};
   double N, kp, nup;
-  niw_posterior_to_smem(a.hyper, D, LD, src, 2, false, A, mp, sxs, N, kp, nup);
+  niw_posterior_to_smem(a.hyper, D, a.ld, LD, src, 2, false, A, mp, sxs, N, kp, nup);
   const bool ok = cta_cholesky(A, D, LD);
   double logdet;
   const double lml = niw_logml_cta(a.hyper, D, LD, A, N, kp, nup, sxs, logdet);
   if (threadIdx.x == 0) *o = ok ? lml : __longlong_as_double(0x7ff8000000000000LL);
 }
 
+// The draw runs at the model's dimension D; mu and lfac are written at the context's dimension ld >= D, with the
+// padded features at mean 0 and unit precision (an identity block of L), as dpmm_set_params_niw pads host parameters.
 struct NiwDrawArgs {
-  int D;
-  float* mu;                 // [3K][D] out
-  float* logdet;             // [3K] out
+  int D, ld;
+  float* mu;                 // [3K][ld] out
+  float* logdet;             // [3K] out (log det of the D x D Sigma)
   const double* hyper;
-  const double* post;        // [K][3][NIW_POST_DOUBLES]
-  double* lfac;              // [3K][D][D] out: L (invSigma = L L'), row-major: input of niw_pack_kernel
+  const double* post;        // [K][3][NIW_POST_DOUBLES(D)]
+  double* lfac;              // [3K][ld][ld] out: L (invSigma = L L'), row-major: input of niw_pack_kernel
   uint64_t seed;
   uint32_t call;
   int first;                 // sample from the prior (init_first_clusters!: sample_clusters!(group, first) semantics)
@@ -245,7 +250,7 @@ struct NiwDrawArgs {
 // One CTA of NIW_PACK_THREADS per distribution t = 3k + s.
 __global__ void __launch_bounds__(NIW_PACK_THREADS) niw_draw_kernel(const NiwDrawArgs a) {
   extern __shared__ double Ls[];   // [D][LD] L | Wk [D][LD] | Bm [D][LD] | xi [D] | y [D]
-  const int D = a.D, LD = D + 1;
+  const int D = a.D, ld = a.ld, LD = D + 1;
   double* Wk = Ls + D * LD;
   double* Bm = Wk + D * LD;
   double* xi = Bm + D * LD;
@@ -331,11 +336,16 @@ __global__ void __launch_bounds__(NIW_PACK_THREADS) niw_draw_kernel(const NiwDra
   __shared__ int ok_s;
   if (tid == 0) ok_s = 1;
   __syncthreads();
-  for (int e = tid; e < D * D; e += NT) {
-    const int i = e / D, j = e - i * D;
-    const double v = j <= i ? Ls[i * LD + j] : 0.0;          // (entries above the diagonal are rounding residue)
-    if (!(fabs(v) < CUDART_INF) || (i == j && !(v > 0.0))) ok_s = 0;
-    a.lfac[(size_t)t * D * D + e] = v;
+  for (int e = tid; e < ld * ld; e += NT) {
+    const int i = e / ld, j = e - i * ld;
+    double v;
+    if (i < D && j < D) {
+      v = j <= i ? Ls[i * LD + j] : 0.0;                     // (entries above the diagonal are rounding residue)
+      if (!(fabs(v) < CUDART_INF) || (i == j && !(v > 0.0))) ok_s = 0;
+    } else {
+      v = i == j ? 1.0 : 0.0;                                // padded feature
+    }
+    a.lfac[(size_t)t * ld * ld + e] = v;
   }
   __syncthreads();
   // ---- the mean: L' y = xi, column-oriented back substitution by warp 0 (lane <-> unknowns k, k + 32);
@@ -362,8 +372,8 @@ __global__ void __launch_bounds__(NIW_PACK_THREADS) niw_draw_kernel(const NiwDra
     __syncwarp();
     const bool okk = ok_s != 0;
     const double rk = 1.0 / sqrt(kp);
-    if (lane < D) a.mu[(size_t)t * D + lane] = (float)(mpost[lane] + y0 * rk);
-    if (lane + 32 < D) a.mu[(size_t)t * D + lane + 32] = (float)(mpost[lane + 32] + y1 * rk);
+    if (lane < ld) a.mu[(size_t)t * ld + lane] = lane < D ? (float)(mpost[lane] + y0 * rk) : 0.f;
+    if (lane + 32 < ld) a.mu[(size_t)t * ld + lane + 32] = lane + 32 < D ? (float)(mpost[lane + 32] + y1 * rk) : 0.f;
     if (lane == 0) a.logdet[t] = okk ? (float)(-2.0 * lg) : __int_as_float(0x7fc00000);
   }
 }

@@ -151,9 +151,11 @@ int dpmm_num_clusters(const dpmm_ctx* ctx);
  *   sample_distribution                        src/priors/niw.jl:34-40; multinomial_prior.jl:23-25
  *   sample_cluster_params / sample_clusters!   src/shared_actions.jl:41-66, src/local_clusters_actions.jl:417-437
  *   should_merge! (the merged log marginal)    src/shared_actions.jl:21-38
- * The host keeps the Hastings accept / reject decisions on 3K scalars (+ the K x K merge table). */
+ * The host keeps the Hastings accept / reject decisions on 3K scalars (+ the K x K merge table).
+ * Every D below is the caller's d of dpmm_create, also where the NIW context runs zero-padded to a wider kernel. */
 
-/* niw_hyperparams (niw.jl:6-11: kappa, m[D], nu, psi[D][D]) and the concentration alpha (ds.jl:9). */
+/* niw_hyperparams (niw.jl:6-11: kappa, m[D], nu, psi[D][D]) and the concentration alpha (ds.jl:9).
+ * DPMM_EINVAL unless kappa > 0, nu > D - 1, alpha > 0 and psi is positive definite. */
 int dpmm_set_hyper_niw(dpmm_ctx* ctx, double kappa, const double* m, double nu, const double* psi, double alpha);
 /* multinomial_hyper (multinomial_prior.jl:6-8: alpha_prior float32 [D], every entry finite and > 0) and the
  * concentration alpha > 0 (ds.jl:9).  DPMM_ESTATE on an NIW context. */
@@ -177,7 +179,8 @@ int dpmm_sample_params(dpmm_ctx* ctx, int32_t k, int32_t from_prior, int32_t uni
  * cluster j <- empty (1-based).  Follow with dpmm_posterior_step(from_table = 1) for i. */
 int dpmm_params_merge(dpmm_ctx* ctx, int64_t i, int64_t j);
 /* The parameters of the last dpmm_sample_params: mu float32 [3K][D], lfac double [3K][D][D] (L lower,
- * invSigma = L L'), logdet float32 [3K] (log det Sigma), weights float32 [K], lr_weights float32 [K][2]. */
+ * invSigma = L L'), logdet float32 [3K] (log det Sigma), weights float32 [K], lr_weights float32 [K][2]; D is the
+ * caller's (the padded features of a zero-padded context are not returned). */
 int dpmm_get_params_niw(dpmm_ctx* ctx, int32_t k, float* mu, double* lfac, float* logdet, float* weights,
                         float* lr_weights);
 /* The parameters of the last dpmm_sample_params of a multinomial context: log_p float32 [3K][D]

@@ -154,6 +154,9 @@ remove_empty!(c::Ctx, pts_count::Vector{Int64}) = check(ccall((:dpmm_remove_empt
 
 """
     set_hyper!(c, h::niw_hyperparams, α)   (niw.jl:6-11, ds.jl:9)
+
+`m` and `ψ` at the data's D, also for a D without NIW kernels of its own (the context runs zero-padded, and the
+parameter step stays on the device).
 """
 function set_hyper!(c::Ctx, κ::Real, m::Vector{Float64}, ν::Real, ψ::Matrix{Float64}, α::Real)
     GC.@preserve m ψ check(ccall((:dpmm_set_hyper_niw, lib), Cint,
@@ -195,7 +198,7 @@ sample_params!(c::Ctx, K::Integer; from_prior::Bool = false, unit_weights::Bool 
 params_merge!(c::Ctx, i::Integer, j::Integer) =
     check(ccall((:dpmm_params_merge, lib), Cint, (Ptr{Cvoid}, Int64, Int64), c.ptr, i, j), c.ptr)
 
-"(mu[D,3,K], L[D,D,3,K] with invΣ = L*L' (stored row-major: read it transposed), logdetΣ[3,K], weights[K], lr[2,K])"
+"(mu[D,3,K], L[D,D,3,K] with invΣ = L*L' (stored row-major: read it transposed), logdetΣ[3,K], weights[K], lr[2,K]); D = the data's D"
 function get_params(c::Ctx, K::Integer)
     D = c.d
     mu = Array{Float32}(undef, D, 3, K); lf = Array{Float64}(undef, D, D, 3, K); ld = Array{Float32}(undef, 3, K)
