@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("DPMM_LIB_PATH") or os.path.join(_HERE, "libdpmm_b200.so")   # (override: development builds)
 
 OK, EINVAL, ECUDA, ESTATE, ELIMIT, ENCCL = 0, -1, -2, -3, -4, -5
-PRIOR_NIW, PRIOR_MULTINOMIAL = 0, 1
+PRIOR_NIW, PRIOR_MULTINOMIAL, PRIOR_DIAG_GAUSSIAN = 0, 1, 2
 SAMPLER_INVERSE_CDF, SAMPLER_GUMBEL = 0, 1
 
 _p = C.c_void_p
@@ -38,6 +38,7 @@ SIGNATURES = {
     "dpmm_set_sublabels": (C.c_int, [_p, _i64p]),
     "dpmm_set_params_niw": (C.c_int, [_p, _i32, _f32p, _f32p, _f32p, _f32p, _f32p]),
     "dpmm_set_params_multinomial": (C.c_int, [_p, _i32, _f32p, _f32p, _f32p]),
+    "dpmm_set_params_diag": (C.c_int, [_p, _i32, _f32p, _f32p, _f32p, _f32p, _f32p]),
     "dpmm_set_sampler": (C.c_int, [_p, _i32]),
     "dpmm_sample_labels": (C.c_int, [_p, _i32]),
     "dpmm_sample_sublabels": (C.c_int, [_p]),

@@ -51,7 +51,8 @@ _DEFAULTS = dict(                                   # src/global_params.jl
 
 def _jl_to_py(src):
     """The subset of Julia the reference's parameter files use (assignments of literals, `nothing`, `Inf`, `true`,
-    `zeros(Float32,d)`, `ones(Float32,d)`, `Matrix{Float32}(I, d, d)`, niw_hyperparams(...), multinomial_hyper(...))."""
+    `zeros(Float32,d)`, `ones(Float32,d)`, `Matrix{Float32}(I, d, d)`, niw_hyperparams(...), multinomial_hyper(...),
+    diag_niw_hyperparams(...))."""
     out = []
     for line in src.splitlines():
         line = re.sub(r"#.*$", "", line).rstrip()
@@ -73,7 +74,8 @@ def read_params(params_file):
     src = open(params_file, encoding="utf-8").read()
     if not params_file.endswith(".py"):
         src = _jl_to_py(src)
-    ns = {"np": np, "niw_hyperparams": P.niw_hyperparams, "multinomial_hyper": P.multinomial_hyper}
+    ns = {"np": np, "niw_hyperparams": P.niw_hyperparams, "multinomial_hyper": P.multinomial_hyper,
+          "diag_niw_hyperparams": P.diag_niw_hyperparams}
     exec(compile(src, params_file, "exec"), ns)        # a parameter file is code, in the reference as here
     g = dict(_DEFAULTS)
     g.update({k: v for k, v in ns.items() if k in _DEFAULTS or k == "alpha"})
@@ -84,7 +86,7 @@ def read_params(params_file):
 
 # ------------------------------------------------------------------------------------- checkpoints ---------
 def _hyper_arrays(h, tag, out):
-    if isinstance(h, P.niw_hyperparams):
+    if isinstance(h, (P.niw_hyperparams, P.diag_niw_hyperparams)):
         out[tag + "kappa"], out[tag + "m"], out[tag + "nu"], out[tag + "psi"] = np.float64(h.κ), h.m, np.float64(h.ν), h.ψ
     else:
         out[tag + "alpha"] = np.asarray(h.α, F32)
@@ -94,8 +96,9 @@ def _hyper_from(z, tag, kind, idx=None):
     def get(name):
         a = z[tag + name]
         return a if idx is None else a[idx]
-    if kind == "niw":
-        return P.niw_hyperparams(float(get("kappa")), np.array(get("m")), float(get("nu")), np.array(get("psi")))
+    if kind in ("niw", "diag"):
+        T = P.niw_hyperparams if kind == "niw" else P.diag_niw_hyperparams
+        return T(float(get("kappa")), np.array(get("m")), float(get("nu")), np.array(get("psi")))
     return P.multinomial_hyper(np.array(get("alpha")))
 
 
@@ -104,7 +107,8 @@ def save_model(model, path, filename, iter, total_time, global_params):
     sub-labels are gathered as create_pts_less_group does with Array(group.labels)).  Returns the file name."""
     g = model.group
     hyper = model.model_hyperparams.distribution_hyper_params
-    kind = "niw" if isinstance(hyper, P.niw_hyperparams) else "multinomial"
+    kind = ("niw" if isinstance(hyper, P.niw_hyperparams) else "diag" if isinstance(hyper, P.diag_niw_hyperparams)
+            else "multinomial")
     K = len(g.local_clusters)
     out = {"labels": np.asarray(g.sweep.get_labels(), np.int64),
            "labels_subcluster": np.asarray(g.sweep.get_sublabels(), np.int64),
@@ -125,6 +129,14 @@ def save_model(model, path, filename, iter, total_time, global_params):
         out["dist_logdet"] = stack(lambda cp: cp.distribution.logdetΣ, F32)
         D = hyper.m.shape[0]
         out["dist_invChol"] = stack(lambda cp: np.zeros((D, D)) if cp.distribution.invChol is None else cp.distribution.invChol)
+    elif kind == "diag":                                # the NIW items, with vectors where NIW has matrices
+        out["stats_sum"] = stack(lambda cp: cp.suff_statistics.points_sum)
+        out["stats_S"] = stack(lambda cp: cp.suff_statistics.S_diag)
+        for name, f in (("kappa", lambda h: h.κ), ("m", lambda h: h.m), ("nu", lambda h: h.ν), ("psi", lambda h: h.ψ)):
+            out["post_" + name] = stack(lambda cp, f=f: f(cp.posterior_hyperparams))
+        out["dist_mu"] = stack(lambda cp: cp.distribution.μ, F32)
+        out["dist_var"] = stack(lambda cp: cp.distribution.σ2, F32)
+        out["dist_logdet"] = stack(lambda cp: cp.distribution.logdetΣ, F32)
     else:
         out["stats_sum"] = stack(lambda cp: cp.suff_statistics.points_sum, F32)
         out["post_alpha"] = stack(lambda cp: cp.posterior_hyperparams.α, F32)
@@ -166,6 +178,11 @@ def load_checkpoint(filename):
                 post = _hyper_from(z, "post_", kind, (k, s))
                 dist = P.mv_gaussian(np.array(z["dist_mu"][k, s]), np.array(z["dist_Sigma"][k, s]), np.array(z["dist_invSigma"][k, s]),
                                      float(z["dist_logdet"][k, s]), np.array(z["dist_invChol"][k, s]))
+            elif kind == "diag":
+                ss = P.diag_niw_sufficient_statistics(float(z["stats_N"][k, s]), np.array(z["stats_sum"][k, s]),
+                                                      np.array(z["stats_S"][k, s]))
+                post = _hyper_from(z, "post_", kind, (k, s))
+                dist = P.diag_gaussian(np.array(z["dist_mu"][k, s]), np.array(z["dist_var"][k, s]), float(z["dist_logdet"][k, s]))
             else:
                 ss = P.multinomial_sufficient_statistics(float(z["stats_N"][k, s]), np.array(z["stats_sum"][k, s]))
                 post = _hyper_from(z, "post_", kind, (k, s))

@@ -16,6 +16,7 @@
 #include "kernels_gauss.cuh"
 #include "kernels_gauss_tc.cuh"
 #include "kernels_gauss_tc2.cuh"
+#include "kernels_diag.cuh"
 #include "kernels_ipc.cuh"
 #include "kernels_mnm.cuh"
 #include "kernels_mnm_sparse.cuh"
@@ -35,6 +36,7 @@ static int keff(const dpmm_ctx* c) { return std::max(std::max(c->K, c->label_bou
 
 static int nrec_floats(const dpmm_ctx* c) {
   if (c->prior == DPMM_PRIOR_MULTINOMIAL) return c->D;
+  if (c->prior == DPMM_PRIOR_DIAG_GAUSSIAN) return 2 * c->D;   // s | b (kernels_diag.cuh)
   const int D = c->D;
   return gauss_col_off(D) + ((D + 3) & ~3);
 }
@@ -84,7 +86,7 @@ static int ensure_k(dpmm_ctx* ctx, int K) {
   CK(cudaStreamSynchronize(ctx->stream));
   const int D = ctx->D;
   ctx->rec_f = nrec_floats(ctx);
-  ctx->stats_rec = (ctx->prior == DPMM_PRIOR_NIW) ? 1 + D + D * D : 1 + D;
+  ctx->stats_rec = ctx->prior == DPMM_PRIOR_NIW ? 1 + D + D * D : ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN ? 1 + 2 * D : 1 + D;
   // preserve nothing: all K-sized buffers are rewritten by the next set_params / sort
   CK(dev_realloc(&ctx->recs, (size_t)3 * cap * ctx->rec_f));
   if (ctx->prior == DPMM_PRIOR_NIW) CK(dev_realloc(&ctx->raw_params, (size_t)3 * cap * (D + D * D + 1)));
@@ -92,6 +94,7 @@ static int ensure_k(dpmm_ctx* ctx, int K) {
   CK(dev_realloc(&ctx->logw, (size_t)cap));
   CK(dev_realloc(&ctx->loglr, (size_t)2 * cap));
   if (ctx->prior == DPMM_PRIOR_MULTINOMIAL) CK(dev_realloc(&ctx->logp_t, (size_t)D * (cap + MNM_KT)));
+  if (ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN) CK(dev_realloc(&ctx->logp_t, (size_t)2 * D * (cap + DIAG_KT)));
   if (ctx->mtc_ok) {
     CK(dev_realloc(&ctx->mtc_w, (size_t)3 * ((D + 31) / 32) * MTC_N * 32));
     ctx->mtc_params = false;
@@ -221,7 +224,8 @@ extern "C" int dpmm_create(dpmm_ctx** out, const float* x, int64_t n_local, int3
   *out = nullptr;
   NEED(x != nullptr && n_local > 0 && d > 0, DPMM_EINVAL, "x must be non-NULL with n_local > 0 and d > 0");
   NEED(n_local < ((int64_t)1 << 31) - 4096, DPMM_ELIMIT, "n_local must fit in int32 (shard the points over more GPUs)");
-  NEED(prior_kind == DPMM_PRIOR_NIW || prior_kind == DPMM_PRIOR_MULTINOMIAL, DPMM_EINVAL, "unknown prior kind");
+  NEED(prior_kind == DPMM_PRIOR_NIW || prior_kind == DPMM_PRIOR_MULTINOMIAL || prior_kind == DPMM_PRIOR_DIAG_GAUSSIAN,
+       DPMM_EINVAL, "unknown prior kind");
   int dpad = d;
   if (prior_kind == DPMM_PRIOR_NIW) {
     // kernels are instantiated for D in {1-8, 12, 16, 24, 32, 48, 64}; any other D <= 64 runs zero-padded to the
@@ -229,8 +233,11 @@ extern "C" int dpmm_create(dpmm_ctx** out, const float* x, int64_t n_local, int3
     // D^2 constant keeps the caller's D)
     NEED(d <= 64, DPMM_ELIMIT, "NIW: D must be <= 64");
     while (!niw_dim_supported(dpad)) ++dpad;
-  } else
+  } else if (prior_kind == DPMM_PRIOR_DIAG_GAUSSIAN) {
+    NEED(d <= DPMM_MNM_MAX_D, DPMM_ELIMIT, "diagonal Gaussian: D must be <= 16384");
+  } else {
     NEED(d <= DPMM_MNM_MAX_D, DPMM_ELIMIT, "multinomial: D must be <= 16384");
+  }
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
     return fail(nullptr, DPMM_ECUDA, "no CUDA device: libdpmm_b200 has no CPU fallback");
@@ -352,7 +359,7 @@ extern "C" int dpmm_create(dpmm_ctx** out, const float* x, int64_t n_local, int3
   }
 #undef CKC
   // work-item length of the statistics kernels: NIW <= StatsCfg::MAX_CHUNK (a CTA per item);
-  // multinomial items are taken by single warps, so they are shorter
+  // multinomial and diagonal Gaussian items are taken by single warps, so they are shorter
   ctx->chunk = prior_kind == DPMM_PRIOR_NIW ? 1024 : 256;
   *out = ctx;
   return 0;
@@ -880,7 +887,7 @@ static int niw_pack_launch(dpmm_ctx* ctx, int K, const double* lfac) {
 extern "C" int dpmm_set_params_niw(dpmm_ctx* ctx, int32_t K, const float* mu, const float* inv_sigma,
                                    const float* logdet, const float* weights, const float* lr_weights) {
   NEED(ctx, DPMM_EINVAL, "ctx is NULL");
-  NEED(ctx->prior == DPMM_PRIOR_NIW, DPMM_ESTATE, "context was created with the multinomial prior");
+  NEED(ctx->prior == DPMM_PRIOR_NIW, DPMM_ESTATE, "not an NIW context");
   NEED(K >= 1 && K <= DPMM_MAX_K, DPMM_ELIMIT, "K out of range");
   NEED(mu && inv_sigma && logdet && weights && lr_weights, DPMM_EINVAL, "NULL parameter array");
   CK(cudaSetDevice(ctx->device));
@@ -947,7 +954,7 @@ static int mnm_pack_launch(dpmm_ctx* ctx, int K) {
 extern "C" int dpmm_set_params_multinomial(dpmm_ctx* ctx, int32_t K, const float* log_p, const float* weights,
                                            const float* lr_weights) {
   NEED(ctx, DPMM_EINVAL, "ctx is NULL");
-  NEED(ctx->prior == DPMM_PRIOR_MULTINOMIAL, DPMM_ESTATE, "context was created with the NIW prior");
+  NEED(ctx->prior == DPMM_PRIOR_MULTINOMIAL, DPMM_ESTATE, "not a multinomial context");
   NEED(K >= 1 && K <= DPMM_MAX_K, DPMM_ELIMIT, "K out of range");
   NEED(log_p && weights && lr_weights, DPMM_EINVAL, "NULL parameter array");
   CK(cudaSetDevice(ctx->device));
@@ -972,10 +979,116 @@ extern "C" int dpmm_set_params_multinomial(dpmm_ctx* ctx, int32_t K, const float
   return mnm_pack_launch(ctx, K);
 }
 
+// The label kernels' transposed s / b tables from the [2][3K][D] records in ctx->recs (mnm_pack_kernel transposes
+// the cluster rows of one [3K][D] block); logw / loglr / cst are already in place.
+static int diag_pack_launch(dpmm_ctx* ctx, int K) {
+  const int D = ctx->D;
+  const int KP = (K + DIAG_KT - 1) / DIAG_KT * DIAG_KT;
+  const int64_t ne = (int64_t)D * KP;
+  for (int h = 0; h < 2; ++h) {
+    MnmPackArgs pa{};
+    pa.D = D; pa.K = K; pa.KP = KP; pa.logp = ctx->recs + (size_t)h * 3 * K * D; pa.logp_t = ctx->logp_t + (size_t)h * D * KP;
+    pa.mtc_w = nullptr;
+    KernelTimer kt(ctx, TK_PARAMS);
+    mnm_pack_kernel<<<(unsigned)std::min<int64_t>((ne + 255) / 256, (int64_t)ctx->sm_count * 4), 256, 0, ctx->stream>>>(pa);
+    CK(cudaGetLastError());
+  }
+  ctx->K = K;
+  ctx->KP = KP;
+  ctx->params_set = true;
+  return 0;
+}
+
+extern "C" int dpmm_set_params_diag(dpmm_ctx* ctx, int32_t K, const float* mu, const float* var, const float* logdet,
+                                    const float* weights, const float* lr_weights) {
+  NEED(ctx, DPMM_EINVAL, "ctx is NULL");
+  NEED(ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN, DPMM_ESTATE, "not a diagonal Gaussian context");
+  NEED(K >= 1 && K <= DPMM_MAX_K, DPMM_ELIMIT, "K out of range");
+  NEED(mu && var && logdet && weights && lr_weights, DPMM_EINVAL, "NULL parameter array");
+  CK(cudaSetDevice(ctx->device));
+  int rc = ensure_k(ctx, K);
+  if (rc) return rc;
+  const int D = ctx->D;
+  const size_t nrec = (size_t)3 * K;
+  const size_t bytes = (2 * nrec * D + nrec + K + 2 * K) * sizeof(float);
+  void* hs = nullptr;
+  const int slot = upload_acquire(ctx, bytes, &hs);
+  if (slot < 0) return slot;
+  float* h_s = (float*)hs;
+  float* h_b = h_s + nrec * D;
+  float* h_cst = h_b + nrec * D;
+  float* h_logw = h_cst + nrec;
+  float* h_loglr = h_logw + K;
+  // s = 1/sigma and b = -s mu, each rounded once from Float64 (the oracle restates exactly this)
+  const double log2pi = 1.8378770664093453;
+  for (size_t t = 0; t < nrec; ++t) {
+    for (int d = 0; d < D; ++d) {
+      const size_t e = t * D + d;
+      const float sv = (float)(1.0 / std::sqrt((double)var[e]));
+      h_s[e] = sv;
+      h_b[e] = (float)(-(double)sv * (double)mu[e]);
+    }
+    h_cst[t] = (float)(-0.5 * ((double)D * log2pi + (double)logdet[t]));
+  }
+  common_weights(ctx, K, weights, lr_weights, h_logw, h_loglr);
+  CK(cudaMemcpyAsync(ctx->recs, h_s, 2 * nrec * D * 4, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(ctx->cst, h_cst, nrec * 4, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(ctx->logw, h_logw, (size_t)K * 4, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(ctx->loglr, h_loglr, (size_t)2 * K * 4, cudaMemcpyHostToDevice, ctx->stream));
+  rc = upload_release(ctx, slot);
+  if (rc) return rc;
+  return diag_pack_launch(ctx, K);
+}
+
 // ------------------------------------------------------------------------------------------------
 // the sweep
 // ------------------------------------------------------------------------------------------------
 static int ensure_sorted(dpmm_ctx* ctx);
+
+template <int TP>
+static int launch_diag_label_stream(dpmm_ctx* ctx, DiagLabelArgs& a) {
+  const size_t sm = DiagStreamCfg<TP>::smem_bytes(a.K);
+  NEED(sm <= (size_t)ctx->smem_optin, DPMM_ELIMIT, "internal: diagonal streaming label kernel does not fit shared memory");
+  a.ntiles = (a.n + TP - 1) / TP;
+  CK(cudaFuncSetAttribute(diag_label_stream_kernel<TP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+  int occ = 1;
+  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, diag_label_stream_kernel<TP>, 256, sm));
+  occ = std::max(occ, 1);
+  const int64_t grid = std::min<int64_t>(a.ntiles, (int64_t)ctx->sm_count * occ);
+  KernelTimer kt(ctx, TK_LABEL);
+  diag_label_stream_kernel<TP><<<(unsigned)grid, 256, sm, ctx->stream>>>(a);
+  CK(cudaGetLastError());
+  return 0;
+}
+
+// Label draw of a diagonal Gaussian context: the thread-per-point kernel while the s / b tables fit shared memory
+// beside a 128-point tile (it pads K to 16 clusters only, where the streaming kernel works on chunks of 128 to 512),
+// else the streaming kernel with the largest point tile whose parr slice fits.
+static int launch_diag_label(dpmm_ctx* ctx, int final_iter, float* dump) {
+  const int K = ctx->K;
+  DiagLabelArgs a{};
+  a.x = ctx->x; a.n = ctx->n; a.D = ctx->D; a.DS = ctx->D | 1; a.K = K; a.KP = ctx->KP; a.s_t = ctx->logp_t;
+  a.b_t = ctx->logp_t + (size_t)ctx->D * ctx->KP; a.cst = ctx->cst; a.logw = ctx->logw; a.labels = ctx->labels;
+  a.hist = ctx->hist; a.u_inj = ctx->u_label; a.seed = ctx->seed; a.call = ctx->call; a.goff = ctx->goff;
+  a.final_iter = final_iter; a.sampler = ctx->sampler; a.dump = dump;
+  const int T = 128;
+  const size_t sm = ((size_t)2 * a.D * a.KP + (size_t)T * a.DS + (size_t)K * T) * 4 + (size_t)K * 4;
+  if (sm <= (size_t)ctx->smem_optin) {
+    a.ntiles = (a.n + T - 1) / T;
+    CK(cudaFuncSetAttribute(diag_label_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+    int occ = 1;
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, diag_label_kernel, T, sm));
+    occ = std::max(occ, 1);
+    const int64_t grid = std::min<int64_t>(a.ntiles, (int64_t)ctx->sm_count * occ);
+    KernelTimer kt(ctx, TK_LABEL);
+    diag_label_kernel<<<(unsigned)grid, T, sm, ctx->stream>>>(a);
+    CK(cudaGetLastError());
+    return 0;
+  }
+  return DiagStreamCfg<128>::smem_bytes(K) <= (size_t)ctx->smem_optin ? launch_diag_label_stream<128>(ctx, a)
+       : DiagStreamCfg<64>::smem_bytes(K) <= (size_t)ctx->smem_optin  ? launch_diag_label_stream<64>(ctx, a)
+                                                                       : launch_diag_label_stream<32>(ctx, a);
+}
 
 // The sweep's kernels are chained with programmatic dependent launch (common.cuh).  The label and fused kernels allocate
 // tensor memory before their grid dependency, i.e. possibly while CTAs of the previous kernel still run.  That is safe
@@ -1179,6 +1292,9 @@ static int run_sample_labels(dpmm_ctx* ctx, int final_iter, float* dump) {
     a.goff = ctx->goff; a.final_iter = final_iter; a.sampler = ctx->sampler; a.dump = dump;
     int rc = niw_launch_label(ctx, a);
     if (rc) return rc;
+  } else if (ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN) {
+    int rc = launch_diag_label(ctx, final_iter, dump);
+    if (rc) return rc;
   } else if (ctx->sparse) {
     int rc = launch_mnm_sparse_label(ctx, final_iter, dump);
     if (rc) return rc;
@@ -1339,6 +1455,13 @@ static int run_sublabels(dpmm_ctx* ctx, bool sample, float* dump) {
   if (ctx->prior == DPMM_PRIOR_NIW) {
     rc = niw_launch_sublabel(ctx, a, sample);
     if (rc) return rc;
+  } else if (ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN) {
+    KernelTimer kt(ctx, TK_SUBLABEL);
+    if (sample)
+      diag_sublabel_kernel<<<(unsigned)((a.n + DIAG_SLS_T - 1) / DIAG_SLS_T), DIAG_SLS_T, 0, ctx->stream>>>(a);
+    else
+      mnm_sublabel_kernel<false><<<(unsigned)((a.n + 127) / 128), 128, 0, ctx->stream>>>(a);
+    CK(cudaGetLastError());
   } else {
     const int T = 128;
     const unsigned grid = (unsigned)((a.n + T - 1) / T);
@@ -1482,6 +1605,13 @@ static int stats_compute(dpmm_ctx* ctx, const int64_t* indices, int32_t n_indice
   } else if (ctx->prior == DPMM_PRIOR_NIW) {
     rc = niw_launch_stats(ctx, sa);
     if (rc) return rc;
+  } else if (ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN) {
+    int occ = 1;
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, diag_stats_kernel, 256, 0));
+    occ = std::max(occ, 1);
+    KernelTimer kt(ctx, TK_STATS);
+    diag_stats_kernel<<<ctx->sm_count * occ, 256, 0, ctx->stream>>>(sa);
+    CK(cudaGetLastError());
   } else if (ctx->sparse) {
     const size_t smem = (size_t)D * 4;
     if (smem > 48 * 1024) CK(cudaFuncSetAttribute(mnm_sparse_stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1574,6 +1704,7 @@ extern "C" int dpmm_suff_stats(dpmm_ctx* ctx, const int64_t* indices, int32_t n_
       if (counts) counts[a * 3 + s] = (int64_t)llround(r[0]);
       const int Du = ctx->D_user;
       if (sum_x) memcpy(sum_x + ((size_t)a * 3 + s) * Du, r + 1, (size_t)Du * 8);
+      if (sum_xx && ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN) memcpy(sum_xx + ((size_t)a * 3 + s) * Du, r + 1 + D, (size_t)Du * 8);
       if (sum_xx && ctx->prior == DPMM_PRIOR_NIW)
         for (int i = 0; i < Du; ++i)
           memcpy(sum_xx + (((size_t)a * 3 + s) * Du + i) * Du, r + 1 + D + (size_t)i * D, (size_t)Du * 8);
@@ -1591,7 +1722,7 @@ extern "C" int dpmm_num_clusters(const dpmm_ctx* ctx) { return ctx ? keff(ctx) :
 // what the sweep reads (lfac, the raw mu) keep the zero-padded context width ctx->D.
 extern "C" int dpmm_set_hyper_niw(dpmm_ctx* ctx, double kappa, const double* m, double nu, const double* psi, double alpha) {
   NEED(ctx && m && psi, DPMM_EINVAL, "NULL argument");
-  NEED(ctx->prior == DPMM_PRIOR_NIW, DPMM_ESTATE, "context was created with the multinomial prior");
+  NEED(ctx->prior == DPMM_PRIOR_NIW, DPMM_ESTATE, "not an NIW context");
   NEED(kappa > 0 && nu > ctx->D_user - 1 && alpha > 0, DPMM_EINVAL, "need kappa > 0, nu > D - 1, alpha > 0");
   CK(cudaSetDevice(ctx->device));
   const int D = ctx->D_user;
@@ -1631,7 +1762,7 @@ extern "C" int dpmm_set_hyper_niw(dpmm_ctx* ctx, double kappa, const double* m, 
 
 extern "C" int dpmm_set_hyper_multinomial(dpmm_ctx* ctx, const float* alpha_prior, double alpha) {
   NEED(ctx, DPMM_EINVAL, "ctx is NULL");
-  NEED(ctx->prior == DPMM_PRIOR_MULTINOMIAL, DPMM_ESTATE, "context was created with the NIW prior");
+  NEED(ctx->prior == DPMM_PRIOR_MULTINOMIAL, DPMM_ESTATE, "not a multinomial context");
   NEED(alpha_prior, DPMM_EINVAL, "alpha_prior is NULL");
   NEED(alpha > 0, DPMM_EINVAL, "need alpha > 0");
   CK(cudaSetDevice(ctx->device));
@@ -1654,7 +1785,8 @@ extern "C" int dpmm_set_hyper_multinomial(dpmm_ctx* ctx, const float* alpha_prio
 }
 
 #define DPMM_NEED_HYPER(what) \
-  NEED(ctx->dev_params, DPMM_ESTATE, "dpmm_set_hyper_niw or dpmm_set_hyper_multinomial must precede " what)
+  NEED(ctx->dev_params, DPMM_ESTATE, "dpmm_set_hyper_niw or dpmm_set_hyper_multinomial must precede " what \
+       " (a diagonal Gaussian context has no device parameter step)")
 
 static size_t niw_post_smem(int D) { return ((size_t)D * (D + 1) + 2 * D) * sizeof(double); }   // D: the caller's
 
@@ -1849,7 +1981,7 @@ extern "C" int dpmm_get_params_niw(dpmm_ctx* ctx, int32_t K, float* mu, double* 
                                    float* lr_weights) {
   NEED(ctx, DPMM_EINVAL, "ctx is NULL");
   CK(cudaSetDevice(ctx->device));
-  NEED(ctx->prior == DPMM_PRIOR_NIW, DPMM_ESTATE, "context was created with the multinomial prior");
+  NEED(ctx->prior == DPMM_PRIOR_NIW, DPMM_ESTATE, "not an NIW context");
   NEED(ctx->dev_params && ctx->params_set && K == ctx->K, DPMM_ESTATE, "no device-sampled parameters for this K");
   const int D = ctx->D, Du = ctx->D_user;
   const size_t nrec = (size_t)3 * K;
@@ -1879,7 +2011,7 @@ extern "C" int dpmm_get_params_niw(dpmm_ctx* ctx, int32_t K, float* mu, double* 
 extern "C" int dpmm_get_params_multinomial(dpmm_ctx* ctx, int32_t K, float* log_p, float* weights, float* lr_weights) {
   NEED(ctx, DPMM_EINVAL, "ctx is NULL");
   CK(cudaSetDevice(ctx->device));
-  NEED(ctx->prior == DPMM_PRIOR_MULTINOMIAL, DPMM_ESTATE, "context was created with the NIW prior");
+  NEED(ctx->prior == DPMM_PRIOR_MULTINOMIAL, DPMM_ESTATE, "not a multinomial context");
   NEED(ctx->dev_params && ctx->params_set && K == ctx->K, DPMM_ESTATE, "no device-sampled parameters for this K");
   CK(cudaStreamSynchronize(ctx->stream));
   if (log_p) CK(cudaMemcpy(log_p, ctx->recs, (size_t)3 * K * ctx->D * 4, cudaMemcpyDeviceToHost));
@@ -1891,7 +2023,7 @@ extern "C" int dpmm_get_params_multinomial(dpmm_ctx* ctx, int32_t K, float* log_
 extern "C" int dpmm_predict_niw(dpmm_ctx* ctx, int32_t K, const float* u, const float* mu, const float* tconst,
                                 const float* df, int64_t* labels, float* probs) {
   NEED(ctx && u && mu && tconst && df && labels, DPMM_EINVAL, "NULL argument");
-  NEED(ctx->prior == DPMM_PRIOR_NIW, DPMM_ESTATE, "context was created with the multinomial prior");
+  NEED(ctx->prior == DPMM_PRIOR_NIW, DPMM_ESTATE, "not an NIW context");
   NEED(K >= 1 && K <= DPMM_MAX_K, DPMM_ELIMIT, "K out of range");
   CK(cudaSetDevice(ctx->device));
   const int D = ctx->D;
@@ -1961,7 +2093,7 @@ extern "C" int dpmm_predict_niw(dpmm_ctx* ctx, int32_t K, const float* u, const 
 extern "C" int dpmm_predict_multinomial(dpmm_ctx* ctx, int32_t K, const double* logp, const float* logw,
                                         int64_t* labels, float* probs) {
   NEED(ctx && logp && logw && labels, DPMM_EINVAL, "NULL argument");
-  NEED(ctx->prior == DPMM_PRIOR_MULTINOMIAL, DPMM_ESTATE, "context was created with the NIW prior");
+  NEED(ctx->prior == DPMM_PRIOR_MULTINOMIAL, DPMM_ESTATE, "not a multinomial context");
   NEED(K >= 1 && K <= DPMM_MAX_K, DPMM_ELIMIT, "K out of range");
   CK(cudaSetDevice(ctx->device));
   const int D = ctx->D;

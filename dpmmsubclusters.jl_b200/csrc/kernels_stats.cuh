@@ -126,7 +126,7 @@ struct StatsArgs {
   const StatsItem* items;
   const int32_t* n_items;
   int32_t* next_item;
-  double* acc;              // [2K][rec]  rec = 1 + D + D*D (NIW) or 1 + D (multinomial); count slot unused here
+  double* acc;              // [2K][rec]  rec = 1 + D + D*D (NIW), 1 + 2D (diagonal) or 1 + D (multinomial); count slot unused
   int rec;
 };
 
@@ -436,7 +436,8 @@ __global__ void __launch_bounds__(256) mnm_stats_kernel(const StatsArgs a) {
 }
 
 // K8: finalise + pack.  out[m][3][rec] for the m requested clusters: cluster = left + right, S
-// mirrored from its upper triangle, counts from the partition cursors.  When `xc` is given the
+// mirrored from its upper triangle (niw != 0), counts from the partition cursors.  With niw == 0 every other entry is
+// a plain sum and is added as it is: [N | sum x] (multinomial), [N | sum x | sum x^2] (diagonal Gaussian).  When `xc` is given the
 // accumulators hold sums of y = x - c about a centre c of every run (centers [2K][D], see
 // kernels_stats_tc.cuh) and are shifted back here in Float64: sum x = s + N c,  S = sum y y' + c s' + s c' + N c c'.
 // `risk` (optional) counts the diagonal entries whose centred sum exceeds 32 x the un-centred one: the

@@ -107,6 +107,7 @@ extern "C" int dpmm_smart_project(dpmm_ctx* ctx, int64_t cluster, const double* 
   NEED(v && mu && lo_hi && count, DPMM_EINVAL, "NULL argument");
   NEED(cluster >= 1 && cluster <= DPMM_MAX_K, DPMM_EINVAL, "cluster index out of range");
   NEED(ctx->x != nullptr, DPMM_ESTATE, "smart splits project the dense points: a sparse context has none");
+  NEED(ctx->prior != DPMM_PRIOR_DIAG_GAUSSIAN, DPMM_ESTATE, "smart splits need the full scatter matrix: not on a diagonal context");
   CK(cudaSetDevice(ctx->device));
   if (!ctx->smart) ctx->smart = new SmartState();
   SmartState* s = ctx->smart;

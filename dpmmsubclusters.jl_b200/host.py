@@ -20,7 +20,7 @@ import scipy.sparse as sps
 from scipy.special import gammaln
 
 from . import priors as P
-from .sweep import GpuSweep, NIW, MULTINOMIAL
+from .sweep import GpuSweep, NIW, MULTINOMIAL, DIAG
 
 F32 = np.float32
 
@@ -225,6 +225,11 @@ def broadcast_cluster_params(group):
         inv = np.array([[d.invΣ for d in t] for t in trip], F32)
         ld = np.array([[d.logdetΣ for d in t] for t in trip], F32)
         group.sweep.set_params_niw(mu, inv, ld, w, lr)
+    elif isinstance(group.model_hyperparams.distribution_hyper_params, P.diag_niw_hyperparams):
+        mu = np.array([[d.μ for d in t] for t in trip], F32)
+        var = np.array([[d.σ2 for d in t] for t in trip], F32)
+        ld = np.array([[d.logdetΣ for d in t] for t in trip], F32)
+        group.sweep.set_params_diag(mu, var, ld, w, lr)
     else:
         lp = np.array([[d.α for d in t] for t in trip], F32)
         group.sweep.set_params_multinomial(lp, w, lr)
@@ -415,7 +420,8 @@ def init_model_from_data(all_data, hyper_params, α, cfg, seed, sweep_factory, s
     """init_model_from_data :36-53: `distribute(all_data)` + random labels become dpmm_create +
     dpmm_init_labels.  `shard` = (global_offset, n_total) when the points are one shard of many."""
     all_data = _points(all_data)
-    kind = NIW if isinstance(hyper_params, P.niw_hyperparams) else MULTINOMIAL
+    kind = (NIW if isinstance(hyper_params, P.niw_hyperparams)
+            else DIAG if isinstance(hyper_params, P.diag_niw_hyperparams) else MULTINOMIAL)
     goff, n_total = shard if shard is not None else (0, all_data.shape[1])
     sweep_seed = int(seed) if seed is not None else int(np.random.default_rng().integers(2 ** 62))
     sweep = sweep_factory(all_data, kind, sweep_seed, goff)
@@ -542,8 +548,10 @@ def dp_parallel(all_data, local_hyper_params=None, α_param=None, iters=100, ini
         raise NotImplementedError("the outlier component is out of scope (DESIGN.md 6)")
     if save_model and save_path is None:
         raise ValueError("save_model=True needs save_path (global_params.jl:37 in the reference)")
-    if sps.issparse(all_data) and isinstance(local_hyper_params, P.niw_hyperparams):
+    if sps.issparse(all_data) and isinstance(local_hyper_params, (P.niw_hyperparams, P.diag_niw_hyperparams)):
         raise ValueError("sparse points are supported for the multinomial prior only")
+    if smart_splits and isinstance(local_hyper_params, P.diag_niw_hyperparams):
+        raise ValueError("smart splits need the full scatter matrix: not available with the diagonal prior")
     if smart_splits and not isinstance(local_hyper_params, P.niw_hyperparams):
         raise ValueError("smart splits are Gaussian only (dp-parallel-sampling.jl:111)")
     if (comm is not None or shard is not None) and seed is None:
@@ -561,6 +569,11 @@ def _run_from_settings(all_data, local_hyper_params, α_param, cfg, seed, sweep_
                        restored=None):
     """init_model + init_first_clusters! + run_model for fresh runs; create_model_from_saved_data + run_model(iter + 1)
     when `restored` = (pts_less_group dict, iter) of a checkpoint."""
+    if isinstance(local_hyper_params, P.diag_niw_hyperparams):
+        if device_params:
+            raise ValueError("device_params: the device parameter step runs the NIW and multinomial priors only")
+        if cfg.use_smart_splits:
+            raise ValueError("smart splits need the full scatter matrix: not available with the diagonal prior")
     if restored is not None and seed is not None:
         seed = int(seed) + 1000003 * int(restored[1])     # a resumed run must not replay the random streams of iteration 1
     rng = np.random.default_rng(seed)
@@ -668,10 +681,15 @@ def predict(dp_model, data, device=0, on_device=None):
     NIW models run on the GPU by default (dpmm_predict_niw: Student-t densities, argmax and softmax per point; the
     host prepares the K factors); multinomial models do with on_device=True (dpmm_predict_multinomial: the host
     prepares log(alpha'/sum alpha') in Float64).  on_device=False, or a multinomial model by default, takes the NumPy
-    formulas below.  Sparse data (scipy.sparse, D x N) runs on a sparse context on the device and as x' logp in NumPy."""
+    formulas below.  Sparse data (scipy.sparse, D x N) runs on a sparse context on the device and as x' logp in NumPy.
+    Diagonal Gaussian models always take the NumPy formula (a product of per-feature Student-t densities)."""
     data = _points(data)
     cl = dp_model.group.local_clusters
     posts = [c.cluster_params.cluster_params.posterior_hyperparams for c in cl]
+    if posts and isinstance(posts[0], P.diag_niw_hyperparams):
+        if on_device:
+            raise ValueError("predict on the device runs the NIW and multinomial priors only")
+        on_device = False
     w = np.asarray(dp_model.group.weights, F32)
     mnm = bool(posts) and isinstance(posts[0], P.multinomial_hyper)
     if on_device is None:

@@ -16,6 +16,7 @@ from . import _lib as L
 
 NIW = L.PRIOR_NIW
 MULTINOMIAL = L.PRIOR_MULTINOMIAL
+DIAG = L.PRIOR_DIAG_GAUSSIAN
 
 
 def _ptr(a, ctype):
@@ -157,6 +158,22 @@ class GpuSweep:
         self._ck(self.lib.dpmm_set_params_multinomial(self.h, K, _ptr(log_p, f), _ptr(weights, f), _ptr(lr_weights, f)))
         self.K = K
 
+    def set_params_diag(self, mu, var, logdet, weights, lr_weights):
+        """mu [K,3,D], var [K,3,D] (per-feature sigma^2), logdet [K,3] = sum log sigma^2, weights [K], lr_weights [K,2]
+        (Float32)."""
+        mu = np.ascontiguousarray(mu, np.float32)
+        K = mu.shape[0]
+        var = np.ascontiguousarray(var, np.float32)
+        logdet = np.ascontiguousarray(logdet, np.float32)
+        weights = np.ascontiguousarray(weights, np.float32)
+        lr_weights = np.ascontiguousarray(lr_weights, np.float32)
+        assert mu.shape == (K, 3, self.D) and var.shape == (K, 3, self.D)
+        assert logdet.shape == (K, 3) and weights.shape == (K,) and lr_weights.size == 2 * K
+        f = C.c_float
+        self._ck(self.lib.dpmm_set_params_diag(self.h, K, _ptr(mu, f), _ptr(var, f), _ptr(logdet, f), _ptr(weights, f),
+                                               _ptr(lr_weights, f)))
+        self.K = K
+
     # ---- sweep ----
     def sample_labels(self, final=False):
         self._ck(self.lib.dpmm_sample_labels(self.h, 1 if final else 0))
@@ -165,7 +182,8 @@ class GpuSweep:
         self._ck(self.lib.dpmm_sample_sublabels(self.h))
 
     def suff_stats(self, indices=None, fetch=True, out=None):
-        """Returns (counts [m,3] i64, sum_x [m,3,D] f64, sum_xx [m,3,D,D] f64 or None).
+        """Returns (counts [m,3] i64, sum_x [m,3,D] f64, sum_xx: [m,3,D,D] f64 (NIW), [m,3,D] f64 (diagonal: sum of
+        x_d^2) or None (multinomial)).
         `out`: an earlier result of the same shape to be overwritten (saves the allocation and the
         first-touch page faults of ~0.5 MB per call in a tight loop)."""
         if indices is None:
@@ -176,19 +194,20 @@ class GpuSweep:
         if not fetch:
             self._ck(self.lib.dpmm_suff_stats(self.h, idx_p, m, None, None, None))
             return None
+        xx_shape = {NIW: (m, 3, self.D, self.D), DIAG: (m, 3, self.D)}.get(self.prior_kind)
         if out is not None:
             counts, sum_x, sum_xx = out
             ok = (counts.shape == (m, 3) and counts.dtype == np.int64 and counts.flags.c_contiguous
                   and sum_x.shape == (m, 3, self.D) and sum_x.dtype == np.float64 and sum_x.flags.c_contiguous
-                  and (sum_xx is None) == (self.prior_kind != NIW)
-                  and (sum_xx is None or (sum_xx.shape == (m, 3, self.D, self.D) and sum_xx.dtype == np.float64
+                  and (sum_xx is None) == (xx_shape is None)
+                  and (sum_xx is None or (sum_xx.shape == xx_shape and sum_xx.dtype == np.float64
                                           and sum_xx.flags.c_contiguous)))
             if not ok:
                 raise ValueError("suff_stats(out=...): arrays of the wrong shape / dtype / layout")
         else:
             counts = np.zeros((m, 3), np.int64)
             sum_x = np.zeros((m, 3, self.D), np.float64)
-            sum_xx = np.zeros((m, 3, self.D, self.D), np.float64) if self.prior_kind == NIW else None
+            sum_xx = None if xx_shape is None else np.zeros(xx_shape, np.float64)
         self._ck(self.lib.dpmm_suff_stats(self.h, idx_p, m, _ptr(counts, C.c_int64), _ptr(sum_x, C.c_double),
                                           _ptr(sum_xx, C.c_double)))
         return counts, sum_x, sum_xx

@@ -40,6 +40,7 @@ extern "C" {
 
 #define DPMM_PRIOR_NIW 0          /* niw_hyperparams   -> mv_gaussian       (src/priors/niw.jl)               */
 #define DPMM_PRIOR_MULTINOMIAL 1  /* multinomial_hyper -> multinomial_dist  (src/priors/multinomial_prior.jl) */
+#define DPMM_PRIOR_DIAG_GAUSSIAN 2 /* diag_niw_hyperparams -> diag_gaussian: an independent D = 1 NIW per feature   */
 
 #define DPMM_SAMPLER_INVERSE_CDF 0 /* reference semantics: StatsBase.sample(ProbabilityWeights), utils.jl:29 */
 #define DPMM_SAMPLER_GUMBEL 1      /* Gumbel-max: same distribution, different stream, no per-point K storage */
@@ -53,8 +54,10 @@ typedef struct dpmm_ctx dpmm_ctx;
  * (0-based) of this shard's first point in the whole data set: the counter-based RNG is keyed by the
  * global point index so results do not depend on how many GPUs the points are spread over.
  * device: CUDA ordinal.  seed: replaces `@everywhere Random.seed!(seed)` (:37-39).
- * d: 1..64 for the NIW prior, 1..16384 for the multinomial prior; larger d returns
- * DPMM_ELIMIT.  Every multinomial d samples with any K up to DPMM_MAX_K. */
+ * d: 1..64 for the NIW prior, 1..16384 for the multinomial and the diagonal Gaussian prior; larger d returns
+ * DPMM_ELIMIT.  Every multinomial or diagonal d samples with any K up to DPMM_MAX_K.  A diagonal Gaussian context
+ * runs the sweep only: the device parameter step (dpmm_set_hyper_*, dpmm_posterior_step, dpmm_sample_params,
+ * dpmm_params_merge, dpmm_get_params_*), dpmm_predict_* and dpmm_smart_* return DPMM_ESTATE on it. */
 int dpmm_create(dpmm_ctx** out, const float* x, int64_t n_local, int32_t d, int32_t prior_kind,
                 int32_t device, uint64_t seed, int64_t global_offset);
 /* init_model_from_data for ONE shard of sparse counts: the three arrays of a Julia SparseMatrixCSC{Float32,Int64}
@@ -78,7 +81,8 @@ const char* dpmm_last_error(const dpmm_ctx* ctx);
 /* Use an externally owned cudaStream_t (e.g. the host framework's current stream) for all work. */
 int dpmm_set_stream(dpmm_ctx* ctx, void* cuda_stream);
 int dpmm_sync(dpmm_ctx* ctx);
-/* out[0]=max D (NIW, 64), out[1]=max D (multinomial, 16384), out[2]=max K (1024, any D of either prior). */
+/* out[0]=max D (NIW, 64), out[1]=max D (multinomial and diagonal Gaussian, 16384), out[2]=max K (1024, any D of
+ * every prior). */
 int dpmm_limits(int32_t* out3);
 
 /* ---- labels: initialisation, gather, resume ------------------------------------------------- */
@@ -114,6 +118,12 @@ int dpmm_set_params_niw(dpmm_ctx* ctx, int32_t k, const float* mu, const float* 
 /* log_p float32 [3K][D] = multinomial_dist.alpha (log-probabilities, multinomial_dist.jl:8-10). */
 int dpmm_set_params_multinomial(dpmm_ctx* ctx, int32_t k, const float* log_p, const float* weights,
                                 const float* lr_weights);
+/* Diagonal Gaussian distributions (diag_gaussian), same order and weights as dpmm_set_params_niw:
+ *   mu float32 [3K][D], var float32 [3K][D] (sigma^2_d > 0), logdet float32 [3K] (sum_d log sigma^2_d).
+ * The log-likelihood is -(D log 2pi + logdet)/2 - 1/2 sum_d ((x_d - mu_d)/sigma_d)^2 in Float32, evaluated as
+ * t = fma(s_d, x_d, -s_d mu_d) with s_d = 1/sigma_d (rounded once from Float64), then sum t^2. */
+int dpmm_set_params_diag(dpmm_ctx* ctx, int32_t k, const float* mu, const float* var, const float* logdet,
+                         const float* weights, const float* lr_weights);
 int dpmm_set_sampler(dpmm_ctx* ctx, int32_t sampler);
 
 /* ---- the sweep ------------------------------------------------------------------------------- */
@@ -136,7 +146,9 @@ int dpmm_sample_sublabels(dpmm_ctx* ctx);
  * synchronise), m = number of indices:
  *   counts  int64  [m][3]            N of {cluster, left, right}
  *   sum_x   double [m][3][D]         points_sum
- *   sum_xx  double [m][3][D][D]      S (symmetric; NIW only, ignored for multinomial) */
+ *   sum_xx  double [m][3][D][D]      S (symmetric; NIW),  double [m][3][D]  sum of x_d^2 per feature (diagonal
+ *                                    Gaussian); ignored for multinomial
+ * Gaussian statistics are accumulated in Float64. */
 int dpmm_suff_stats(dpmm_ctx* ctx, const int64_t* indices, int32_t n_indices, int64_t* counts,
                     double* sum_x, double* sum_xx);
 

@@ -12,6 +12,7 @@ const lib = get(ENV, "DPMM_B200_LIB", "libdpmm_b200.so")
 
 const PRIOR_NIW = Cint(0)
 const PRIOR_MULTINOMIAL = Cint(1)
+const PRIOR_DIAG_GAUSSIAN = Cint(2)   # an independent D = 1 NIW per feature (the Python host's diag_niw_hyperparams)
 
 mutable struct Ctx
     ptr::Ptr{Cvoid}
@@ -91,8 +92,9 @@ set_sublabels!(c::Ctx, l::Vector{Int64}) = check(ccall((:dpmm_set_sublabels, lib
     set_params!(c, clusters::Vector{<:thin_cluster_params}, weights::Vector{Float32})
 
 Replaces `broadcast_cluster_params` (local_clusters_actions.jl:518-549).  Packs, for every cluster,
-(cluster_dist, l_dist, r_dist): mv_gaussian fields mu, invSigma, logdetSigma (mv_gaussian.jl:12-18) or
-multinomial_dist.alpha (multinomial_dist.jl:8-10).
+(cluster_dist, l_dist, r_dist): mv_gaussian fields mu, invSigma, logdetSigma (mv_gaussian.jl:12-18),
+multinomial_dist.alpha (multinomial_dist.jl:8-10), or, on a PRIOR_DIAG_GAUSSIAN context, the diagonal Gaussian's
+mu, per-feature variances σ² and logdetΣ = Σ log σ² (dpmm_set_params_diag).
 """
 function set_params!(c::Ctx, clusters, weights::Vector{Float32})
     K = length(clusters)
@@ -110,6 +112,15 @@ function set_params!(c::Ctx, clusters, weights::Vector{Float32})
         GC.@preserve mu inv ld weights lr check(ccall((:dpmm_set_params_niw, lib), Cint,
             (Ptr{Cvoid}, Int32, Ptr{Cfloat}, Ptr{Cfloat}, Ptr{Cfloat}, Ptr{Cfloat}, Ptr{Cfloat}),
             c.ptr, K, mu, inv, ld, weights, lr), c.ptr)
+    elseif c.prior == PRIOR_DIAG_GAUSSIAN
+        D = c.d
+        mu = Array{Float32}(undef, D, 3, K); var = Array{Float32}(undef, D, 3, K); ld = Array{Float32}(undef, 3, K)
+        for (k, cl) in enumerate(clusters), (s, dist) in enumerate(dists(cl))
+            mu[:, s, k] .= dist.μ; var[:, s, k] .= dist.σ²; ld[s, k] = dist.logdetΣ
+        end
+        GC.@preserve mu var ld weights lr check(ccall((:dpmm_set_params_diag, lib), Cint,
+            (Ptr{Cvoid}, Int32, Ptr{Cfloat}, Ptr{Cfloat}, Ptr{Cfloat}, Ptr{Cfloat}, Ptr{Cfloat}),
+            c.ptr, K, mu, var, ld, weights, lr), c.ptr)
     else
         D = c.d
         lp = Array{Float32}(undef, D, 3, K)
@@ -125,7 +136,7 @@ sample_labels!(c::Ctx, final::Bool) = check(ccall((:dpmm_sample_labels, lib), Ci
 sample_sublabels!(c::Ctx) = check(ccall((:dpmm_sample_sublabels, lib), Cint, (Ptr{Cvoid},), c.ptr), c.ptr)
 
 """
-    suff_stats(c, indices) -> (counts[3,m], sum_x[D,3,m], sum_xx[D,D,3,m])
+    suff_stats(c, indices) -> (counts[3,m], sum_x[D,3,m], sum_xx[D,D,3,m] (NIW) or sum_xx[D,3,m] (diagonal Gaussian))
 
 Replaces `update_suff_stats_posterior!`'s remote part (local_clusters_actions.jl:206-236): the caller
 builds niw_sufficient_statistics / multinomial_sufficient_statistics from the three arrays and runs
@@ -134,10 +145,11 @@ calc_posterior unchanged (:237-251).
 function suff_stats(c::Ctx, indices::Vector{Int64})
     m = length(indices); D = c.d
     counts = Array{Int64}(undef, 3, m); sx = Array{Float64}(undef, D, 3, m)
-    sxx = c.prior == PRIOR_NIW ? Array{Float64}(undef, D, D, 3, m) : Array{Float64}(undef, 0, 0, 0, 0)
+    sxx = c.prior == PRIOR_NIW ? Array{Float64}(undef, D, D, 3, m) :
+          c.prior == PRIOR_DIAG_GAUSSIAN ? Array{Float64}(undef, D, 3, m) : Array{Float64}(undef, 0, 0, 0, 0)
     GC.@preserve indices counts sx sxx check(ccall((:dpmm_suff_stats, lib), Cint,
         (Ptr{Cvoid}, Ptr{Int64}, Int32, Ptr{Int64}, Ptr{Cdouble}, Ptr{Cdouble}),
-        c.ptr, indices, m, counts, sx, c.prior == PRIOR_NIW ? pointer(sxx) : C_NULL), c.ptr)
+        c.ptr, indices, m, counts, sx, c.prior == PRIOR_MULTINOMIAL ? C_NULL : pointer(sxx)), c.ptr)
     counts, sx, sxx
 end
 
