@@ -46,11 +46,13 @@ SIGNATURES = {
     "dpmm_num_clusters": (C.c_int, [_p]),
     "dpmm_set_hyper_niw": (C.c_int, [_p, C.c_double, _f64p, C.c_double, _f64p, C.c_double]),
     "dpmm_set_hyper_multinomial": (C.c_int, [_p, _f32p, C.c_double]),
+    "dpmm_set_hyper_diag": (C.c_int, [_p, C.c_double, _f64p, C.c_double, _f64p, C.c_double]),
     "dpmm_posterior_step": (C.c_int, [_p, _i64p, _i32, _i32, _u8p, _i32, _i64p, _f64p, _f64p]),
     "dpmm_sample_params": (C.c_int, [_p, _i32, _i32, _i32]),
     "dpmm_params_merge": (C.c_int, [_p, _i64, _i64]),
     "dpmm_get_params_niw": (C.c_int, [_p, _i32, _f32p, _f64p, _f32p, _f32p, _f32p]),
     "dpmm_get_params_multinomial": (C.c_int, [_p, _i32, _f32p, _f32p, _f32p]),
+    "dpmm_get_params_diag": (C.c_int, [_p, _i32, _f32p, _f32p, _f32p, _f32p, _f32p]),
     "dpmm_predict_niw": (C.c_int, [_p, _i32, _f32p, _f32p, _f32p, _f32p, _i64p, _f32p]),
     "dpmm_predict_multinomial": (C.c_int, [_p, _i32, _f64p, _f32p, _i64p, _f32p]),
     "dpmm_apply_split": (C.c_int, [_p, _i64p, _i64p, _i32]),

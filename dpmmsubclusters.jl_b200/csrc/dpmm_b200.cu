@@ -23,6 +23,7 @@
 #include "kernels_mnm_tc.cuh"
 #include "kernels_pack.cuh"
 #include "kernels_params.cuh"
+#include "kernels_params_diag.cuh"
 #include "kernels_params_mnm.cuh"
 #include "kernels_sort.cuh"
 #include "kernels_stats.cuh"
@@ -55,14 +56,21 @@ static cudaError_t dev_grow_keep(T** p, size_t old_count, size_t new_count) {
 }
 // doubles per distribution of the posterior table (NIW: at the caller's D, also in a zero-padded context)
 static int post_doubles(const dpmm_ctx* c) {
-  return c->prior == DPMM_PRIOR_NIW ? NIW_POST_DOUBLES(c->D_user) : MNM_POST_DOUBLES(c->D);
+  return c->prior == DPMM_PRIOR_NIW ? NIW_POST_DOUBLES(c->D_user)
+       : c->prior == DPMM_PRIOR_DIAG_GAUSSIAN ? DIAG_POST_DOUBLES
+                                               : MNM_POST_DOUBLES(c->D);
+}
+// doubles per distribution of the statistics records (N | sum x | NIW: S, diagonal: sum x^2)
+static int stats_rec_doubles(const dpmm_ctx* c) {
+  const int D = c->D;
+  return c->prior == DPMM_PRIOR_NIW ? 1 + D + D * D : c->prior == DPMM_PRIOR_DIAG_GAUSSIAN ? 1 + 2 * D : 1 + D;
 }
 static int ensure_tables(dpmm_ctx* ctx, int cap) {
   if (cap <= ctx->Kcap_tab) return 0;
   CK(cudaStreamSynchronize(ctx->stream));
   const int D = ctx->D, old = ctx->Kcap_tab;
   const bool niw = ctx->prior == DPMM_PRIOR_NIW;
-  const size_t rec3 = (size_t)3 * (niw ? 1 + D + D * D : 1 + D), post3 = (size_t)3 * post_doubles(ctx);
+  const size_t rec3 = (size_t)3 * stats_rec_doubles(ctx), post3 = (size_t)3 * post_doubles(ctx);
   CK(dev_grow_keep(&ctx->ptab, old * rec3, cap * rec3));
   CK(dev_grow_keep(&ctx->ptab_alt, 0, cap * rec3));
   CK(dev_grow_keep(&ctx->post, old * post3, cap * post3));
@@ -86,10 +94,11 @@ static int ensure_k(dpmm_ctx* ctx, int K) {
   CK(cudaStreamSynchronize(ctx->stream));
   const int D = ctx->D;
   ctx->rec_f = nrec_floats(ctx);
-  ctx->stats_rec = ctx->prior == DPMM_PRIOR_NIW ? 1 + D + D * D : ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN ? 1 + 2 * D : 1 + D;
+  ctx->stats_rec = stats_rec_doubles(ctx);
   // preserve nothing: all K-sized buffers are rewritten by the next set_params / sort
   CK(dev_realloc(&ctx->recs, (size_t)3 * cap * ctx->rec_f));
   if (ctx->prior == DPMM_PRIOR_NIW) CK(dev_realloc(&ctx->raw_params, (size_t)3 * cap * (D + D * D + 1)));
+  if (ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN) CK(dev_realloc(&ctx->raw_params, (size_t)3 * cap * (2 * D + 1)));
   CK(dev_realloc(&ctx->cst, (size_t)3 * cap));
   CK(dev_realloc(&ctx->logw, (size_t)cap));
   CK(dev_realloc(&ctx->loglr, (size_t)2 * cap));
@@ -979,11 +988,22 @@ extern "C" int dpmm_set_params_multinomial(dpmm_ctx* ctx, int32_t K, const float
   return mnm_pack_launch(ctx, K);
 }
 
-// The label kernels' transposed s / b tables from the [2][3K][D] records in ctx->recs (mnm_pack_kernel transposes
-// the cluster rows of one [3K][D] block); logw / loglr / cst are already in place.
+// Every image of the diagonal sweep kernels from the raw parameters in ctx->raw_params = [mu [3K][D] | sigma^2 [3K][D] |
+// logdet [3K]]: the s / b records and cst (diag_pack_kernel), then the label kernels' transposed s / b tables
+// (mnm_pack_kernel transposes the cluster rows of one [3K][D] block); logw / loglr are already in place.
 static int diag_pack_launch(dpmm_ctx* ctx, int K) {
   const int D = ctx->D;
   const int KP = (K + DIAG_KT - 1) / DIAG_KT * DIAG_KT;
+  const size_t nrec = (size_t)3 * K;
+  {
+    DiagPackArgs pa{};
+    pa.D = D; pa.nrec = (int)nrec; pa.mu = ctx->raw_params; pa.var = ctx->raw_params + nrec * D;
+    pa.logdet = ctx->raw_params + 2 * nrec * D; pa.s = ctx->recs; pa.b = ctx->recs + nrec * D; pa.cst = ctx->cst;
+    const int64_t ne = (int64_t)nrec * D;
+    KernelTimer kt(ctx, TK_PARAMS);
+    diag_pack_kernel<<<(unsigned)std::min<int64_t>((ne + 255) / 256, (int64_t)ctx->sm_count * 8), 256, 0, ctx->stream>>>(pa);
+    CK(cudaGetLastError());
+  }
   const int64_t ne = (int64_t)D * KP;
   for (int h = 0; h < 2; ++h) {
     MnmPackArgs pa{};
@@ -1010,29 +1030,20 @@ extern "C" int dpmm_set_params_diag(dpmm_ctx* ctx, int32_t K, const float* mu, c
   if (rc) return rc;
   const int D = ctx->D;
   const size_t nrec = (size_t)3 * K;
-  const size_t bytes = (2 * nrec * D + nrec + K + 2 * K) * sizeof(float);
+  // raw parameters -> pinned staging -> device; s = 1/sigma, b = -s mu and cst are derived on the device
+  const size_t raw_floats = 2 * nrec * D + nrec;
+  const size_t bytes = (raw_floats + K + 2 * K) * sizeof(float);
   void* hs = nullptr;
   const int slot = upload_acquire(ctx, bytes, &hs);
   if (slot < 0) return slot;
-  float* h_s = (float*)hs;
-  float* h_b = h_s + nrec * D;
-  float* h_cst = h_b + nrec * D;
-  float* h_logw = h_cst + nrec;
+  float* h_raw = (float*)hs;
+  float* h_logw = h_raw + raw_floats;
   float* h_loglr = h_logw + K;
-  // s = 1/sigma and b = -s mu, each rounded once from Float64 (the oracle restates exactly this)
-  const double log2pi = 1.8378770664093453;
-  for (size_t t = 0; t < nrec; ++t) {
-    for (int d = 0; d < D; ++d) {
-      const size_t e = t * D + d;
-      const float sv = (float)(1.0 / std::sqrt((double)var[e]));
-      h_s[e] = sv;
-      h_b[e] = (float)(-(double)sv * (double)mu[e]);
-    }
-    h_cst[t] = (float)(-0.5 * ((double)D * log2pi + (double)logdet[t]));
-  }
+  memcpy(h_raw, mu, nrec * D * 4);
+  memcpy(h_raw + nrec * D, var, nrec * D * 4);
+  memcpy(h_raw + 2 * nrec * D, logdet, nrec * 4);
   common_weights(ctx, K, weights, lr_weights, h_logw, h_loglr);
-  CK(cudaMemcpyAsync(ctx->recs, h_s, 2 * nrec * D * 4, cudaMemcpyHostToDevice, ctx->stream));
-  CK(cudaMemcpyAsync(ctx->cst, h_cst, nrec * 4, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(ctx->raw_params, h_raw, raw_floats * 4, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemcpyAsync(ctx->logw, h_logw, (size_t)K * 4, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemcpyAsync(ctx->loglr, h_loglr, (size_t)2 * K * 4, cudaMemcpyHostToDevice, ctx->stream));
   rc = upload_release(ctx, slot);
@@ -1714,7 +1725,7 @@ extern "C" int dpmm_suff_stats(dpmm_ctx* ctx, const int64_t* indices, int32_t n_
 
 
 // ------------------------------------------------------------------------------------------------
-// device-side parameter step (NIW and multinomial): SURVEY.md 8f-1
+// device-side parameter step (NIW, multinomial and diagonal Gaussian): SURVEY.md 8f-1
 // ------------------------------------------------------------------------------------------------
 extern "C" int dpmm_num_clusters(const dpmm_ctx* ctx) { return ctx ? keff(ctx) : 0; }
 
@@ -1784,14 +1795,50 @@ extern "C" int dpmm_set_hyper_multinomial(dpmm_ctx* ctx, const float* alpha_prio
   return ensure_tables(ctx, std::max(ctx->Kcap, 8));
 }
 
+extern "C" int dpmm_set_hyper_diag(dpmm_ctx* ctx, double kappa, const double* m, double nu, const double* psi, double alpha) {
+  NEED(ctx && m && psi, DPMM_EINVAL, "NULL argument");
+  NEED(ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN, DPMM_ESTATE, "not a diagonal Gaussian context");
+  NEED(kappa > 0 && nu > 0 && alpha > 0, DPMM_EINVAL, "need kappa > 0, nu > 0, alpha > 0");
+  // diag_niw_hyperparams stores kappa and nu as Float32, as niw_hyperparams does
+  const double kf = (double)(float)kappa, nf = (double)(float)nu;
+  NEED(kf > 0 && std::isfinite(kf) && nf > 0 && std::isfinite(nf), DPMM_EINVAL, "kappa and nu must be finite and > 0 in Float32");
+  CK(cudaSetDevice(ctx->device));
+  const int D = ctx->D;
+  std::vector<double> h(DIAG_HYPER_DOUBLES(D));
+  double slp = 0.0;
+  for (int d = 0; d < D; ++d) {
+    NEED(std::isfinite(m[d]), DPMM_EINVAL, "every m[d] must be finite");
+    NEED(std::isfinite(psi[d]) && psi[d] > 0, DPMM_EINVAL, "every psi[d] must be finite and > 0");
+    h[4 + d] = m[d];
+    h[4 + D + d] = psi[d];
+    slp += std::log(psi[d]);
+  }
+  h[0] = kf; h[1] = nf; h[2] = slp;
+  h[3] = (double)(float)std::lgamma(nf / 2.0);   // log_multivariate_gamma(nu / 2, 1)
+  if (!ctx->hyper_d) CK(cudaMalloc((void**)&ctx->hyper_d, h.size() * 8));
+  CK(cudaStreamSynchronize(ctx->stream));
+  CK(cudaMemcpy(ctx->hyper_d, h.data(), h.size() * 8, cudaMemcpyHostToDevice));
+  ctx->alpha = (double)(float)alpha;
+  ctx->dev_params = true;
+  return ensure_tables(ctx, std::max(ctx->Kcap, 8));
+}
+
 #define DPMM_NEED_HYPER(what) \
-  NEED(ctx->dev_params, DPMM_ESTATE, "dpmm_set_hyper_niw or dpmm_set_hyper_multinomial must precede " what \
-       " (a diagonal Gaussian context has no device parameter step)")
+  NEED(ctx->dev_params, DPMM_ESTATE, "dpmm_set_hyper_niw, dpmm_set_hyper_multinomial or dpmm_set_hyper_diag must precede " what)
 
 static size_t niw_post_smem(int D) { return ((size_t)D * (D + 1) + 2 * D) * sizeof(double); }   // D: the caller's
 
 // posterior + log marginal likelihood of the listed clusters (device list idx_d, or all m = K in order) from the table
 static int launch_post(dpmm_ctx* ctx, const int32_t* idx_d, int m, double* out) {
+  if (ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN) {
+    DiagPostArgs pa{};
+    pa.D = ctx->D; pa.rec = ctx->stats_rec; pa.hyper = ctx->hyper_d; pa.ptab = ctx->ptab; pa.idx_list = idx_d;
+    pa.post = ctx->post; pa.out = out;
+    KernelTimer kt(ctx, TK_PARAMS);
+    diag_post_kernel<<<dim3((unsigned)m, 3), DIAG_PARAM_THREADS, 0, ctx->stream>>>(pa);
+    CK(cudaGetLastError());
+    return 0;
+  }
   if (ctx->prior == DPMM_PRIOR_MULTINOMIAL) {
     MnmPostArgs pa{};
     pa.D = ctx->D; pa.rec = ctx->stats_rec; pa.hyper = ctx->hyper_d; pa.ptab = ctx->ptab; pa.idx_list = idx_d;
@@ -1869,6 +1916,14 @@ extern "C" int dpmm_posterior_step(dpmm_ctx* ctx, const int64_t* indices, int32_
       if (rcf) return rcf;
       ctx->launches += 1;
       mnm_merge_kernel<<<grid, MNM_PARAM_THREADS, 0, ctx->side>>>(ma);
+    } else if (ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN) {
+      DiagMergeArgs ma{};
+      ma.D = ctx->D; ma.rec = rec; ma.K = k_merge; ma.hyper = ctx->hyper_d; ma.ptab = ctx->ptab;
+      ma.splittable = ctx->splittable_d; ma.out = merge_d;
+      int rcf = side_fork(ctx);
+      if (rcf) return rcf;
+      ctx->launches += 1;
+      diag_merge_kernel<<<grid, DIAG_PARAM_THREADS, 0, ctx->side>>>(ma);
     } else {
       NiwMergeArgs ma{};
       ma.D = ctx->D_user; ma.ld = ctx->D; ma.rec = rec; ma.K = k_merge; ma.hyper = ctx->hyper_d; ma.ptab = ctx->ptab;
@@ -1949,6 +2004,20 @@ extern "C" int dpmm_sample_params(dpmm_ctx* ctx, int32_t K, int32_t from_prior, 
     if (rc) return rc;
     return side_join(ctx);
   }
+  if (ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN) {
+    DiagDrawArgs da{};
+    da.D = D; da.rec = ctx->stats_rec; da.hyper = ctx->hyper_d; da.ptab = ctx->ptab; da.post = ctx->post;
+    da.mu = ctx->raw_params; da.var = ctx->raw_params + nrec * D; da.logdet = ctx->raw_params + 2 * nrec * D;
+    da.seed = ctx->seed; da.call = ctx->pcall; da.first = from_prior;
+    {
+      KernelTimer kt(ctx, TK_PARAMS);
+      diag_draw_kernel<<<(unsigned)nrec, DIAG_PARAM_THREADS, 0, ctx->stream>>>(da);
+      CK(cudaGetLastError());
+    }
+    rc = diag_pack_launch(ctx, K);
+    if (rc) return rc;
+    return side_join(ctx);
+  }
   {
     const int Du = ctx->D_user;
     NiwDrawArgs da{};
@@ -2015,6 +2084,22 @@ extern "C" int dpmm_get_params_multinomial(dpmm_ctx* ctx, int32_t K, float* log_
   NEED(ctx->dev_params && ctx->params_set && K == ctx->K, DPMM_ESTATE, "no device-sampled parameters for this K");
   CK(cudaStreamSynchronize(ctx->stream));
   if (log_p) CK(cudaMemcpy(log_p, ctx->recs, (size_t)3 * K * ctx->D * 4, cudaMemcpyDeviceToHost));
+  if (weights) CK(cudaMemcpy(weights, ctx->w_out, (size_t)K * 4, cudaMemcpyDeviceToHost));
+  if (lr_weights) CK(cudaMemcpy(lr_weights, ctx->lr_out, (size_t)2 * K * 4, cudaMemcpyDeviceToHost));
+  return 0;
+}
+
+extern "C" int dpmm_get_params_diag(dpmm_ctx* ctx, int32_t K, float* mu, float* var, float* logdet, float* weights,
+                                    float* lr_weights) {
+  NEED(ctx, DPMM_EINVAL, "ctx is NULL");
+  CK(cudaSetDevice(ctx->device));
+  NEED(ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN, DPMM_ESTATE, "not a diagonal Gaussian context");
+  NEED(ctx->dev_params && ctx->params_set && K == ctx->K, DPMM_ESTATE, "no device-sampled parameters for this K");
+  const size_t nrec = (size_t)3 * K, D = (size_t)ctx->D;
+  CK(cudaStreamSynchronize(ctx->stream));
+  if (mu) CK(cudaMemcpy(mu, ctx->raw_params, nrec * D * 4, cudaMemcpyDeviceToHost));
+  if (var) CK(cudaMemcpy(var, ctx->raw_params + nrec * D, nrec * D * 4, cudaMemcpyDeviceToHost));
+  if (logdet) CK(cudaMemcpy(logdet, ctx->raw_params + 2 * nrec * D, nrec * 4, cudaMemcpyDeviceToHost));
   if (weights) CK(cudaMemcpy(weights, ctx->w_out, (size_t)K * 4, cudaMemcpyDeviceToHost));
   if (lr_weights) CK(cudaMemcpy(lr_weights, ctx->lr_out, (size_t)2 * K * 4, cudaMemcpyDeviceToHost));
   return 0;

@@ -491,9 +491,12 @@ def _clusters_from_device(group, st, cfg):
     if params is not None and params[0].shape[0] != K:
         params = None                                     # K changed after the parameters were fetched (mid-run checkpoint)
     niw = isinstance(hyper, P.niw_hyperparams)
+    diag = isinstance(hyper, P.diag_niw_hyperparams)
     if params is not None:
         if niw:
             mu, lfac, logdet, w, lr = params
+        elif diag:
+            mu, var, logdet, w, lr = params
         else:
             log_p, w, lr = params
     else:
@@ -508,7 +511,12 @@ def _clusters_from_device(group, st, cfg):
         for s_ in range(3):
             ss = P.make_suff_stats(hyper, counts[k, s_], sum_x[k, s_], None if sum_xx is None else sum_xx[k, s_])
             post = P.calc_posterior(hyper, ss)
-            if not niw:
+            if diag:
+                if params is not None:
+                    dist = P.diag_gaussian(mu[k, s_].copy(), var[k, s_].copy(), float(logdet[k, s_]))
+                else:
+                    dist = P.diag_gaussian(post.m.astype(F32), post.ψ.astype(F32), float(F32(np.log(post.ψ).sum())))
+            elif not niw:
                 if params is not None:
                     dist = P.multinomial_dist(log_p[k, s_].copy())
                 else:
@@ -539,8 +547,8 @@ def dp_parallel(all_data, local_hyper_params=None, α_param=None, iters=100, ini
     """dp_parallel :121-157.  `sweep_factory`, `shard`, `comm`, `device`, `device_params` have no reference
     counterpart: they select the device / inject a test double / attach the multi-GPU communicator / choose
     where the parameter step runs (default: on the device for the NIW prior, SURVEY 8f-1, and on the host for the
-    multinomial prior, which takes the device with device_params=True; False = the Python mirror of the reference's
-    master functions below)."""
+    multinomial and diagonal Gaussian priors, which take the device with device_params=True; False = the Python mirror
+    of the reference's master functions below)."""
     if isinstance(all_data, (str, os.PathLike)):
         return dp_parallel_params_file(str(all_data), verbose=verbose, gt=gt, sweep_factory=sweep_factory, shard=shard,
                                        comm=comm, device=device, device_params=device_params)
@@ -570,8 +578,6 @@ def _run_from_settings(all_data, local_hyper_params, α_param, cfg, seed, sweep_
     """init_model + init_first_clusters! + run_model for fresh runs; create_model_from_saved_data + run_model(iter + 1)
     when `restored` = (pts_less_group dict, iter) of a checkpoint."""
     if isinstance(local_hyper_params, P.diag_niw_hyperparams):
-        if device_params:
-            raise ValueError("device_params: the device parameter step runs the NIW and multinomial priors only")
         if cfg.use_smart_splits:
             raise ValueError("smart splits need the full scatter matrix: not available with the diagonal prior")
     if restored is not None and seed is not None:
@@ -583,7 +589,10 @@ def _run_from_settings(all_data, local_hyper_params, α_param, cfg, seed, sweep_
     if comm is not None:
         sw.comm_init(*comm)
     niw = isinstance(local_hyper_params, P.niw_hyperparams)
-    if device_params is None:                              # (multinomial: the host loop unless asked for explicitly)
+    if device_params and isinstance(local_hyper_params, P.diag_niw_hyperparams) and not hasattr(sw, "sample_params"):
+        raise ValueError("device_params: this sweep has no device parameter step; off the GPU, device_params is "
+                         "accepted for the NIW and multinomial priors only, which fall back to the host loop")
+    if device_params is None:                              # (multinomial, diagonal: the host loop unless asked for)
         device_params = niw and os.environ.get("DPMM_DEVICE_PARAMS", "1") != "0"
     first_iter = 1
     if restored is not None:                               # create_model_from_saved_data, ds.jl:89-92; :437-439

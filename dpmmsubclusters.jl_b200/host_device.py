@@ -1,7 +1,7 @@
-"""Host loop for the device-side parameter step (NIW and multinomial priors; SURVEY.md 8f-1).
+"""Host loop for the device-side parameter step (NIW, multinomial and diagonal Gaussian priors; SURVEY.md 8f-1).
 
-What stays here is what north_star leaves to the host once the K x D^2 (NIW) or K x D (multinomial) work has
-moved: cluster
+What stays here is what north_star leaves to the host once the K x D^2 (NIW) or K x D (multinomial, diagonal) work
+has moved: cluster
 bookkeeping and the Hastings accept / reject decisions on scalars.  Per iteration the host reads one
 small block back from the device -- 3K counts, 3K log marginal likelihoods and the K x K table of merged
 log marginal likelihoods (GpuSweep.posterior_step) -- and issues the relabel operations.  Written from the
@@ -22,7 +22,7 @@ import numpy as np
 from scipy.special import gammaln
 
 from . import priors as P
-from .sweep import NIW
+from .sweep import DIAG, NIW
 
 
 class DeviceState:
@@ -72,7 +72,8 @@ def group_step_device(sw, st, α, no_more_splits, final, cfg, rng, keep_params=F
     history_step(st, cfg)
     sw.sample_params(st.K)
     if keep_params:                                        # the distributions fit() returns (last iteration only)
-        st.params = sw.get_params_niw(st.K) if sw.prior_kind == NIW else sw.get_params_multinomial(st.K)
+        get = {NIW: sw.get_params_niw, DIAG: sw.get_params_diag}.get(sw.prior_kind, sw.get_params_multinomial)
+        st.params = get(st.K)
     sw.sample_labels(True if cfg.hard_clustering else final)
     sw.sample_sublabels()
     # update_suff_stats_posterior! for every cluster; the merge table rides along when merges are possible
@@ -182,6 +183,8 @@ def run_model_device(dp_model, cfg, rng, normalized_mutual_info, first_iter=1, r
     α = g.model_hyperparams.α
     if isinstance(hyper, P.niw_hyperparams):
         sw.set_hyper_niw(hyper.κ, hyper.m, hyper.ν, hyper.ψ, α)
+    elif isinstance(hyper, P.diag_niw_hyperparams):
+        sw.set_hyper_diag(hyper.κ, hyper.m, hyper.ν, hyper.ψ, α)
     else:
         sw.set_hyper_multinomial(hyper.α, α)
     if resume:

@@ -225,6 +225,14 @@ class GpuSweep:
         assert a.shape == (self.D,)
         self._ck(self.lib.dpmm_set_hyper_multinomial(self.h, _ptr(a, C.c_float), float(alpha)))
 
+    def set_hyper_diag(self, kappa, m, nu, psi, alpha):
+        """diag_niw_hyperparams: m [D] and psi [D] (per-feature), shared kappa and nu."""
+        m = np.ascontiguousarray(m, np.float64).reshape(-1)
+        psi = np.ascontiguousarray(psi, np.float64).reshape(-1)
+        assert m.shape == (self.D,) and psi.shape == (self.D,)
+        self._ck(self.lib.dpmm_set_hyper_diag(self.h, float(kappa), _ptr(m, C.c_double), float(nu), _ptr(psi, C.c_double),
+                                              float(alpha)))
+
     def posterior_step(self, indices=None, splittable=None, from_table=False, fetch=True):
         """Statistics (unless from_table) -> table -> posteriors.  Returns (counts [m,3] i64, logml [m,3] f64,
         merge [K,K] f64 or None); `splittable` (bool [K]) requests the merge table."""
@@ -273,6 +281,17 @@ class GpuSweep:
         self._ck(self.lib.dpmm_get_params_multinomial(self.h, int(K), _ptr(lp, C.c_float), _ptr(w, C.c_float),
                                                       _ptr(lr, C.c_float)))
         return lp, w, lr
+
+    def get_params_diag(self, K):
+        """(mu [K,3,D] f32, var [K,3,D] f32 (sigma^2), logdet [K,3] f32, weights [K] f32, lr [K,2] f32)."""
+        mu = np.empty((K, 3, self.D), np.float32)
+        var = np.empty((K, 3, self.D), np.float32)
+        ld = np.empty((K, 3), np.float32)
+        w = np.empty(K, np.float32)
+        lr = np.empty((K, 2), np.float32)
+        self._ck(self.lib.dpmm_get_params_diag(self.h, int(K), _ptr(mu, C.c_float), _ptr(var, C.c_float), _ptr(ld, C.c_float),
+                                               _ptr(w, C.c_float), _ptr(lr, C.c_float)))
+        return mu, var, ld, w, lr
 
     def predict_niw(self, u, mu, tconst, df, want_probs=True):
         """Posterior-predictive labels (and probabilities) of this context's points; see dpmm_predict_niw."""

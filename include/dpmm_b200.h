@@ -56,8 +56,8 @@ typedef struct dpmm_ctx dpmm_ctx;
  * device: CUDA ordinal.  seed: replaces `@everywhere Random.seed!(seed)` (:37-39).
  * d: 1..64 for the NIW prior, 1..16384 for the multinomial and the diagonal Gaussian prior; larger d returns
  * DPMM_ELIMIT.  Every multinomial or diagonal d samples with any K up to DPMM_MAX_K.  A diagonal Gaussian context
- * runs the sweep only: the device parameter step (dpmm_set_hyper_*, dpmm_posterior_step, dpmm_sample_params,
- * dpmm_params_merge, dpmm_get_params_*), dpmm_predict_* and dpmm_smart_* return DPMM_ESTATE on it. */
+ * runs the sweep and, after dpmm_set_hyper_diag, the device parameter step; dpmm_predict_* and dpmm_smart_* return
+ * DPMM_ESTATE on it. */
 int dpmm_create(dpmm_ctx** out, const float* x, int64_t n_local, int32_t d, int32_t prior_kind,
                 int32_t device, uint64_t seed, int64_t global_offset);
 /* init_model_from_data for ONE shard of sparse counts: the three arrays of a Julia SparseMatrixCSC{Float32,Int64}
@@ -121,7 +121,9 @@ int dpmm_set_params_multinomial(dpmm_ctx* ctx, int32_t k, const float* log_p, co
 /* Diagonal Gaussian distributions (diag_gaussian), same order and weights as dpmm_set_params_niw:
  *   mu float32 [3K][D], var float32 [3K][D] (sigma^2_d > 0), logdet float32 [3K] (sum_d log sigma^2_d).
  * The log-likelihood is -(D log 2pi + logdet)/2 - 1/2 sum_d ((x_d - mu_d)/sigma_d)^2 in Float32, evaluated as
- * t = fma(s_d, x_d, -s_d mu_d) with s_d = 1/sigma_d (rounded once from Float64), then sum t^2. */
+ * t = fma(s_d, x_d, -s_d mu_d) with s_d = 1/sigma_d (rounded once from Float64), then sum t^2.  The images are
+ * derived on the device by the same kernel that packs device-sampled parameters (dpmm_sample_params), so that
+ * dpmm_get_params_diag -> dpmm_set_params_diag reproduces them bit for bit. */
 int dpmm_set_params_diag(dpmm_ctx* ctx, int32_t k, const float* mu, const float* var, const float* logdet,
                          const float* weights, const float* lr_weights);
 int dpmm_set_sampler(dpmm_ctx* ctx, int32_t sampler);
@@ -158,7 +160,8 @@ int dpmm_num_clusters(const dpmm_ctx* ctx);
 
 /* ---- device-side parameter step (NIW and multinomial; SURVEY 8f-1) ----------------------------
  * Optional: the host may keep sampling parameters itself (dpmm_set_params_*).  With these calls the
- * per-iteration master work that scales with K D^3 (NIW) or K D (multinomial) runs next to the statistics:
+ * per-iteration master work that scales with K D^3 (NIW) or K D (multinomial, diagonal Gaussian) runs next to the
+ * statistics:
  *   calc_posterior / log_marginal_likelihood   src/priors/niw.jl:20-31, 53-62; multinomial_prior.jl:16-21, 34-39
  *   sample_distribution                        src/priors/niw.jl:34-40; multinomial_prior.jl:23-25
  *   sample_cluster_params / sample_clusters!   src/shared_actions.jl:41-66, src/local_clusters_actions.jl:417-437
@@ -172,6 +175,11 @@ int dpmm_set_hyper_niw(dpmm_ctx* ctx, double kappa, const double* m, double nu, 
 /* multinomial_hyper (multinomial_prior.jl:6-8: alpha_prior float32 [D], every entry finite and > 0) and the
  * concentration alpha > 0 (ds.jl:9).  DPMM_ESTATE on an NIW context. */
 int dpmm_set_hyper_multinomial(dpmm_ctx* ctx, const float* alpha_prior, double alpha);
+/* diag_niw_hyperparams (kappa, m double [D], nu, psi double [D]: an independent NIW at D = 1 per feature, shared kappa
+ * and nu) and the concentration alpha.  kappa, nu and alpha are kept rounded to Float32.  DPMM_EINVAL for a NULL
+ * pointer, kappa <= 0, nu <= 0, alpha <= 0, a non-finite m[d] or a psi[d] that is not finite and > 0; DPMM_ESTATE on
+ * a context of another prior. */
+int dpmm_set_hyper_diag(dpmm_ctx* ctx, double kappa, const double* m, double nu, const double* psi, double alpha);
 /* update_suff_stats_posterior! (local_clusters_actions.jl:206-254) kept on the device: statistics of the
  * listed clusters (NULL = all) -> all-reduce -> persistent table -> posterior hyper-parameters and log
  * marginal likelihoods of {cluster, left, right}.  from_table != 0: skip the statistics and re-evaluate the
@@ -198,6 +206,11 @@ int dpmm_get_params_niw(dpmm_ctx* ctx, int32_t k, float* mu, double* lfac, float
 /* The parameters of the last dpmm_sample_params of a multinomial context: log_p float32 [3K][D]
  * (multinomial_dist.alpha), weights float32 [K], lr_weights float32 [K][2].  Each output may be NULL. */
 int dpmm_get_params_multinomial(dpmm_ctx* ctx, int32_t k, float* log_p, float* weights, float* lr_weights);
+/* The parameters of the last dpmm_sample_params of a diagonal Gaussian context (diag_gaussian): mu float32 [3K][D],
+ * var float32 [3K][D] (sigma^2), logdet float32 [3K] (sum_d log sigma^2_d over the Float32 var), weights float32 [K],
+ * lr_weights float32 [K][2].  Each output may be NULL.  DPMM_ESTATE without device-sampled parameters for this K. */
+int dpmm_get_params_diag(dpmm_ctx* ctx, int32_t k, float* mu, float* var, float* logdet, float* weights,
+                         float* lr_weights);
 
 /* predict / predict_points (src/dp-parallel-sampling.jl:509-537, src/local_clusters_actions.jl:23-40) for the
  * points of THIS context under K NIW posterior predictives (multivariate Student-t, niw.jl:68-76):

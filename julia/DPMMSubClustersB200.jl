@@ -183,6 +183,18 @@ set_hyper!(c::Ctx, α_prior::Vector{Float32}, α::Real) =
         (Ptr{Cvoid}, Ptr{Cfloat}, Cdouble), c.ptr, α_prior, α), c.ptr)
 
 """
+    set_hyper!(c, h::diag_niw_hyperparams, α)
+
+The diagonal Gaussian prior of a PRIOR_DIAG_GAUSSIAN context: shared κ and ν, per-feature `m[D]` and `ψ[D]` (an
+independent NIW at D = 1 per feature).  Afterwards posterior_step, sample_params!, params_merge! and
+get_params_diag run on that context.
+"""
+function set_hyper!(c::Ctx, κ::Real, m::Vector{Float64}, ν::Real, ψ::Vector{Float64}, α::Real)
+    GC.@preserve m ψ check(ccall((:dpmm_set_hyper_diag, lib), Cint,
+        (Ptr{Cvoid}, Cdouble, Ptr{Cdouble}, Cdouble, Ptr{Cdouble}, Cdouble), c.ptr, κ, m, ν, ψ, α), c.ptr)
+end
+
+"""
     posterior_step(c, indices; splittable=nothing, from_table=false) -> (counts[3,m], logml[3,m], merge[K,K] or nothing)
 
 update_suff_stats_posterior! (local_clusters_actions.jl:206-254) kept on the device.  `indices === nothing`
@@ -226,6 +238,16 @@ function get_params_multinomial(c::Ctx, K::Integer)
     GC.@preserve lp w lr check(ccall((:dpmm_get_params_multinomial, lib), Cint,
         (Ptr{Cvoid}, Int32, Ptr{Cfloat}, Ptr{Cfloat}, Ptr{Cfloat}), c.ptr, K, lp, w, lr), c.ptr)
     lp, w, lr
+end
+
+"(mu[D,3,K], σ²[D,3,K], logdetΣ[3,K] = Σ log σ², weights[K], lr[2,K]) of a PRIOR_DIAG_GAUSSIAN context"
+function get_params_diag(c::Ctx, K::Integer)
+    D = c.d
+    mu = Array{Float32}(undef, D, 3, K); var = Array{Float32}(undef, D, 3, K); ld = Array{Float32}(undef, 3, K)
+    w = Vector{Float32}(undef, K); lr = Array{Float32}(undef, 2, K)
+    GC.@preserve mu var ld w lr check(ccall((:dpmm_get_params_diag, lib), Cint,
+        (Ptr{Cvoid}, Int32, Ptr{Cfloat}, Ptr{Cfloat}, Ptr{Cfloat}, Ptr{Cfloat}, Ptr{Cfloat}), c.ptr, K, mu, var, ld, w, lr), c.ptr)
+    mu, var, ld, w, lr
 end
 
 """

@@ -1,7 +1,14 @@
 """Per-stage device times of diagonal Gaussian sweeps (DPMM_PRIOR_DIAG_GAUSSIAN) at four shapes, and fit() iterations
-per second at G1, one JSON line per measurement on stdout and in profiles/diag_bench.jsonl.
+per second with the parameter step on the device and on the host, one JSON line per measurement on stdout and in
+profiles/diag_bench.jsonl.
 
-    python tools/bench_diag.py [--shapes G1,G2,G3,G4] [--sweeps 20] [--warmup 3] [--fit-iters 40]
+    python tools/bench_diag.py [--shapes G1,G2,G3,G4] [--sweeps 20] [--warmup 3] [--fit-shapes G1,G2,G3]
+                               [--fit-iters 40] [--fit-reps 2]
+
+fit() runs from one cluster on data drawn like the sweep shapes', the two paths alternated --fit-reps times each; it
+reports iterations per second inside the loop and for the whole call.  One more fit per path runs with kernel timing
+on and reports the `params` kernel time per iteration (the device parameter step and the packing of the parameter
+images; on the host path only the packing).
 
 Stage times come from dpmm_timing_read (CUDA events around each kernel), after the warm-up sweeps.  Each stage's
 share is of the larger of its two bounds, computed from the shapes here:
@@ -98,16 +105,43 @@ def run_shape(pkg, tag, n, D, K, sweeps, warmup, ffma_tflops, hbm_gbs):
                 label_tflops=4.0 * n * K * D / (ms["label"] * 1e-3) / 1e12)
 
 
-def run_fit(pkg, iters):
-    from dpmmsubclusters_jl_b200 import host as H, priors as P
-    n, D, K = SHAPES["G1"]
+def run_fit(pkg, tag, iters, reps):
+    from dpmmsubclusters_jl_b200 import priors as P
+    n, D, K = SHAPES[tag]
     x, _, _ = make_data(n, D, K, 7)
+    xt = x.T
     hyper = P.diag_niw_hyperparams(1.0, np.zeros(D), 10.0, np.ones(D))
-    t0 = time.perf_counter()
-    labels, clusters, _, iter_count, *_ = pkg.fit(x.T, hyper, 10.0, iters=iters, seed=1, burnout=10)
-    wall = time.perf_counter() - t0
-    return dict(shape="G1-fit", n=n, D=D, K_true=K, K_final=len(clusters), init_clusters=1, iters=iters,
-                fit_iters_per_s=len(iter_count) / float(np.sum(iter_count)), fit_wall_s=wall)
+    made = []
+
+    def factory(timing):
+        def make(xx, kind, seed, goff):
+            g = pkg.GpuSweep(xx, kind, seed=seed, global_offset=goff)
+            g.timing_enable(timing)
+            made.append(g)
+            return g
+        return make
+
+    def one(dev, timing):
+        made.clear()
+        t0 = time.perf_counter()
+        _, clusters, _, iter_count, *_ = pkg.fit(xt, hyper, 10.0, iters=iters, seed=1, burnout=10, device_params=dev,
+                                                 sweep_factory=factory(timing))
+        made[0].sync()
+        wall = time.perf_counter() - t0
+        params_ms = made[0].timing_read(reset=True)["params"][0] / len(iter_count) if timing else None
+        return len(clusters), len(iter_count) / float(np.sum(iter_count)), len(iter_count) / wall, params_ms
+
+    recs = {dev: dict(shape=f"{tag}-fit", path="device" if dev else "host", n=n, D=D, K_true=K, init_clusters=1,
+                      iters=iters, loop_iters_per_s=[], call_iters_per_s=[], K_final=[]) for dev in (True, False)}
+    for _ in range(reps):
+        for dev in (True, False):
+            kf, loop, call, _ = one(dev, False)
+            recs[dev]["loop_iters_per_s"].append(loop)
+            recs[dev]["call_iters_per_s"].append(call)
+            recs[dev]["K_final"].append(kf)
+    for dev in (True, False):
+        recs[dev]["params_kernel_ms_per_iter"] = one(dev, True)[3]
+    return [recs[True], recs[False]]
 
 
 def main():
@@ -115,7 +149,9 @@ def main():
     ap.add_argument("--shapes", default="G1,G2,G3,G4")
     ap.add_argument("--sweeps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--fit-shapes", default="G1,G2,G3")
     ap.add_argument("--fit-iters", type=int, default=40)
+    ap.add_argument("--fit-reps", type=int, default=2)
     ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "diag_bench.jsonl"))
     args = ap.parse_args()
     import bench
@@ -131,7 +167,8 @@ def main():
         n, D, K = SHAPES[tag]
         recs.append(run_shape(pkg, tag, n, D, K, args.sweeps, args.warmup, bench.FFMA2_PEAK_TFLOPS, hbm_gbs))
     if args.fit_iters > 0:
-        recs.append(run_fit(pkg, args.fit_iters))
+        for tag in filter(None, args.fit_shapes.split(",")):
+            recs.extend(run_fit(pkg, tag, args.fit_iters, args.fit_reps))
     with open(args.out, "w") as f:
         for r in recs:
             r.update(device=name, power_limit_and_max_sm_clock=power, ffma2_peak_tflops=bench.FFMA2_PEAK_TFLOPS, hbm_gbs=hbm_gbs)
