@@ -47,6 +47,9 @@ SIGNATURES = {
     "dpmm_set_hyper_niw": (C.c_int, [_p, C.c_double, _f64p, C.c_double, _f64p, C.c_double]),
     "dpmm_set_hyper_multinomial": (C.c_int, [_p, _f32p, C.c_double]),
     "dpmm_set_hyper_diag": (C.c_int, [_p, C.c_double, _f64p, C.c_double, _f64p, C.c_double]),
+    "dpmm_set_outlier_niw": (C.c_int, [_p, C.c_double, C.c_double, _f64p, C.c_double, _f64p]),
+    "dpmm_set_outlier_multinomial": (C.c_int, [_p, C.c_double, _f32p]),
+    "dpmm_set_outlier_diag": (C.c_int, [_p, C.c_double, C.c_double, _f64p, C.c_double, _f64p]),
     "dpmm_posterior_step": (C.c_int, [_p, _i64p, _i32, _i32, _u8p, _i32, _i64p, _f64p, _f64p]),
     "dpmm_sample_params": (C.c_int, [_p, _i32, _i32, _i32]),
     "dpmm_params_merge": (C.c_int, [_p, _i64, _i64]),

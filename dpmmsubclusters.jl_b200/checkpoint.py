@@ -8,7 +8,8 @@
 The reference stores its checkpoints as JLD2 (serialised Julia structs).  Here a checkpoint is one `.npz` of plain
 arrays holding the same five items -- `group` (the pts_less_group: hyper-parameters, labels, sub-labels, every
 local_cluster, weights), `hyperparams`, `iter`, `total_time`, `global_params` -- which NPZ.jl (a dependency the
-reference already has) reads on the Julia side.  Labels and sub-labels are restored through
+reference already has) reads on the Julia side.  A model with the outlier component also stores its weight and prior
+as `outlier_weight` and `outlier_*` next to `prior_*`; files without them hold a model without the component.  Labels and sub-labels are restored through
 dpmm_set_labels / dpmm_set_sublabels (`group.labels = distribute(group.labels)`, :437-439); X is reloaded from
 `data_path`/`data_prefix` exactly as the reference does.
 """
@@ -114,6 +115,9 @@ def save_model(model, path, filename, iter, total_time, global_params):
            "labels_subcluster": np.asarray(g.sweep.get_sublabels(), np.int64),
            "weights": np.asarray(g.weights, F32)}
     _hyper_arrays(hyper, "prior_", out)
+    if getattr(model, "outlier_weight", 0) > 0:
+        out["outlier_weight"] = np.float64(model.outlier_weight)
+        _hyper_arrays(model.outlier_params, "outlier_", out)
     trip = lambda c: (c.cluster_params.cluster_params, c.cluster_params.cluster_params_l, c.cluster_params.cluster_params_r)
     stack = lambda f, dt=np.float64: np.array([[f(cp) for cp in trip(c)] for c in g.local_clusters], dt).reshape(
         (K, 3) + np.shape(f(trip(g.local_clusters[0])[0]))) if K else np.zeros((0, 3), dt)
@@ -168,6 +172,9 @@ def load_checkpoint(filename):
     kind = meta["kind"]
     prior = _hyper_from(z, "prior_", kind)
     mh = H.model_hyper_params(prior, meta["alpha"], meta["total_dim"])
+    ow, op = 0.0, None
+    if "outlier_weight" in z.files:
+        ow, op = float(z["outlier_weight"]), _hyper_from(z, "outlier_", kind)
     K = z["stats_N"].shape[0]
     clusters = []
     for k in range(K):
@@ -187,11 +194,12 @@ def load_checkpoint(filename):
                 ss = P.multinomial_sufficient_statistics(float(z["stats_N"][k, s]), np.array(z["stats_sum"][k, s]))
                 post = _hyper_from(z, "post_", kind, (k, s))
                 dist = P.multinomial_dist(np.array(z["dist_alpha"][k, s]))
-            cps.append(H.cluster_parameters(prior, dist, ss, post))
+            cps.append(H.cluster_parameters(op if (ow > 0 and k == 0) else prior, dist, ss, post))
         sp = H.splittable_cluster_params(cps[0], cps[1], cps[2], np.array(z["lr_weights"][k]), bool(z["splittable"][k]),
                                          np.array(z["logsublikelihood_hist"][k]))
         pc = z["points_count"][k]
         clusters.append(H.local_cluster(sp, meta["total_dim"], int(pc[0]), int(pc[1]), int(pc[2])))
     group = {"model_hyperparams": mh, "labels": np.array(z["labels"]), "labels_subcluster": np.array(z["labels_subcluster"]),
-             "local_clusters": clusters, "weights": np.array(z["weights"], F32)}
+             "local_clusters": clusters, "weights": np.array(z["weights"], F32), "outlier_weight": ow,
+             "outlier_params": op}
     return group, mh, meta["iter"], meta["total_time"], meta["global_params"]

@@ -192,6 +192,9 @@ struct dpmm_ctx {
   bool dev_params = false;
   double alpha = 0.0;
   double* hyper_d = nullptr;     // [NIW_HYPER_DOUBLES(D_user)]
+  // the outlier component (dpmm_set_outlier_*): cluster 0's prior, in the layout of hyper_d, and its fixed weight
+  double* hyper_out_d = nullptr;
+  double outlier_w = 0.0;        // 0: no outlier component
   double* ptab = nullptr;        // [Kcap][3][stats_rec]   (records at D)
   double* ptab_alt = nullptr;
   double* post = nullptr;        // [Kcap][3][NIW_POST_DOUBLES(D_user)]

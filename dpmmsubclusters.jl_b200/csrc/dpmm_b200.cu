@@ -495,7 +495,7 @@ extern "C" int dpmm_destroy(dpmm_ctx* ctx) {
   void* ptrs[] = {ctx->x, ctx->sp_ptr, ctx->sp_idx, ctx->sp_val, ctx->labels, ctx->sub, ctx->perm, ctx->perm2, ctx->u_label, ctx->u_sub, ctx->r_bits,
                   ctx->raw_params, ctx->recs, ctx->cst, ctx->logw, ctx->loglr, ctx->logp_t, ctx->t2_piv, ctx->t2_scr, ctx->t2_u, ctx->t2_bias, ctx->t2_fro8, ctx->ctr_sets, ctx->tc_w, ctx->tc_b, ctx->tc_mu, ctx->tc_fro, ctx->ss_w, ctx->ss_b, ctx->ss_c, ctx->lcount, ctx->mtc_w, ctx->hist_mem, ctx->seg_off,
                   ctx->scat_cursor, ctx->lr_cursor, ctx->lut_l, ctx->lut_r, ctx->rule, ctx->wanted,
-                  ctx->idx_list, ctx->acc, ctx->centers, ctx->outbuf, ctx->items, ctx->item_ctr, ctx->hyper_d, ctx->ptab,
+                  ctx->idx_list, ctx->acc, ctx->centers, ctx->outbuf, ctx->items, ctx->item_ctr, ctx->hyper_d, ctx->hyper_out_d, ctx->ptab,
                   ctx->ptab_alt, ctx->post, ctx->post_alt, ctx->lfac, ctx->pm_out, ctx->splittable_d, ctx->newof_d,
                   ctx->w_out, ctx->lr_out, ctx->wide, ctx->wide_status};
   for (void* p : ptrs)
@@ -1731,13 +1731,14 @@ extern "C" int dpmm_num_clusters(const dpmm_ctx* ctx) { return ctx ? keff(ctx) :
 
 // The hyper-parameters, the posterior table and the draws are at the caller's D; only the statistics records and
 // what the sweep reads (lfac, the raw mu) keep the zero-padded context width ctx->D.
-extern "C" int dpmm_set_hyper_niw(dpmm_ctx* ctx, double kappa, const double* m, double nu, const double* psi, double alpha) {
-  NEED(ctx && m && psi, DPMM_EINVAL, "NULL argument");
-  NEED(ctx->prior == DPMM_PRIOR_NIW, DPMM_ESTATE, "not an NIW context");
-  NEED(kappa > 0 && nu > ctx->D_user - 1 && alpha > 0, DPMM_EINVAL, "need kappa > 0, nu > D - 1, alpha > 0");
-  CK(cudaSetDevice(ctx->device));
+//
+// Each *_hyper_block validates one prior as its dpmm_set_hyper_* documents and lays it out for the kernels; the
+// model's prior (dpmm_set_hyper_*) and the outlier component's (dpmm_set_outlier_*) are built by the same code.
+static int niw_hyper_block(dpmm_ctx* ctx, double kappa, const double* m, double nu, const double* psi, std::vector<double>& h) {
+  NEED(m && psi, DPMM_EINVAL, "NULL argument");
+  NEED(kappa > 0 && nu > ctx->D_user - 1, DPMM_EINVAL, "need kappa > 0, nu > D - 1");
   const int D = ctx->D_user;
-  std::vector<double> h(NIW_HYPER_DOUBLES(D));
+  h.assign(NIW_HYPER_DOUBLES(D), 0.0);
   // logdet psi by a host Cholesky of the symmetrised matrix (one-time, D <= 64)
   std::vector<double> A((size_t)D * D);
   for (int i = 0; i < D; ++i)
@@ -1763,22 +1764,13 @@ extern "C" int dpmm_set_hyper_niw(dpmm_ctx* ctx, double kappa, const double* m, 
   h[0] = kf; h[1] = nf; h[2] = logdet; h[3] = (double)lmv;
   for (int i = 0; i < D; ++i) h[4 + i] = m[i];
   for (int e = 0; e < D * D; ++e) h[4 + D + e] = psi[e];
-  if (!ctx->hyper_d) CK(cudaMalloc((void**)&ctx->hyper_d, h.size() * 8));
-  CK(cudaStreamSynchronize(ctx->stream));
-  CK(cudaMemcpy(ctx->hyper_d, h.data(), h.size() * 8, cudaMemcpyHostToDevice));
-  ctx->alpha = (double)(float)alpha;   // model_hyper_params.alpha is Float32 (ds.jl:9)
-  ctx->dev_params = true;
-  return ensure_tables(ctx, std::max(ctx->Kcap, 8));
+  return 0;
 }
 
-extern "C" int dpmm_set_hyper_multinomial(dpmm_ctx* ctx, const float* alpha_prior, double alpha) {
-  NEED(ctx, DPMM_EINVAL, "ctx is NULL");
-  NEED(ctx->prior == DPMM_PRIOR_MULTINOMIAL, DPMM_ESTATE, "not a multinomial context");
+static int mnm_hyper_block(dpmm_ctx* ctx, const float* alpha_prior, std::vector<double>& h) {
   NEED(alpha_prior, DPMM_EINVAL, "alpha_prior is NULL");
-  NEED(alpha > 0, DPMM_EINVAL, "need alpha > 0");
-  CK(cudaSetDevice(ctx->device));
   const int D = ctx->D;
-  std::vector<double> h(MNM_HYPER_DOUBLES(D));
+  h.assign(MNM_HYPER_DOUBLES(D), 0.0);
   double sa = 0.0;
   for (int d = 0; d < D; ++d) {
     NEED(std::isfinite(alpha_prior[d]) && alpha_prior[d] > 0.f, DPMM_EINVAL, "every alpha_prior[d] must be finite and > 0");
@@ -1787,24 +1779,17 @@ extern "C" int dpmm_set_hyper_multinomial(dpmm_ctx* ctx, const float* alpha_prio
   }
   h[0] = sa;
   h[1] = std::lgamma(sa);
-  if (!ctx->hyper_d) CK(cudaMalloc((void**)&ctx->hyper_d, h.size() * 8));
-  CK(cudaStreamSynchronize(ctx->stream));
-  CK(cudaMemcpy(ctx->hyper_d, h.data(), h.size() * 8, cudaMemcpyHostToDevice));
-  ctx->alpha = (double)(float)alpha;
-  ctx->dev_params = true;
-  return ensure_tables(ctx, std::max(ctx->Kcap, 8));
+  return 0;
 }
 
-extern "C" int dpmm_set_hyper_diag(dpmm_ctx* ctx, double kappa, const double* m, double nu, const double* psi, double alpha) {
-  NEED(ctx && m && psi, DPMM_EINVAL, "NULL argument");
-  NEED(ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN, DPMM_ESTATE, "not a diagonal Gaussian context");
-  NEED(kappa > 0 && nu > 0 && alpha > 0, DPMM_EINVAL, "need kappa > 0, nu > 0, alpha > 0");
+static int diag_hyper_block(dpmm_ctx* ctx, double kappa, const double* m, double nu, const double* psi, std::vector<double>& h) {
+  NEED(m && psi, DPMM_EINVAL, "NULL argument");
+  NEED(kappa > 0 && nu > 0, DPMM_EINVAL, "need kappa > 0, nu > 0");
   // diag_niw_hyperparams stores kappa and nu as Float32, as niw_hyperparams does
   const double kf = (double)(float)kappa, nf = (double)(float)nu;
   NEED(kf > 0 && std::isfinite(kf) && nf > 0 && std::isfinite(nf), DPMM_EINVAL, "kappa and nu must be finite and > 0 in Float32");
-  CK(cudaSetDevice(ctx->device));
   const int D = ctx->D;
-  std::vector<double> h(DIAG_HYPER_DOUBLES(D));
+  h.assign(DIAG_HYPER_DOUBLES(D), 0.0);
   double slp = 0.0;
   for (int d = 0; d < D; ++d) {
     NEED(std::isfinite(m[d]), DPMM_EINVAL, "every m[d] must be finite");
@@ -1815,16 +1800,102 @@ extern "C" int dpmm_set_hyper_diag(dpmm_ctx* ctx, double kappa, const double* m,
   }
   h[0] = kf; h[1] = nf; h[2] = slp;
   h[3] = (double)(float)std::lgamma(nf / 2.0);   // log_multivariate_gamma(nu / 2, 1)
-  if (!ctx->hyper_d) CK(cudaMalloc((void**)&ctx->hyper_d, h.size() * 8));
+  return 0;
+}
+
+// *dst <- h, in stream order after every kernel that may still read the old block
+static int upload_hyper(dpmm_ctx* ctx, double** dst, const std::vector<double>& h) {
+  if (!*dst) CK(cudaMalloc((void**)dst, h.size() * 8));
+  CK(cudaMemcpyAsync(*dst, h.data(), h.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
-  CK(cudaMemcpy(ctx->hyper_d, h.data(), h.size() * 8, cudaMemcpyHostToDevice));
-  ctx->alpha = (double)(float)alpha;
+  return 0;
+}
+
+static int set_model_hyper(dpmm_ctx* ctx, const std::vector<double>& h, double alpha) {
+  int rc = upload_hyper(ctx, &ctx->hyper_d, h);
+  if (rc) return rc;
+  ctx->alpha = (double)(float)alpha;   // model_hyper_params.alpha is Float32 (ds.jl:9)
   ctx->dev_params = true;
   return ensure_tables(ctx, std::max(ctx->Kcap, 8));
 }
 
+extern "C" int dpmm_set_hyper_niw(dpmm_ctx* ctx, double kappa, const double* m, double nu, const double* psi, double alpha) {
+  NEED(ctx, DPMM_EINVAL, "ctx is NULL");
+  NEED(ctx->prior == DPMM_PRIOR_NIW, DPMM_ESTATE, "not an NIW context");
+  NEED(alpha > 0, DPMM_EINVAL, "need alpha > 0");
+  std::vector<double> h;
+  int rc = niw_hyper_block(ctx, kappa, m, nu, psi, h);
+  if (rc) return rc;
+  CK(cudaSetDevice(ctx->device));
+  return set_model_hyper(ctx, h, alpha);
+}
+
+extern "C" int dpmm_set_hyper_multinomial(dpmm_ctx* ctx, const float* alpha_prior, double alpha) {
+  NEED(ctx, DPMM_EINVAL, "ctx is NULL");
+  NEED(ctx->prior == DPMM_PRIOR_MULTINOMIAL, DPMM_ESTATE, "not a multinomial context");
+  NEED(alpha > 0, DPMM_EINVAL, "need alpha > 0");
+  std::vector<double> h;
+  int rc = mnm_hyper_block(ctx, alpha_prior, h);
+  if (rc) return rc;
+  CK(cudaSetDevice(ctx->device));
+  return set_model_hyper(ctx, h, alpha);
+}
+
+extern "C" int dpmm_set_hyper_diag(dpmm_ctx* ctx, double kappa, const double* m, double nu, const double* psi, double alpha) {
+  NEED(ctx, DPMM_EINVAL, "ctx is NULL");
+  NEED(ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN, DPMM_ESTATE, "not a diagonal Gaussian context");
+  NEED(alpha > 0, DPMM_EINVAL, "need alpha > 0");
+  std::vector<double> h;
+  int rc = diag_hyper_block(ctx, kappa, m, nu, psi, h);
+  if (rc) return rc;
+  CK(cudaSetDevice(ctx->device));
+  return set_model_hyper(ctx, h, alpha);
+}
+
 #define DPMM_NEED_HYPER(what) \
   NEED(ctx->dev_params, DPMM_ESTATE, "dpmm_set_hyper_niw, dpmm_set_hyper_multinomial or dpmm_set_hyper_diag must precede " what)
+
+// ---- the outlier component (DESIGN.md 6.1): cluster 1 under a prior of its own, at a fixed weight ----
+static int outlier_precheck(dpmm_ctx* ctx, int prior, double weight) {
+  NEED(ctx, DPMM_EINVAL, "ctx is NULL");
+  NEED(ctx->prior == prior, DPMM_ESTATE, "the outlier prior must be of the context's prior type");
+  DPMM_NEED_HYPER("dpmm_set_outlier_*");
+  NEED(weight >= 0.0 && weight < 1.0, DPMM_EINVAL, "the outlier weight must lie in [0, 1)");
+  CK(cudaSetDevice(ctx->device));
+  return 0;
+}
+static int set_outlier_block(dpmm_ctx* ctx, double weight, const std::vector<double>& h) {
+  int rc = upload_hyper(ctx, &ctx->hyper_out_d, h);
+  if (rc) return rc;
+  ctx->outlier_w = weight;
+  return 0;
+}
+// the prior of cluster 0 in the parameter kernels
+static const double* hyper0(const dpmm_ctx* ctx) { return ctx->outlier_w > 0.0 ? ctx->hyper_out_d : ctx->hyper_d; }
+
+extern "C" int dpmm_set_outlier_niw(dpmm_ctx* ctx, double weight, double kappa, const double* m, double nu, const double* psi) {
+  int rc = outlier_precheck(ctx, DPMM_PRIOR_NIW, weight);
+  if (rc) return rc;
+  std::vector<double> h;
+  rc = niw_hyper_block(ctx, kappa, m, nu, psi, h);
+  return rc ? rc : set_outlier_block(ctx, weight, h);
+}
+
+extern "C" int dpmm_set_outlier_multinomial(dpmm_ctx* ctx, double weight, const float* alpha_prior) {
+  int rc = outlier_precheck(ctx, DPMM_PRIOR_MULTINOMIAL, weight);
+  if (rc) return rc;
+  std::vector<double> h;
+  rc = mnm_hyper_block(ctx, alpha_prior, h);
+  return rc ? rc : set_outlier_block(ctx, weight, h);
+}
+
+extern "C" int dpmm_set_outlier_diag(dpmm_ctx* ctx, double weight, double kappa, const double* m, double nu, const double* psi) {
+  int rc = outlier_precheck(ctx, DPMM_PRIOR_DIAG_GAUSSIAN, weight);
+  if (rc) return rc;
+  std::vector<double> h;
+  rc = diag_hyper_block(ctx, kappa, m, nu, psi, h);
+  return rc ? rc : set_outlier_block(ctx, weight, h);
+}
 
 static size_t niw_post_smem(int D) { return ((size_t)D * (D + 1) + 2 * D) * sizeof(double); }   // D: the caller's
 
@@ -1832,8 +1903,8 @@ static size_t niw_post_smem(int D) { return ((size_t)D * (D + 1) + 2 * D) * size
 static int launch_post(dpmm_ctx* ctx, const int32_t* idx_d, int m, double* out) {
   if (ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN) {
     DiagPostArgs pa{};
-    pa.D = ctx->D; pa.rec = ctx->stats_rec; pa.hyper = ctx->hyper_d; pa.ptab = ctx->ptab; pa.idx_list = idx_d;
-    pa.post = ctx->post; pa.out = out;
+    pa.D = ctx->D; pa.rec = ctx->stats_rec; pa.hyper = ctx->hyper_d; pa.hyper0 = hyper0(ctx); pa.ptab = ctx->ptab;
+    pa.idx_list = idx_d; pa.post = ctx->post; pa.out = out;
     KernelTimer kt(ctx, TK_PARAMS);
     diag_post_kernel<<<dim3((unsigned)m, 3), DIAG_PARAM_THREADS, 0, ctx->stream>>>(pa);
     CK(cudaGetLastError());
@@ -1841,15 +1912,16 @@ static int launch_post(dpmm_ctx* ctx, const int32_t* idx_d, int m, double* out) 
   }
   if (ctx->prior == DPMM_PRIOR_MULTINOMIAL) {
     MnmPostArgs pa{};
-    pa.D = ctx->D; pa.rec = ctx->stats_rec; pa.hyper = ctx->hyper_d; pa.ptab = ctx->ptab; pa.idx_list = idx_d;
-    pa.post = ctx->post; pa.out = out;
+    pa.D = ctx->D; pa.rec = ctx->stats_rec; pa.hyper = ctx->hyper_d; pa.hyper0 = hyper0(ctx); pa.ptab = ctx->ptab;
+    pa.idx_list = idx_d; pa.post = ctx->post; pa.out = out;
     KernelTimer kt(ctx, TK_PARAMS);
     mnm_post_kernel<<<dim3((unsigned)m, 3), MNM_PARAM_THREADS, 0, ctx->stream>>>(pa);
     CK(cudaGetLastError());
     return 0;
   }
   NiwPostArgs pa{};
-  pa.D = ctx->D_user; pa.ld = ctx->D; pa.rec = ctx->stats_rec; pa.hyper = ctx->hyper_d; pa.ptab = ctx->ptab;
+  pa.D = ctx->D_user; pa.ld = ctx->D; pa.rec = ctx->stats_rec; pa.hyper = ctx->hyper_d; pa.hyper0 = hyper0(ctx);
+  pa.ptab = ctx->ptab;
   pa.idx_list = idx_d; pa.post = ctx->post; pa.out = out;
   const size_t sm = niw_post_smem(ctx->D_user);
   if (sm > 48 * 1024) CK(cudaFuncSetAttribute(niw_post_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
@@ -1910,7 +1982,7 @@ extern "C" int dpmm_posterior_step(dpmm_ctx* ctx, const int64_t* indices, int32_
     const dim3 grid((unsigned)k_merge, (unsigned)k_merge);
     if (ctx->prior == DPMM_PRIOR_MULTINOMIAL) {
       MnmMergeArgs ma{};
-      ma.D = ctx->D; ma.rec = rec; ma.K = k_merge; ma.hyper = ctx->hyper_d; ma.ptab = ctx->ptab;
+      ma.D = ctx->D; ma.rec = rec; ma.K = k_merge; ma.hyper = ctx->hyper_d; ma.hyper0 = hyper0(ctx); ma.ptab = ctx->ptab;
       ma.splittable = ctx->splittable_d; ma.out = merge_d;
       int rcf = side_fork(ctx);
       if (rcf) return rcf;
@@ -1918,7 +1990,7 @@ extern "C" int dpmm_posterior_step(dpmm_ctx* ctx, const int64_t* indices, int32_
       mnm_merge_kernel<<<grid, MNM_PARAM_THREADS, 0, ctx->side>>>(ma);
     } else if (ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN) {
       DiagMergeArgs ma{};
-      ma.D = ctx->D; ma.rec = rec; ma.K = k_merge; ma.hyper = ctx->hyper_d; ma.ptab = ctx->ptab;
+      ma.D = ctx->D; ma.rec = rec; ma.K = k_merge; ma.hyper = ctx->hyper_d; ma.hyper0 = hyper0(ctx); ma.ptab = ctx->ptab;
       ma.splittable = ctx->splittable_d; ma.out = merge_d;
       int rcf = side_fork(ctx);
       if (rcf) return rcf;
@@ -1926,7 +1998,8 @@ extern "C" int dpmm_posterior_step(dpmm_ctx* ctx, const int64_t* indices, int32_
       diag_merge_kernel<<<grid, DIAG_PARAM_THREADS, 0, ctx->side>>>(ma);
     } else {
       NiwMergeArgs ma{};
-      ma.D = ctx->D_user; ma.ld = ctx->D; ma.rec = rec; ma.K = k_merge; ma.hyper = ctx->hyper_d; ma.ptab = ctx->ptab;
+      ma.D = ctx->D_user; ma.ld = ctx->D; ma.rec = rec; ma.K = k_merge; ma.hyper = ctx->hyper_d; ma.hyper0 = hyper0(ctx);
+      ma.ptab = ctx->ptab;
       ma.splittable = ctx->splittable_d; ma.out = merge_d;
       const size_t sm = niw_post_smem(ctx->D_user);
       if (sm > 48 * 1024) CK(cudaFuncSetAttribute(niw_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
@@ -1982,7 +2055,7 @@ extern "C" int dpmm_sample_params(dpmm_ctx* ctx, int32_t K, int32_t from_prior, 
     WeightsArgs wa{};
     wa.K = K; wa.D = D; wa.post = ctx->post; wa.stride = post_doubles(ctx); wa.alpha = ctx->alpha; wa.logw = ctx->logw;
     wa.loglr = ctx->loglr; wa.w_out = ctx->w_out; wa.lr_out = ctx->lr_out; wa.seed = ctx->seed; wa.call = ctx->pcall;
-    wa.unit = unit_weights;
+    wa.unit = unit_weights; wa.outlier = ctx->outlier_w;
     rc = side_fork(ctx);
     if (rc) return rc;
     ctx->launches += 1;
@@ -1991,7 +2064,8 @@ extern "C" int dpmm_sample_params(dpmm_ctx* ctx, int32_t K, int32_t from_prior, 
   }
   if (ctx->prior == DPMM_PRIOR_MULTINOMIAL) {
     MnmDrawArgs da{};
-    da.D = D; da.hyper = ctx->hyper_d; da.post = ctx->post; da.logp = ctx->recs; da.seed = ctx->seed; da.call = ctx->pcall;
+    da.D = D; da.hyper = ctx->hyper_d; da.hyper0 = hyper0(ctx); da.post = ctx->post; da.logp = ctx->recs; da.seed = ctx->seed;
+    da.call = ctx->pcall;
     da.first = from_prior;
     {
       KernelTimer kt(ctx, TK_PARAMS);
@@ -2006,7 +2080,7 @@ extern "C" int dpmm_sample_params(dpmm_ctx* ctx, int32_t K, int32_t from_prior, 
   }
   if (ctx->prior == DPMM_PRIOR_DIAG_GAUSSIAN) {
     DiagDrawArgs da{};
-    da.D = D; da.rec = ctx->stats_rec; da.hyper = ctx->hyper_d; da.ptab = ctx->ptab; da.post = ctx->post;
+    da.D = D; da.rec = ctx->stats_rec; da.hyper = ctx->hyper_d; da.hyper0 = hyper0(ctx); da.ptab = ctx->ptab; da.post = ctx->post;
     da.mu = ctx->raw_params; da.var = ctx->raw_params + nrec * D; da.logdet = ctx->raw_params + 2 * nrec * D;
     da.seed = ctx->seed; da.call = ctx->pcall; da.first = from_prior;
     {
@@ -2022,7 +2096,8 @@ extern "C" int dpmm_sample_params(dpmm_ctx* ctx, int32_t K, int32_t from_prior, 
     const int Du = ctx->D_user;
     NiwDrawArgs da{};
     da.D = Du; da.ld = D; da.mu = ctx->raw_params; da.logdet = ctx->raw_params + nrec * D + nrec * D * D;
-    da.hyper = ctx->hyper_d; da.post = ctx->post; da.lfac = ctx->lfac; da.seed = ctx->seed; da.call = ctx->pcall;
+    da.hyper = ctx->hyper_d; da.hyper0 = hyper0(ctx); da.post = ctx->post; da.lfac = ctx->lfac; da.seed = ctx->seed;
+    da.call = ctx->pcall;
     da.first = from_prior;
     const size_t sm = ((size_t)3 * Du * (Du + 1) + 2 * Du) * sizeof(double);
     if (sm > 48 * 1024) CK(cudaFuncSetAttribute(niw_draw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
@@ -2040,6 +2115,7 @@ extern "C" int dpmm_params_merge(dpmm_ctx* ctx, int64_t i, int64_t j) {
   CK(cudaSetDevice(ctx->device));
   DPMM_NEED_HYPER("dpmm_params_merge");
   NEED(i >= 1 && j >= 1 && i != j && i <= ctx->Kcap_tab && j <= ctx->Kcap_tab, DPMM_EINVAL, "bad cluster pair");
+  NEED(!(ctx->outlier_w > 0.0 && (i == 1 || j == 1)), DPMM_EINVAL, "the outlier component (cluster 1) is never merged");
   KernelTimer kt(ctx, TK_PARAMS);
   ptab_merge_kernel<<<1, 256, 0, ctx->stream>>>(ctx->ptab, ctx->stats_rec, (int)i - 1, (int)j - 1);
   CK(cudaGetLastError());

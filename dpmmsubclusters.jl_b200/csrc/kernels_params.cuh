@@ -22,6 +22,9 @@
 //   niw_merge_kernel  one CTA per candidate pair (i < j): log marginal likelihood of the summed statistics.
 //   dpmm_weights_kernel  mixture weights and sub-cluster weights (Gamma draws), written as the Float32 logs
 //                     the sweep kernels read.
+// The outlier component (DESIGN.md 6.1): cluster index 0 may have a prior of its own.  The posterior, draw and merge
+// kernels of every prior take it as `hyper0`, which CTAs of cluster 0 read instead of `hyper`; without the component
+// it is the model's block, so the kernels do what they did before it existed.
 // Randomness: Philox4x32-10 keyed by (seed, stream PARAMS, parameter-call counter, distribution, variate,
 // attempt): every rank of a multi-GPU run draws identical parameters from identical all-reduced statistics.
 #pragma once
@@ -167,6 +170,7 @@ __device__ inline double niw_logml_cta(const double* hyper, int D, int LD, const
 struct NiwPostArgs {
   int D, ld, rec;
   const double* hyper;
+  const double* hyper0;      // prior of cluster 0 (the outlier component's, or == hyper)
   const double* ptab;        // [K][3][rec]
   const int32_t* idx_list;   // [m] or nullptr (a = k)
   double* post;              // [K][3][NIW_POST_DOUBLES]
@@ -181,15 +185,16 @@ __global__ void __launch_bounds__(256) niw_post_kernel(const NiwPostArgs a) {
   double* sxs = mp + D;
   const int ai = blockIdx.x, s = blockIdx.y;
   const int k = a.idx_list != nullptr ? a.idx_list[ai] : ai;
+  const double* hyper = k == 0 ? a.hyper0 : a.hyper;
   const double* src[1] = {a.ptab + ((size_t)k * 3 + s) * a.rec};
   double N, kp, nup;
-  niw_posterior_to_smem(a.hyper, D, a.ld, LD, src, 1, true, A, mp, sxs, N, kp, nup);
+  niw_posterior_to_smem(hyper, D, a.ld, LD, src, 1, true, A, mp, sxs, N, kp, nup);
   const bool ok = cta_cholesky(A, D, LD);
   double* P = a.post + ((size_t)k * 3 + s) * NIW_POST_DOUBLES(D);
   for (int e = threadIdx.x; e < D * D; e += blockDim.x) P[8 + D + e] = A[(e / D) * LD + (e % D)];
   for (int i = threadIdx.x; i < D; i += blockDim.x) P[8 + i] = mp[i];
   double logdet;
-  double lml = niw_logml_cta(a.hyper, D, LD, A, N, kp, nup, sxs, logdet);
+  double lml = niw_logml_cta(hyper, D, LD, A, N, kp, nup, sxs, logdet);
   if (threadIdx.x == 0) {
     if (!ok) lml = __longlong_as_double(0x7ff8000000000000LL);
     P[0] = kp; P[1] = nup; P[2] = N; P[3] = lml; P[4] = logdet; P[5] = ok ? 1.0 : 0.0;
@@ -201,6 +206,7 @@ __global__ void __launch_bounds__(256) niw_post_kernel(const NiwPostArgs a) {
 struct NiwMergeArgs {
   int D, ld, rec, K;         // D, ld, rec as in NiwPostArgs
   const double* hyper;
+  const double* hyper0;        // as in NiwPostArgs (pairs (0, j))
   const double* ptab;
   const uint8_t* splittable;   // [K]
   double* out;                 // [K][K]: entry (i, j), i < j both splittable and non-empty; NaN elsewhere
@@ -224,12 +230,13 @@ __global__ void __launch_bounds__(256) niw_merge_kernel(const NiwMergeArgs a) {
   double* A = ps;
   double* mp = A + D * LD;
   double* sxs = mp + D;
+  const double* hyper = i == 0 ? a.hyper0 : a.hyper;
   const double* src[2] = {si, sj};
   double N, kp, nup;
-  niw_posterior_to_smem(a.hyper, D, a.ld, LD, src, 2, false, A, mp, sxs, N, kp, nup);
+  niw_posterior_to_smem(hyper, D, a.ld, LD, src, 2, false, A, mp, sxs, N, kp, nup);
   const bool ok = cta_cholesky(A, D, LD);
   double logdet;
-  const double lml = niw_logml_cta(a.hyper, D, LD, A, N, kp, nup, sxs, logdet);
+  const double lml = niw_logml_cta(hyper, D, LD, A, N, kp, nup, sxs, logdet);
   if (threadIdx.x == 0) *o = ok ? lml : __longlong_as_double(0x7ff8000000000000LL);
 }
 
@@ -240,6 +247,7 @@ struct NiwDrawArgs {
   float* mu;                 // [3K][ld] out
   float* logdet;             // [3K] out (log det of the D x D Sigma)
   const double* hyper;
+  const double* hyper0;      // prior of cluster 0 (distributions t < 3)
   const double* post;        // [K][3][NIW_POST_DOUBLES(D)]
   double* lfac;              // [3K][ld][ld] out: L (invSigma = L L'), row-major: input of niw_pack_kernel
   uint64_t seed;
@@ -257,15 +265,16 @@ __global__ void __launch_bounds__(NIW_PACK_THREADS) niw_draw_kernel(const NiwDra
   double* y = xi + D;
   const int t = blockIdx.x, tid = threadIdx.x, NT = NIW_PACK_THREADS;
   const double* P = a.post + (size_t)t * NIW_POST_DOUBLES(D);
+  const double* hyper = t < 3 ? a.hyper0 : a.hyper;
   const bool prior = a.first != 0 || !(P[2] > 0.0);
   double kp, nup;
   const double* mpost;
   if (prior) {
     // factor of the prior psi in reversed order
-    kp = a.hyper[0];
-    nup = a.hyper[1];
-    mpost = a.hyper + 4;
-    const double* psi = a.hyper + 4 + D;
+    kp = hyper[0];
+    nup = hyper[1];
+    mpost = hyper + 4;
+    const double* psi = hyper + 4 + D;
     for (int e = tid; e < D * D; e += NT) {
       const int i = e / D, j = e - i * D;
       Wk[(D - 1 - i) * LD + (D - 1 - j)] = 0.5 * (psi[e] + psi[j * D + i]);
@@ -390,12 +399,20 @@ struct WeightsArgs {
   uint64_t seed;
   uint32_t call;
   int unit;               // 1: weights = 1/K (init_first_clusters!, dp-parallel-sampling.jl:77), lr = (0.5, 0.5)... see host
+  double outlier;         // weight of the outlier component (cluster 0), 0 without it
 };
 // sample_clusters! :430-436 and sample_cluster_params shared_actions.jl:46-49.  One CTA.
+// With the outlier component (outlier = w > 0): w_0 = fl32(w), w_k = (1 - w) Dirichlet(N_1..N_{K-1}, alpha)[k] for
+// k >= 1 (unit: (1 - w) / (K - 1)).  Cluster 0 takes no Gamma draw; every other variate keeps its Philox key.
 __global__ void __launch_bounds__(256) dpmm_weights_kernel(const WeightsArgs a) {
   extern __shared__ double gs[];   // [K + 1]
   const int K = a.K, tid = threadIdx.x;
+  const bool outlier = a.outlier > 0.0;
   for (int k = tid; k <= K; k += blockDim.x) {
+    if (outlier && k == 0) {
+      gs[0] = 0.0;   // (adds nothing to the total: 0 + x == x)
+      continue;
+    }
     ParamRng rng(a.seed, a.call, 0xFFFFFFu, (uint32_t)k);
     const double shape = k < K ? fmax(a.post[(size_t)(3 * k) * a.stride + 2], 1e-300) : a.alpha;
     gs[k] = rng.gamma(shape);
@@ -419,7 +436,13 @@ __global__ void __launch_bounds__(256) dpmm_weights_kernel(const WeightsArgs a) 
   }
   __syncthreads();
   for (int k = tid; k < K; k += blockDim.x) {
-    const float w = a.unit ? (float)(1.0 / K) : (float)(gs[k] / tot);
+    float w;
+    if (!outlier)
+      w = a.unit ? (float)(1.0 / K) : (float)(gs[k] / tot);
+    else if (k == 0)
+      w = (float)a.outlier;
+    else
+      w = a.unit ? (float)((1.0 - a.outlier) / (K - 1)) : (float)((1.0 - a.outlier) * (gs[k] / tot));
     a.w_out[k] = w;
     a.logw[k] = (float)log((double)w);
   }

@@ -80,6 +80,7 @@ __device__ inline double diag_logml_cta(const double* hyper, int D, double N, St
 struct DiagPostArgs {
   int D, rec;                // rec = 1 + 2D: N | sum x[D] | sum x^2[D]
   const double* hyper;       // [DIAG_HYPER_DOUBLES(D)]
+  const double* hyper0;      // prior of cluster 0 (the outlier component's, or == hyper)
   const double* ptab;        // [K][3][rec]
   const int32_t* idx_list;   // [m] or nullptr (a = k)
   double* post;              // [K][3][DIAG_POST_DOUBLES]
@@ -94,7 +95,7 @@ __global__ void __launch_bounds__(DIAG_PARAM_THREADS) diag_post_kernel(const Dia
   const double N = src[0];
   double kp, nup;
   const double lml = diag_logml_cta(
-      a.hyper, D, N,
+      k == 0 ? a.hyper0 : a.hyper, D, N,
       [&](int d, double& sx, double& sxx) {
         sx = src[1 + d];
         sxx = src[1 + D + d];
@@ -111,6 +112,7 @@ __global__ void __launch_bounds__(DIAG_PARAM_THREADS) diag_post_kernel(const Dia
 struct DiagMergeArgs {
   int D, rec, K;
   const double* hyper;
+  const double* hyper0;        // as in DiagPostArgs (pairs (0, j))
   const double* ptab;
   const uint8_t* splittable;   // [K]
   double* out;                 // [K][K]: entry (i, j), i < j both splittable and non-empty; NaN elsewhere
@@ -129,7 +131,7 @@ __global__ void __launch_bounds__(DIAG_PARAM_THREADS) diag_merge_kernel(const Di
   // aggregate_suff_stats: the sums of the two cluster records
   double kp, nup;
   const double lml = diag_logml_cta(
-      a.hyper, D, si[0] + sj[0],
+      i == 0 ? a.hyper0 : a.hyper, D, si[0] + sj[0],
       [&](int d, double& sx, double& sxx) {
         sx = si[1 + d] + sj[1 + d];
         sxx = si[1 + D + d] + sj[1 + D + d];
@@ -141,6 +143,7 @@ __global__ void __launch_bounds__(DIAG_PARAM_THREADS) diag_merge_kernel(const Di
 struct DiagDrawArgs {
   int D, rec;
   const double* hyper;
+  const double* hyper0;      // prior of cluster 0 (distributions t < 3)
   const double* ptab;        // [3K][rec]: m' and psi' are recomputed from the statistics
   const double* post;        // [3K][DIAG_POST_DOUBLES]
   float* mu;                 // [3K][D] out
@@ -157,18 +160,19 @@ __global__ void __launch_bounds__(DIAG_PARAM_THREADS) diag_draw_kernel(const Dia
   const int t = blockIdx.x, D = a.D;
   const double* P = a.post + (size_t)t * DIAG_POST_DOUBLES;
   const double* S = a.ptab + (size_t)t * a.rec;
+  const double* hyper = t < 3 ? a.hyper0 : a.hyper;
   const bool prior = a.first != 0 || !(P[2] > 0.0);
   const double N = prior ? 0.0 : P[2];
-  const double kp = a.hyper[0] + N, nup = a.hyper[1] + N;       // what m' and psi' are computed with
-  const double kd = prior ? a.hyper[0] : P[0], nd = prior ? a.hyper[1] : P[1];   // the Float32 kappa', nu'
+  const double kp = hyper[0] + N, nup = hyper[1] + N;       // what m' and psi' are computed with
+  const double kd = prior ? hyper[0] : P[0], nd = prior ? hyper[1] : P[1];   // the Float32 kappa', nu'
   double lsum = 0.0;
   for (int d = threadIdx.x; d < D; d += DIAG_PARAM_THREADS) {
     double mp, psip;
     if (prior) {
-      mp = a.hyper[4 + d];
-      psip = a.hyper[4 + D + d];
+      mp = hyper[4 + d];
+      psip = hyper[4 + D + d];
     } else {
-      diag_posterior_feature(a.hyper, D, d, kp, nup, S[1 + d], S[1 + D + d], mp, psip);
+      diag_posterior_feature(hyper, D, d, kp, nup, S[1 + d], S[1 + D + d], mp, psip);
     }
     ParamRng rng(a.seed, a.call, (uint32_t)t, (uint32_t)d);
     const double chi2 = 2.0 * rng.gamma(0.5 * nd);

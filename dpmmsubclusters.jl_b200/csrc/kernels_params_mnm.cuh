@@ -79,6 +79,7 @@ __device__ inline double mnm_logml_cta(const double* hyper, int D, bool empty, S
 struct MnmPostArgs {
   int D, rec;
   const double* hyper;       // [MNM_HYPER_DOUBLES]
+  const double* hyper0;      // prior of cluster 0 (the outlier component's, or == hyper)
   const double* ptab;        // [K][3][rec]: N | sum x[D]
   const int32_t* idx_list;   // [m] or nullptr (a = k)
   double* post;              // [K][3][MNM_POST_DOUBLES]
@@ -92,7 +93,8 @@ __global__ void __launch_bounds__(MNM_PARAM_THREADS) mnm_post_kernel(const MnmPo
   const double* src = a.ptab + ((size_t)k * 3 + s) * a.rec;
   double* P = a.post + ((size_t)k * 3 + s) * MNM_POST_DOUBLES(D);
   const double N = src[0];
-  const double lml = mnm_logml_cta(a.hyper, D, !(N > 0.0), [&](int d) { return (float)src[1 + d]; }, P + 4, red);
+  const double lml = mnm_logml_cta(k == 0 ? a.hyper0 : a.hyper, D, !(N > 0.0), [&](int d) { return (float)src[1 + d]; },
+                                   P + 4, red);
   if (threadIdx.x == 0) {
     P[2] = N;
     P[3] = lml;
@@ -104,6 +106,7 @@ __global__ void __launch_bounds__(MNM_PARAM_THREADS) mnm_post_kernel(const MnmPo
 struct MnmMergeArgs {
   int D, rec, K;
   const double* hyper;
+  const double* hyper0;        // as in MnmPostArgs (pairs (0, j))
   const double* ptab;
   const uint8_t* splittable;   // [K]
   double* out;                 // [K][K]: entry (i, j), i < j both splittable and non-empty; NaN elsewhere
@@ -120,7 +123,7 @@ __global__ void __launch_bounds__(MNM_PARAM_THREADS) mnm_merge_kernel(const MnmM
     return;
   }
   // aggregate_suff_stats adds the two Float32 statistics in Float32
-  const double lml = mnm_logml_cta(a.hyper, a.D, false,
+  const double lml = mnm_logml_cta(i == 0 ? a.hyper0 : a.hyper, a.D, false,
                                    [&](int d) { return __fadd_rn((float)si[1 + d], (float)sj[1 + d]); }, nullptr, red);
   if (threadIdx.x == 0) *o = lml;
 }
@@ -136,6 +139,7 @@ __device__ inline double mnm_log_gamma(ParamRng& rng, double a) {
 struct MnmDrawArgs {
   int D;
   const double* hyper;
+  const double* hyper0;      // prior of cluster 0 (distributions t < 3)
   const double* post;        // [3K][MNM_POST_DOUBLES]
   float* logp;               // [3K][D] out
   uint64_t seed;
@@ -148,7 +152,7 @@ __global__ void __launch_bounds__(MNM_PARAM_THREADS) mnm_draw_kernel(const MnmDr
   __shared__ double red[MNM_PARAM_THREADS / 32];
   const int t = blockIdx.x, D = a.D;
   const double* P = a.post + (size_t)t * MNM_POST_DOUBLES(D);
-  const double* alpha = (a.first != 0 || !(P[2] > 0.0)) ? a.hyper + 2 : P + 4;
+  const double* alpha = (a.first != 0 || !(P[2] > 0.0)) ? (t < 3 ? a.hyper0 : a.hyper) + 2 : P + 4;
   double mx = -CUDART_INF;
   for (int d = threadIdx.x; d < D; d += MNM_PARAM_THREADS) {
     ParamRng rng(a.seed, a.call, (uint32_t)t, (uint32_t)d);

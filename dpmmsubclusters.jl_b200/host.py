@@ -78,6 +78,8 @@ class local_group:                   # ds.jl:51-58; points/labels/labels_subclus
 class dp_parallel_sampling:          # ds.jl:76-79
     model_hyperparams: model_hyper_params
     group: local_group
+    outlier_weight: float = 0.0          # the outlier component (DESIGN.md 6.1), recorded by save_model
+    outlier_params: object = None
 
 
 @dataclass
@@ -90,7 +92,8 @@ class Settings:
     split_stop: int = 5
     burnout_period: int = 20
     max_num_of_clusters: float = np.inf
-    outlier_mod: float = 0.0
+    outlier_mod: float = 0.0             # weight of the outlier component (cluster 1); 0 = no component
+    outlier_hyper_params: object = None  # its prior, of the model prior's type and dimension
     use_verbose: bool = False
     ground_truth: object = None
     use_smart_splits: bool = False
@@ -178,6 +181,17 @@ def create_first_local_cluster(group, cfg, rng):
     return cluster
 
 
+def create_outlier_local_cluster(group, outlier_params, cfg, rng):
+    """:42-61.  Cluster 1 of a model with the outlier component: its own prior, distributions drawn from it, lr
+    weights (0.5, 0.5), no points (the initial labels start at 2)."""
+    suff = P.empty_suff_stats(outlier_params)
+    dist = P.sample_distribution(outlier_params, rng)
+    cp = cluster_parameters(outlier_params, dist, suff, outlier_params)
+    cpl, cpr = copy.deepcopy(cp), copy.deepcopy(cp)
+    splittable = splittable_cluster_params(cp, cpl, cpr, np.array([0.5, 0.5]), False, _neg_inf_hist(cfg))
+    return local_cluster(splittable, group.model_hyperparams.total_dim, 0, 0, 0)
+
+
 def update_suff_stats_posterior(group, indices=None):
     """update_suff_stats_posterior! :206-254.  The fetch of the workers' dictionaries and their
     aggregate_suff_stats reduction (:229-248) is one dpmm_suff_stats call (all-reduce inside)."""
@@ -207,8 +221,12 @@ def sample_clusters(group, first, cfg, rng):
         cluster.points_count = int(cluster.cluster_params.cluster_params.suff_statistics.N)
         points_count.append(cluster.points_count)
     points_count.append(α)
+    om = cfg.outlier_mod
+    if om > 0:                                                      # cluster 1 keeps its fixed weight
+        points_count = points_count[1:]
     pc = np.maximum(np.asarray(points_count, np.float64), 1e-300)   # Dirichlet needs positive parameters
-    group.weights = (rng.dirichlet(pc)[:-1] * (1 - cfg.outlier_mod)).astype(F32)
+    w = rng.dirichlet(pc)[:-1] * (1 - om)
+    group.weights = (np.concatenate([[om], w]) if om > 0 else w).astype(F32)
 
 
 def broadcast_cluster_params(group):
@@ -323,12 +341,15 @@ def check_and_merge(group, final, cfg, rng):
 
 
 def remove_empty_clusters(group, cfg):
-    """remove_empty_clusters! :457-471."""
+    """remove_empty_clusters! :457-471.  The sweep drops exactly the clusters the host drops: a kept empty cluster (the
+    outlier component, or cluster 2 while K = 2) is passed with a count of 1."""
     new_vec, pts_count = [], []
     n = len(group.local_clusters)
     for index, cluster in enumerate(group.local_clusters, start=1):
-        pts_count.append(int(cluster.points_count))
-        if cluster.points_count > 0 or (cfg.outlier_mod > 0 and index == 1) or (cfg.outlier_mod > 0 and index == 2 and n == 2):
+        keep = (cluster.points_count > 0 or (cfg.outlier_mod > 0 and index == 1)
+                or (cfg.outlier_mod > 0 and index == 2 and n == 2))
+        pts_count.append(max(int(cluster.points_count), 1) if keep else 0)
+        if keep:
             new_vec.append(cluster)
     group.sweep.remove_empty(pts_count)                    # remove_empty_clusters_worker! :446-455
     group.local_clusters = new_vec
@@ -428,21 +449,28 @@ def init_model_from_data(all_data, hyper_params, α, cfg, seed, sweep_factory, s
     sweep.n_total = n_total
     mh = model_hyper_params(hyper_params, float(F32(α)), all_data.shape[1])
     sweep.init_labels(cfg.initial_clusters, cfg.outlier_mod > 0)
-    return dp_parallel_sampling(mh, local_group(mh, sweep))
+    return dp_parallel_sampling(mh, local_group(mh, sweep), cfg.outlier_mod, cfg.outlier_hyper_params)
 
 
 def init_first_clusters(dp_model, cfg, rng):
     """init_first_clusters! :62-78."""
     g = dp_model.group
+    om = cfg.outlier_mod
+    if om > 0:                                             # :66-68: the outlier component is cluster 1
+        g.local_clusters.append(create_outlier_local_cluster(g, cfg.outlier_hyper_params, cfg, rng))
     for _ in range(cfg.initial_clusters):
         g.local_clusters.append(create_first_local_cluster(g, cfg, rng))
     update_suff_stats_posterior(g)
-    if cfg.use_smart_splits:                               # :70-75
-        for i in range(1, len(g.local_clusters) + 1):
+    if cfg.use_smart_splits:                               # :70-75 (never the outlier component)
+        for i in range(2 if om > 0 else 1, len(g.local_clusters) + 1):
             smart_cluster_init(g, i, cfg)
         update_suff_stats_posterior(g)
     sample_clusters(g, False, cfg, rng)
-    g.weights = np.full(len(g.local_clusters), 1.0 / len(g.local_clusters), F32) if len(g.local_clusters) > 1 else np.ones(1, F32)
+    K = len(g.local_clusters)
+    if om > 0:
+        g.weights = np.array([om] + [(1 - om) / (K - 1)] * (K - 1), F32)
+    else:
+        g.weights = np.full(K, 1.0 / K, F32) if K > 1 else np.ones(1, F32)
     broadcast_cluster_params(g)
 
 
@@ -484,6 +512,7 @@ def _clusters_from_device(group, st, cfg):
     """Rebuild the reference's host objects (local_cluster list, weights) from the final device state, so that
     the tuple fit() returns, predict() and calculate_posterior() see what the host path would have left."""
     hyper = group.model_hyperparams.distribution_hyper_params
+    om = cfg.outlier_mod
     sw = group.sweep
     K = st.K
     counts, sum_x, sum_xx = sw.suff_stats(list(range(1, K + 1)))
@@ -504,13 +533,16 @@ def _clusters_from_device(group, st, cfg):
         # distribution and weight before anything reads them (sample_clusters!, :659), so these never reach a sweep.
         tot = max(float(counts[:, 0].sum()), 1.0)
         w = counts[:, 0] / tot
+        if om > 0:
+            w = np.concatenate([[om], (1 - om) * counts[1:, 0] / max(float(counts[1:, 0].sum()), 1.0)])
         lr = (counts[:, 1:3] + 0.5) / (counts[:, 1:3] + 0.5).sum(axis=1, keepdims=True)
     group.local_clusters = []
     for k in range(K):
+        h = cfg.outlier_hyper_params if (om > 0 and k == 0) else hyper     # cluster 1: the outlier component's prior
         cps = []
         for s_ in range(3):
             ss = P.make_suff_stats(hyper, counts[k, s_], sum_x[k, s_], None if sum_xx is None else sum_xx[k, s_])
-            post = P.calc_posterior(hyper, ss)
+            post = P.calc_posterior(h, ss)
             if diag:
                 if params is not None:
                     dist = P.diag_gaussian(mu[k, s_].copy(), var[k, s_].copy(), float(logdet[k, s_]))
@@ -532,7 +564,7 @@ def _clusters_from_device(group, st, cfg):
                 inv = np.linalg.inv(post.ψ)
                 dist = P.mv_gaussian(post.m.astype(F32), post.ψ.astype(F32), inv.astype(F32),
                                      float(np.linalg.slogdet(post.ψ)[1]), np.linalg.cholesky(inv).T)
-            cps.append(cluster_parameters(hyper, dist, ss, post))
+            cps.append(cluster_parameters(h, dist, ss, post))
         sp = splittable_cluster_params(cps[0], cps[1], cps[2], lr[k].astype(np.float64), bool(st.splittable[k]),
                                        st.hist[k].copy())
         group.local_clusters.append(local_cluster(sp, group.model_hyperparams.total_dim, int(counts[k, 0]),
@@ -552,8 +584,7 @@ def dp_parallel(all_data, local_hyper_params=None, α_param=None, iters=100, ini
     if isinstance(all_data, (str, os.PathLike)):
         return dp_parallel_params_file(str(all_data), verbose=verbose, gt=gt, sweep_factory=sweep_factory, shard=shard,
                                        comm=comm, device=device, device_params=device_params)
-    if outlier_weight:
-        raise NotImplementedError("the outlier component is out of scope (DESIGN.md 6)")
+    outlier_weight, outlier_params = _outlier_settings(local_hyper_params, outlier_weight, outlier_params)
     if save_model and save_path is None:
         raise ValueError("save_model=True needs save_path (global_params.jl:37 in the reference)")
     if sps.issparse(all_data) and isinstance(local_hyper_params, (P.niw_hyperparams, P.diag_niw_hyperparams)):
@@ -568,9 +599,28 @@ def dp_parallel(all_data, local_hyper_params=None, α_param=None, iters=100, ini
     cfg = Settings(iterations=int(iters), initial_clusters=int(init_clusters), burnout_period=int(burnout),
                    max_num_of_clusters=max_clusters, use_verbose=bool(verbose), ground_truth=gt,
                    use_smart_splits=bool(smart_splits), should_save_model=bool(save_model), save_path=save_path or "",
-                   save_file_prefix=save_file_prefix, model_save_interval=int(model_save_interval))
+                   save_file_prefix=save_file_prefix, model_save_interval=int(model_save_interval),
+                   outlier_mod=outlier_weight, outlier_hyper_params=outlier_params)
     return _run_from_settings(all_data, local_hyper_params, α_param, cfg, seed, sweep_factory, shard, comm, device,
                               device_params)
+
+
+def _outlier_settings(hyper, weight, params):
+    """(weight, prior) of the outlier component, validated; (0.0, None) when it is off (weight 0)."""
+    weight = float(weight)
+    if not 0.0 <= weight < 1.0:
+        raise ValueError(f"outlier_weight must lie in [0, 1), got {weight}")
+    if weight == 0.0:
+        return 0.0, None
+    if params is None:
+        raise ValueError("outlier_weight > 0 needs outlier_params")
+    if type(params) is not type(hyper):
+        raise ValueError(f"outlier_params must be a {type(hyper).__name__}, as the model's prior, "
+                         f"not a {type(params).__name__}")
+    shape = lambda h: np.shape(h.α) if isinstance(h, P.multinomial_hyper) else (np.shape(h.m), np.shape(h.ψ))
+    if shape(params) != shape(hyper):
+        raise ValueError("outlier_params must have the dimension of the model's prior")
+    return weight, params
 
 
 def _run_from_settings(all_data, local_hyper_params, α_param, cfg, seed, sweep_factory, shard, comm, device, device_params,
@@ -614,6 +664,11 @@ def _run_from_settings(all_data, local_hyper_params, α_param, cfg, seed, sweep_
 
 
 def _settings_from_params(gp, verbose, gt):
+    """The component is on when the file sets outlier_mod > 0 and outlier_hyper_params (global_params.jl defaults to
+    outlier_mod = 0.05 without hyper-parameters: off)."""
+    om, ohp = 0.0, None
+    if gp["outlier_hyper_params"] is not None and gp["outlier_mod"] > 0 and gp["hyper_params"] is not None:
+        om, ohp = _outlier_settings(gp["hyper_params"], gp["outlier_mod"], gp["outlier_hyper_params"])
     return Settings(iterations=int(gp["iterations"]), hard_clustering=bool(gp["hard_clustering"]),
                     initial_clusters=int(gp["initial_clusters"]), argmax_sample_stop=int(gp["argmax_sample_stop"]),
                     split_stop=int(gp["split_stop"]), burnout_period=int(gp["burnout_period"]),
@@ -621,7 +676,7 @@ def _settings_from_params(gp, verbose, gt):
                     use_smart_splits=bool(gp["smart_splits"]), max_split_iter=int(gp["max_split_iter"]),
                     should_save_model=bool(gp["enable_saving"]), model_save_interval=int(gp["model_save_interval"]),
                     save_path=gp["save_path"], save_file_prefix=gp["save_file_prefix"], data_path=gp["data_path"],
-                    data_prefix=gp["data_prefix"])
+                    data_prefix=gp["data_prefix"], outlier_mod=om, outlier_hyper_params=ohp)
 
 
 def dp_parallel_params_file(model_params, verbose=True, gt=None, **kw):
@@ -656,6 +711,8 @@ def run_model_from_checkpoint(filename, verbose=True, gt=None, data=None, **kw):
                 setattr(cfg, k, v)
         cfg.global_params = gparams
         seed = (gparams or {}).get("random_seed")
+    # the component is part of the saved model: cluster 1 of the restored list is it, or there is none
+    cfg.outlier_mod, cfg.outlier_hyper_params = grp["outlier_weight"], grp["outlier_params"]
     if data is None:
         data = load_data(cfg.data_path, prefix=cfg.data_prefix)                   # :435
     data = _points(data)

@@ -68,8 +68,11 @@ def history_step(st, cfg):
 
 def group_step_device(sw, st, α, no_more_splits, final, cfg, rng, keep_params=False):
     """One Gibbs iteration; returns nothing, mutates `st` and the device state."""
+    outlier = cfg.outlier_mod > 0                          # cluster 1 (index 0) is the outlier component
     # sample_clusters! + broadcast (device)
     history_step(st, cfg)
+    if outlier:
+        st.splittable[0] = False                           # so it is never a split candidate nor in a merge pair
     sw.sample_params(st.K)
     if keep_params:                                        # the distributions fit() returns (last iteration only)
         get = {NIW: sw.get_params_niw, DIAG: sw.get_params_diag}.get(sw.prior_kind, sw.get_params_multinomial)
@@ -150,10 +153,15 @@ def group_step_device(sw, st, α, no_more_splits, final, cfg, rng, keep_params=F
                 for i, j in zip(merged_i, merged_j):
                     sw.params_merge(i + 1, j + 1)
                 sw.posterior_step(mi + 1, from_table=True, fetch=False)
-    # remove_empty_clusters!
-    if (st.N[:, 0] == 0).any():
-        sw.remove_empty(st.N[:, 0])
-        mask = st.N[:, 0] > 0
+    # remove_empty_clusters!: the outlier component, and cluster 2 while K = 2, stay even when empty; the sweep is
+    # told a count of 1 for them so that it keeps exactly the clusters kept here
+    mask = st.N[:, 0] > 0
+    if outlier:
+        mask[0] = True
+        if st.K == 2:
+            mask[1] = True
+    if not mask.all():
+        sw.remove_empty(np.where(mask, np.maximum(st.N[:, 0], 1), 0))
         if keep_params and getattr(st, "params", None) is not None:
             kp = mask[:st.params[0].shape[0]]
             st.params = tuple(a[kp] for a in st.params)
@@ -181,12 +189,19 @@ def run_model_device(dp_model, cfg, rng, normalized_mutual_info, first_iter=1, r
     sw = g.sweep
     hyper = g.model_hyperparams.distribution_hyper_params
     α = g.model_hyperparams.α
+    om, oh = cfg.outlier_mod, cfg.outlier_hyper_params
     if isinstance(hyper, P.niw_hyperparams):
         sw.set_hyper_niw(hyper.κ, hyper.m, hyper.ν, hyper.ψ, α)
+        if om > 0:
+            sw.set_outlier_niw(om, oh.κ, oh.m, oh.ν, oh.ψ)
     elif isinstance(hyper, P.diag_niw_hyperparams):
         sw.set_hyper_diag(hyper.κ, hyper.m, hyper.ν, hyper.ψ, α)
+        if om > 0:
+            sw.set_outlier_diag(om, oh.κ, oh.m, oh.ν, oh.ψ)
     else:
         sw.set_hyper_multinomial(hyper.α, α)
+        if om > 0:
+            sw.set_outlier_multinomial(om, oh.α)
     if resume:
         K = len(g.local_clusters)
         st = DeviceState(K, cfg.burnout_period + 5)
@@ -197,12 +212,13 @@ def run_model_device(dp_model, cfg, rng, normalized_mutual_info, first_iter=1, r
         counts, logml, _ = sw.posterior_step(np.arange(1, K + 1))
         st.N[:], st.logml[:] = counts[:K], logml[:K]
     else:
-        st = DeviceState(cfg.initial_clusters, cfg.burnout_period + 5)
+        c0 = 2 if om > 0 else 1                                # the outlier component (no points yet) is cluster 1
+        st = DeviceState(cfg.initial_clusters + c0 - 1, cfg.burnout_period + 5)
         for _ in range(cfg.initial_clusters):
             sw.randomize_sublabels(None)                       # split_first_cluster_worker! per first cluster
         counts, logml, _ = sw.posterior_step(None)
         if cfg.use_smart_splits:                               # init_first_clusters! :70-75
-            smart_init_device(sw, np.arange(1, st.K + 1), cfg)
+            smart_init_device(sw, np.arange(c0, st.K + 1), cfg)
             counts, logml, _ = sw.posterior_step(None)
         st.N[:], st.logml[:] = counts[:st.K], logml[:st.K]
         history_step(st, cfg)                                  # sample_clusters!(group, false) of init_first_clusters!

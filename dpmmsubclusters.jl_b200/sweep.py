@@ -233,6 +233,27 @@ class GpuSweep:
         self._ck(self.lib.dpmm_set_hyper_diag(self.h, float(kappa), _ptr(m, C.c_double), float(nu), _ptr(psi, C.c_double),
                                               float(alpha)))
 
+    def set_outlier_niw(self, weight, kappa, m, nu, psi):
+        """The outlier component (cluster 1) under niw_hyperparams(kappa, m, nu, psi) at the fixed weight; after
+        set_hyper_niw.  weight = 0 turns it off."""
+        m = np.ascontiguousarray(m, np.float64).reshape(-1)
+        psi = np.ascontiguousarray(psi, np.float64)
+        assert m.shape == (self.D,) and psi.shape == (self.D, self.D)
+        self._ck(self.lib.dpmm_set_outlier_niw(self.h, float(weight), float(kappa), _ptr(m, C.c_double), float(nu),
+                                               _ptr(psi, C.c_double)))
+
+    def set_outlier_multinomial(self, weight, alpha_prior):
+        a = np.ascontiguousarray(alpha_prior, np.float32).reshape(-1)
+        assert a.shape == (self.D,)
+        self._ck(self.lib.dpmm_set_outlier_multinomial(self.h, float(weight), _ptr(a, C.c_float)))
+
+    def set_outlier_diag(self, weight, kappa, m, nu, psi):
+        m = np.ascontiguousarray(m, np.float64).reshape(-1)
+        psi = np.ascontiguousarray(psi, np.float64).reshape(-1)
+        assert m.shape == (self.D,) and psi.shape == (self.D,)
+        self._ck(self.lib.dpmm_set_outlier_diag(self.h, float(weight), float(kappa), _ptr(m, C.c_double), float(nu),
+                                                _ptr(psi, C.c_double)))
+
     def posterior_step(self, indices=None, splittable=None, from_table=False, fetch=True):
         """Statistics (unless from_table) -> table -> posteriors.  Returns (counts [m,3] i64, logml [m,3] f64,
         merge [K,K] f64 or None); `splittable` (bool [K]) requests the merge table."""

@@ -180,6 +180,16 @@ int dpmm_set_hyper_multinomial(dpmm_ctx* ctx, const float* alpha_prior, double a
  * pointer, kappa <= 0, nu <= 0, alpha <= 0, a non-finite m[d] or a psi[d] that is not finite and > 0; DPMM_ESTATE on
  * a context of another prior. */
 int dpmm_set_hyper_diag(dpmm_ctx* ctx, double kappa, const double* m, double nu, const double* psi, double alpha);
+/* The outlier component (DESIGN.md 6.1): cluster 1 becomes a cluster under a prior of its own with the fixed mixture
+ * weight fl32(weight); the other weights are (1 - weight) Dirichlet(N_2..N_K, alpha), or (1 - weight) / (K - 1) with
+ * unit_weights.  The posterior, draws (from_prior too) and log marginal likelihood of cluster 1 use this prior; the
+ * sweep is unchanged.  The host never splits or merges cluster 1 (dpmm_params_merge refuses it) and keeps it through
+ * dpmm_remove_empty.  Each call follows the matching dpmm_set_hyper_* (DPMM_ESTATE before it or on a context of another
+ * prior), validates the prior exactly as dpmm_set_hyper_* does and needs 0 <= weight < 1 (DPMM_EINVAL otherwise);
+ * weight = 0 turns the component off again. */
+int dpmm_set_outlier_niw(dpmm_ctx* ctx, double weight, double kappa, const double* m, double nu, const double* psi);
+int dpmm_set_outlier_multinomial(dpmm_ctx* ctx, double weight, const float* alpha_prior);
+int dpmm_set_outlier_diag(dpmm_ctx* ctx, double weight, double kappa, const double* m, double nu, const double* psi);
 /* update_suff_stats_posterior! (local_clusters_actions.jl:206-254) kept on the device: statistics of the
  * listed clusters (NULL = all) -> all-reduce -> persistent table -> posterior hyper-parameters and log
  * marginal likelihoods of {cluster, left, right}.  from_table != 0: skip the statistics and re-evaluate the
@@ -196,7 +206,8 @@ int dpmm_posterior_step(dpmm_ctx* ctx, const int64_t* indices, int32_t n_indices
  * init_first_clusters!, dp-parallel-sampling.jl:77), and pack them for the sweep.  Replaces dpmm_set_params_*. */
 int dpmm_sample_params(dpmm_ctx* ctx, int32_t k, int32_t from_prior, int32_t unit_weights);
 /* merge_clusters_to_splittable (shared_actions.jl:12-18) on the statistics table: cluster i <- {i + j, i, j},
- * cluster j <- empty (1-based).  Follow with dpmm_posterior_step(from_table = 1) for i. */
+ * cluster j <- empty (1-based).  Follow with dpmm_posterior_step(from_table = 1) for i.  DPMM_EINVAL for i or j = 1
+ * while the outlier component is on. */
 int dpmm_params_merge(dpmm_ctx* ctx, int64_t i, int64_t j);
 /* The parameters of the last dpmm_sample_params: mu float32 [3K][D], lfac double [3K][D][D] (L lower,
  * invSigma = L L'), logdet float32 [3K] (log det Sigma), weights float32 [K], lr_weights float32 [K][2]; D is the

@@ -195,6 +195,28 @@ function set_hyper!(c::Ctx, κ::Real, m::Vector{Float64}, ν::Real, ψ::Vector{F
 end
 
 """
+    set_outlier_niw!(c, weight, κ, m, ν, ψ)
+    set_outlier_multinomial!(c, weight, α_prior)
+    set_outlier_diag!(c, weight, κ, m, ν, ψ)
+
+The outlier component of `dp_parallel(...; outlier_weight, outlier_params)` on the device parameter path: cluster 1
+gets the prior `outlier_params` and the fixed mixture weight `outlier_weight` (0 turns it off again).  Call after the
+matching set_hyper!, with initial labels from init_labels!(c, initial_clusters, true); never mark cluster 1 splittable
+and keep it (count >= 1) in remove_empty!.
+"""
+function set_outlier_niw!(c::Ctx, weight::Real, κ::Real, m::Vector{Float64}, ν::Real, ψ::Matrix{Float64})
+    GC.@preserve m ψ check(ccall((:dpmm_set_outlier_niw, lib), Cint,
+        (Ptr{Cvoid}, Cdouble, Cdouble, Ptr{Cdouble}, Cdouble, Ptr{Cdouble}), c.ptr, weight, κ, m, ν, ψ), c.ptr)
+end
+set_outlier_multinomial!(c::Ctx, weight::Real, α_prior::Vector{Float32}) =
+    GC.@preserve α_prior check(ccall((:dpmm_set_outlier_multinomial, lib), Cint,
+        (Ptr{Cvoid}, Cdouble, Ptr{Cfloat}), c.ptr, weight, α_prior), c.ptr)
+function set_outlier_diag!(c::Ctx, weight::Real, κ::Real, m::Vector{Float64}, ν::Real, ψ::Vector{Float64})
+    GC.@preserve m ψ check(ccall((:dpmm_set_outlier_diag, lib), Cint,
+        (Ptr{Cvoid}, Cdouble, Cdouble, Ptr{Cdouble}, Cdouble, Ptr{Cdouble}), c.ptr, weight, κ, m, ν, ψ), c.ptr)
+end
+
+"""
     posterior_step(c, indices; splittable=nothing, from_table=false) -> (counts[3,m], logml[3,m], merge[K,K] or nothing)
 
 update_suff_stats_posterior! (local_clusters_actions.jl:206-254) kept on the device.  `indices === nothing`
